@@ -14,7 +14,8 @@ Workloads (`--workload`, default `auto`):
                gather, no collective), MS-TCN over each rank's sequences, logits gathered the same way.  Strong scaling.
   native480    (`--hw 480x854`; BASELINE.json configs[4])  a step = one batch of `--batch` (64) frames at 480x854 per GPU through the
                encoder + embedding head (no MS-TCN: 64 unrelated frames are not a sequence).
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0).  `--dump-outputs DIR` also writes what the last timed step computed (rank 0) as DIR/<name>.npy; weights
+and inputs come from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -60,6 +61,26 @@ def gemm_kernel_sha256(root):
         h.update(open(os.path.join(d, f)).read().encode())
     return h.hexdigest()
 
+
+DUMP_BYTES = 64 << 20   # cap on what --dump-outputs writes
+
+
+def dump_outputs(out_dir, arrays, frames):
+    """Writes {name: (tensor, frame axis)} as out_dir/<name>.npy in float32.  Every tensor has `frames` entries along its frame axis;
+    when the set is larger than DUMP_BYTES, the same fixed, seeded sample of frames is kept in each, and frame_index.npy lists them."""
+    os.makedirs(out_dir, exist_ok=True)
+    per_frame = sum(t.numel() // frames * 4 for t, _ in arrays.values())
+    keep = None
+    if per_frame * frames > DUMP_BYTES:
+        n = DUMP_BYTES // (per_frame + 8)
+        keep = torch.randperm(frames, generator=torch.Generator().manual_seed(0))[:n].sort().values
+        np.save(os.path.join(out_dir, "frame_index.npy"), keep.double().numpy())
+    for name, (t, axis) in arrays.items():
+        if keep is not None:
+            t = t.index_select(axis, keep.to(t.device))
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -78,7 +99,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32), to compare two builds output for output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     a.H, a.W = (int(v) for v in a.hw.lower().split("x"))
     if a.workload == "auto":
         a.workload = "native480" if (a.H, a.W) != (224, 224) else ("video2300" if a.gpus <= 1 else "cholec80x80")
@@ -303,7 +330,7 @@ class Ctx:
 
     def timed(self, step, steps, warmup):
         """W warm-up steps, then exactly K steps between CUDA events on the launching stream, barrier + synchronize on both sides,
-        max over ranks; nvidia-smi clocks sampled during the timed region (rank 0)."""
+        max over ranks; nvidia-smi clocks sampled during the timed region (rank 0).  Also returns what the last step returned."""
         sampler = ClockSampler(self.local)
         nwarm = max(3, warmup)
         for i in range(nwarm):
@@ -316,13 +343,13 @@ class Ctx:
         sampler.mark_begin()
         e0.record()
         for _ in range(steps):
-            step()
+            out = step()
         e1.record()
         self.barrier()
         sampler.mark_end()
         ms = self.max_over_ranks(e0.elapsed_time(e1))
         clocks = sampler.stop() if self.rank == 0 else None
-        return ms, clocks, nwarm
+        return ms, clocks, nwarm, out
 
     def wall(self, fn):
         """Host wall-clock of fn() between barriers, max over ranks (the end-to-end legs: copies, launches and synchronisation included)."""
@@ -452,8 +479,11 @@ def run_video(ctx):
         launches["n"] = n + tcn.last_launch_count(dev)
         return logits
 
-    ms_total, clocks, nwarm = ctx.timed(step, a.steps, a.warmup)
+    ms_total, clocks, nwarm, out = ctx.timed(step, a.steps, a.warmup)
     value = world * T * a.steps / (ms_total / 1e3)
+    if a.dump_outputs and rank == 0:
+        # features [T, 2048]; video2300 adds the MS-TCN logits [stages, classes, T]
+        dump_outputs(a.dump_outputs, {"features": (feats, 0)} if native else {"features": (feats, 0), "logits": (out, 2)}, T)
 
     # ---- end-to-end through the public API with HOST buffers (pinned), H2D + D2H inside the timed region
     e2e = None
@@ -585,8 +615,11 @@ def run_cholec80(ctx):
         cur.wait_stream(side)                                     # the step ends when the last block is gathered
         launches["n"] = n
 
-    ms_total, clocks, nwarm = ctx.timed(step, a.steps, a.warmup)
+    ms_total, clocks, nwarm, _ = ctx.timed(step, a.steps, a.warmup)
     value = total * a.steps / (ms_total / 1e3)
+    if a.dump_outputs and rank == 0:
+        # the gathered arrays every rank's blocks landed in, rows in video order: features [total, 2048], logits [total, stages x classes]
+        dump_outputs(a.dump_outputs, {"features": (shared.array, 0), "logits": (shared_lg.array, 0)}, total)
 
     e2e = None
     numa_cpus = lfb.bind_to_gpu_numa_node(ctx.local) if world > 1 else None

@@ -1,6 +1,6 @@
 """Pins the oracle (oracle/*.py, a CPU restatement of the reference) against
   (a) the committed golden vectors, which are outputs of the REAL reference (tests/golden/make_golden.py), and
-  (b) the real reference itself when /root/reference is present (this container only).
+  (b) a known answer recorded from the reference's own MS-TCN module.
 The reference ships no tests or golden vectors of its own (SURVEY.md F4)."""
 import os
 
@@ -11,8 +11,8 @@ import torch
 import surgvid_b200  # noqa: F401
 from oracle import evp_oracle as EO
 from oracle import mstcn_oracle as MO
-from oracle.ref_loader import load_reference, reference_available
 from surgvid_b200 import synthetic as S
+from surgvid_b200.mstcn import MultiStageModel_S
 
 CFG = S.EVP_CONFIGS["mit_b3_evp"]
 
@@ -74,25 +74,16 @@ def test_mstcn_causality():
     assert torch.equal(oa[..., :400], ob[..., :400])
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present (GPU box)")
-def test_oracle_matches_live_reference():
-    evp, mstcn = load_reference()
+def test_oracle_matches_reference_known_answer():
+    """Known answer of the reference's MS-TCN (SURVEY.md §8c): its own init under manual_seed(0), applied to a seeded 2 300-frame
+    sequence, gives logits summing to -4348.2007 with mean |logit| 0.256878.  The drop-in module draws the same initial weights
+    (tests/test_host_cpu.py), so the oracle must reproduce both numbers.  The EVP oracle is pinned to the reference's outputs by the
+    golden tests above."""
     torch.manual_seed(0)
-    m = evp.mit_b3_evp().eval()
-    sd = S.synth_state_dict(S.evp_key_shapes("mit_b3_evp"), seed=3, mode="stress")
-    assert list(sd.keys()) == list(m.state_dict().keys())
-    m.load_state_dict(sd, strict=True)
-    x, seg, flow = S.synth_frames(1, seed=21)
-    with torch.no_grad():
-        ref = m(x, seg, flow, return_features=True)
-    assert (EO.evp_forward(sd, CFG, x, seg, flow) - ref).abs().max() < 5e-5
-    # survey known answer (SURVEY.md §8c): the reference module's own init under manual_seed(0)
-    torch.manual_seed(0)
-    mm = mstcn.MultiStageModel_S(2, 8, 32, 2048, 14, True).eval()
+    sd = MultiStageModel_S(2, 8, 32, 2048, 14, True).state_dict()
     gen = torch.Generator().manual_seed(1234)
     xx = torch.randn(1, 2300, 2048, generator=gen).transpose(2, 1)
     with torch.no_grad():
-        o = mm(xx)
+        o = MO.mstcn_forward(sd, xx)
     assert abs(float(o.double().sum()) - (-4348.2007)) < 5e-3
-    mine = MO.mstcn_forward({k: v for k, v in mm.state_dict().items()}, xx)
-    assert (mine - o).abs().max() < 1e-5
+    assert abs(float(o.abs().mean()) - 0.256878) < 1e-6
