@@ -26,7 +26,7 @@ EXPORTED_SYMBOLS = [
     "sv_evp_forward", "sv_evp_classify", "sv_evp_read_tap", "sv_evp_last_launch_count", "sv_evp_set_profile", "sv_evp_get_profile", "sv_evp_dump_profile",
     "sv_mstcn_create", "sv_mstcn_destroy", "sv_mstcn_set_tensor", "sv_mstcn_pack_weights", "sv_mstcn_workspace_bytes",
     "sv_mstcn_forward", "sv_mstcn_last_launch_count", "sv_mstcn_forward_query", "sv_op_causal_windows",
-    "sv_op_gemm_bf16", "sv_op_layernorm", "sv_op_im2col", "sv_op_dwconv3x3_gelu", "sv_op_attention", "sv_op_gauss5x5",
+    "sv_op_gemm_bf16", "sv_op_layernorm", "sv_op_im2col", "sv_op_dwconv3x3_gelu", "sv_op_attention", "sv_op_attention_kernel", "sv_op_gauss5x5",
     "sv_op_bilinear_tokens", "sv_op_token_mean", "sv_op_stem_conv", "sv_op_mixffn_fc2", "sv_op_gemm_bf16_cat",
     "sv_prep_create", "sv_prep_destroy", "sv_prep_workspace_bytes", "sv_prep_images", "sv_prep_flow",
     "sv_trans_create", "sv_trans_destroy", "sv_trans_set_tensor", "sv_trans_pack_weights", "sv_trans_forward",
@@ -128,6 +128,7 @@ def _declare(lib):
     lib.sv_op_dwconv3x3_gelu.argtypes = [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]
     lib.sv_op_attention.argtypes = [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_int32, c_int32,
                                     c_int32, c_int32, c_float, c_void_p]
+    lib.sv_op_attention_kernel.argtypes = [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_int32]
     lib.sv_op_gauss5x5.argtypes = [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p]
     lib.sv_op_bilinear_tokens.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int64, c_void_p]
     lib.sv_op_stem_conv.argtypes = [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_float, c_int32, c_int32, c_int32, c_int32, c_int32,

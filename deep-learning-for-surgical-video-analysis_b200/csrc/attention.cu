@@ -526,12 +526,24 @@ __global__ void __launch_bounds__(128) attention_resident_multi_kernel(const bf1
   cp_async_wait<0>();
 }
 
+// the kernel launch_attention runs for these operands (SV_ATTN_*, include/surgvid.h)
+int attention_kernel_for(int hd, int Nkv, int64_t ldq, int64_t ldk, int64_t ldv, int64_t ldo, const void* q, const void* k, const void* v,
+                         const void* o) {
+  if (attention_tc_enabled() && attention_tc_supported(hd, Nkv, ldq, ldk, ldv, ldo, q, k, v, o))
+    return Nkv <= kTile ? SV_ATTN_TC_SINGLE : SV_ATTN_TC_MULTI;
+  // the resident kernels store 16-byte chunks of output rows (heads of 20 columns stay 8-byte aligned under these)
+  const bool o16 = ldo % 8 == 0 && (reinterpret_cast<uintptr_t>(o) & 15) == 0;
+  if (o16 && Nkv <= kTile) return SV_ATTN_RESIDENT;
+  if (o16 && Nkv <= 4 * kTile) return SV_ATTN_RESIDENT_MULTI;
+  return SV_ATTN_STREAM;
+}
+
 template <int HD>
-int attn_launch(const bf16* q, int64_t ldq, const bf16* k, int64_t ldk, const bf16* v, int64_t ldv, bf16* o, int64_t ldo, int B, int heads,
-                int Nq, int Nkv, float scale, cudaStream_t st) {
+int attn_launch(int kernel, const bf16* q, int64_t ldq, const bf16* k, int64_t ldk, const bf16* v, int64_t ldv, bf16* o, int64_t ldo, int B,
+                int heads, int Nq, int Nkv, float scale, cudaStream_t st) {
   const float scale_log2 = scale * 1.4426950408889634f;
   const int qtiles = ceil_div(Nq, kTile);
-  if (Nkv <= kTile && ldo % 8 == 0 && (reinterpret_cast<uintptr_t>(o) & 15) == 0) {  // (heads of 20 columns stay 8-byte aligned under these)
+  if (kernel == SV_ATTN_RESIDENT) {
     // enough CTAs to fill the machine a few times over, but as many query tiles per CTA as that allows (K/V loaded once per CTA)
     int tpc = 1;
     while (tpc < 8 && tpc < qtiles && static_cast<long long>(ceil_div(qtiles, tpc * 2)) * heads * B >= 4LL * 148 * 4) tpc *= 2;
@@ -540,7 +552,7 @@ int attn_launch(const bf16* q, int64_t ldq, const bf16* k, int64_t ldk, const bf
     attention_resident_kv_kernel<HD><<<grid, 128, 0, st>>>(q, ldq, k, ldk, v, ldv, o, ldo, Nq, Nkv, scale_log2, tpc);
     return launch_status("attention_resident_kv_kernel");
   }
-  if (Nkv <= 4 * kTile && ldo % 8 == 0 && (reinterpret_cast<uintptr_t>(o) & 15) == 0) {
+  if (kernel == SV_ATTN_RESIDENT_MULTI) {
     using S = AttnShape<HD>;
     const int kv_tiles = ceil_div(Nkv, kTile);
     const int smem = (2 + 2 * kv_tiles) * kTile * S::LDS * static_cast<int>(sizeof(bf16));
@@ -563,16 +575,18 @@ int launch_attention(const bf16* q, int64_t ldq, const bf16* k, int64_t ldk, con
   SV_CHECK(B <= 65535 && heads <= 65535, "attention grid limits");
   SV_CHECK(ldq % 8 == 0 && ldk % 8 == 0 && ldv % 8 == 0 && ldo % 2 == 0, "attention leading dims must keep 16-byte row alignment");
   SV_CHECK(((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(k) | reinterpret_cast<uintptr_t>(v)) & 15) == 0, "attention operand alignment");
-  if (attention_tc_enabled() && attention_tc_supported(hd, Nkv, ldq, ldk, ldv, ldo, q, k, v, o)) {
+  SV_CHECK((reinterpret_cast<uintptr_t>(o) & 3) == 0, "attention output must be 4-byte aligned (the kernels store bf16 pairs)");
+  const int kernel = attention_kernel_for(hd, Nkv, ldq, ldk, ldv, ldo, q, k, v, o);
+  if (kernel == SV_ATTN_TC_SINGLE || kernel == SV_ATTN_TC_MULTI) {
     AttnTcPlan plan;
     SV_TRY(attention_tc_plan(q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, &plan));
     return attention_tc_launch(plan, st);
   }
   switch (hd) {
-    case 20: return attn_launch<20>(q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, st);
-    case 32: return attn_launch<32>(q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, st);
-    case 40: return attn_launch<40>(q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, st);
-    case 64: return attn_launch<64>(q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, st);
+    case 20: return attn_launch<20>(kernel, q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, st);
+    case 32: return attn_launch<32>(kernel, q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, st);
+    case 40: return attn_launch<40>(kernel, q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, st);
+    case 64: return attn_launch<64>(kernel, q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, st);
     default: return fail(SV_ERR_UNSUPPORTED, "attention head_dim must be 20, 32, 40 or 64");
   }
 }
@@ -584,4 +598,9 @@ extern "C" int sv_op_attention(const uint16_t* q, int64_t ldq, const uint16_t* k
   return sv::launch_attention(reinterpret_cast<const sv::bf16*>(q), ldq, reinterpret_cast<const sv::bf16*>(k), ldk,
                               reinterpret_cast<const sv::bf16*>(v), ldv, reinterpret_cast<sv::bf16*>(o), ldo, B, heads, Nq, Nkv, hd, scale,
                               static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int sv_op_attention_kernel(const uint16_t* q, int64_t ldq, const uint16_t* k, int64_t ldk, const uint16_t* v, int64_t ldv,
+                                      const uint16_t* o, int64_t ldo, int32_t Nkv, int32_t hd) {
+  return sv::attention_kernel_for(hd, Nkv, ldq, ldk, ldv, ldo, q, k, v, o);
 }

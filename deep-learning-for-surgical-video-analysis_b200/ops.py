@@ -179,15 +179,19 @@ def dwconv3x3_gelu(x: torch.Tensor, w9c: torch.Tensor, bias: torch.Tensor) -> to
     return out
 
 
-def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, B: int, heads: int, hd: int, scale: float) -> torch.Tensor:
-    """q [B*Nq, >=heads*hd] bf16, k/v [B*Nkv, ...] bf16 (row-strided views allowed) -> o [B*Nq, heads*hd] bf16."""
-    _require_cuda(q, k, v)
+def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, B: int, heads: int, hd: int, scale: float,
+              out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """q [B*Nq, >=heads*hd] bf16, k/v [B*Nkv, ...] bf16 (row-strided views allowed) -> o [B*Nq, heads*hd] bf16, written into `out`
+    when given (its row stride may exceed heads*hd)."""
+    _require_cuda(q, k, v, out)
     Nq, Nkv = q.shape[0] // B, k.shape[0] // B
-    o = torch.empty((q.shape[0], heads * hd), dtype=torch.bfloat16, device=q.device)
-    rc = _native.lib().sv_op_attention(_ptr(q), q.stride(0), _ptr(k), k.stride(0), _ptr(v), v.stride(0), _ptr(o), o.stride(0), B, heads, Nq, Nkv,
-                                       hd, scale, _stream_ptr(q.device))
+    if out is None:
+        out = torch.empty((q.shape[0], heads * hd), dtype=torch.bfloat16, device=q.device)
+    assert out.dtype == torch.bfloat16 and tuple(out.shape) == (q.shape[0], heads * hd) and out.stride(1) == 1
+    rc = _native.lib().sv_op_attention(_ptr(q), q.stride(0), _ptr(k), k.stride(0), _ptr(v), v.stride(0), _ptr(out), out.stride(0), B, heads, Nq,
+                                       Nkv, hd, scale, _stream_ptr(q.device))
     _native.check(rc, "sv_op_attention")
-    return o
+    return out
 
 
 def gauss5x5(x: torch.Tensor) -> torch.Tensor:

@@ -181,10 +181,21 @@ int sv_op_dwconv3x3_gelu(const uint16_t* x, const float* w, const float* bias, i
                          int32_t C, uint16_t* out, void* stream);
 
 /* softmax(Q K^T * scale) V per (frame, head). Q rows = B*Nq, K/V rows = B*Nkv; head h occupies columns
- * [h*hd, (h+1)*hd) of each; hd in {32, 40, 64} (mix_transformer_evp.py:123-127, 868-883). */
+ * [h*hd, (h+1)*hd) of each; hd in {20, 32, 40, 64} (mix_transformer_evp.py:123-127, 868-883).  ldq, ldk, ldv % 8 == 0 and
+ * q, k, v 16-byte aligned; ldo even and o 4-byte aligned; only the [B*Nq, heads*hd] block of o is written. */
 int sv_op_attention(const uint16_t* q, int64_t ldq, const uint16_t* k, int64_t ldk, const uint16_t* v, int64_t ldv,
                     uint16_t* o, int64_t ldo, int32_t B, int32_t heads, int32_t Nq, int32_t Nkv, int32_t hd, float scale,
                     void* stream);
+
+/* Which kernel sv_op_attention runs for these operands (it depends on pointer alignment, leading dims, N_kv, hd and the
+ * SURGVID_ATTN_TC switch, not on B, heads or Nq): one of SV_ATTN_*.  Host only; nothing is read through the pointers. */
+#define SV_ATTN_TC_SINGLE 0      /* attention_tc_single_kernel: tcgen05, hd 64, N_kv <= 64 */
+#define SV_ATTN_TC_MULTI 1       /* attention_tc_kernel<true>: tcgen05, hd 64, 64 < N_kv <= 448 */
+#define SV_ATTN_RESIDENT 2       /* attention_resident_kv_kernel: mma.sync, N_kv <= 64 */
+#define SV_ATTN_RESIDENT_MULTI 3 /* attention_resident_multi_kernel: mma.sync, N_kv <= 256 */
+#define SV_ATTN_STREAM 4         /* attention_kernel: mma.sync, streamed key tiles, online softmax */
+int sv_op_attention_kernel(const uint16_t* q, int64_t ldq, const uint16_t* k, int64_t ldk, const uint16_t* v, int64_t ldv,
+                           const uint16_t* o, int64_t ldo, int32_t Nkv, int32_t hd);
 
 /* reflect-pad-2 + 5x5 binomial/256 depthwise filter on fp32 NCHW (mix_transformer_evp.py:500-514). */
 int sv_op_gauss5x5(const float* x, float* out, int32_t planes, int32_t H, int32_t W, void* stream);

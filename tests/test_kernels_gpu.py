@@ -7,6 +7,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+import attn_ref
 import surgvid_b200  # noqa: F401
 from surgvid_b200 import ops
 
@@ -150,13 +151,8 @@ def test_attention(cfg):
     kv = _rand((B * Nkv, 2 * C), 51, dtype=torch.bfloat16)
     scale = hd ** -0.5
     o = ops.attention(q, kv[:, :C], kv[:, C:], B, heads, hd, scale)
-    torch.cuda.synchronize()
-    qf = q.float().view(B, Nq, heads, hd).transpose(1, 2)
-    kf = kv[:, :C].float().view(B, Nkv, heads, hd).transpose(1, 2)
-    vf = kv[:, C:].float().view(B, Nkv, heads, hd).transpose(1, 2)
-    ref = ((qf @ kf.transpose(-1, -2)) * scale).softmax(-1) @ vf
-    ref = ref.transpose(1, 2).reshape(B * Nq, C)
-    assert (o.float() - ref).abs().max().item() < 3e-2
+    ref = attn_ref.reference(q, kv[:, :C], kv[:, C:], B, heads, hd, scale)
+    attn_ref.assert_gate(o, ref, heads, hd, Nq, str(cfg))
 
 
 def test_gauss5x5():
