@@ -30,6 +30,8 @@ EXPORTED_SYMBOLS = [
     "sv_op_bilinear_tokens", "sv_op_token_mean", "sv_op_stem_conv", "sv_op_mixffn_fc2", "sv_op_gemm_bf16_cat",
     "sv_prep_create", "sv_prep_destroy", "sv_prep_workspace_bytes", "sv_prep_images", "sv_prep_flow",
     "sv_trans_create", "sv_trans_destroy", "sv_trans_set_tensor", "sv_trans_pack_weights", "sv_trans_forward",
+    "sv_mstcn_stream_state_bytes", "sv_mstcn_stream_workspace_bytes", "sv_mstcn_stream_reset", "sv_mstcn_stream_step",
+    "sv_trans_stream_state_bytes", "sv_trans_stream_reset", "sv_trans_stream_forward",
 ]
 
 
@@ -141,6 +143,19 @@ def _declare(lib):
     lib.sv_trans_set_tensor.argtypes = [c_void_p, c_char_p, c_void_p, i64p, c_int32]
     lib.sv_trans_pack_weights.argtypes = [c_void_p]
     lib.sv_trans_forward.argtypes = [c_void_p, c_void_p, c_int64, c_void_p, i64p, c_int32, c_void_p, c_void_p]
+    i32p = POINTER(c_int32)
+    lib.sv_mstcn_stream_state_bytes.argtypes = [c_void_p, c_int32]
+    lib.sv_mstcn_stream_state_bytes.restype = c_size_t
+    lib.sv_mstcn_stream_workspace_bytes.argtypes = [c_void_p, c_int64]
+    lib.sv_mstcn_stream_workspace_bytes.restype = c_size_t
+    lib.sv_mstcn_stream_reset.argtypes = [c_void_p, c_void_p, c_size_t, c_int32, i32p, c_int32, c_void_p]
+    lib.sv_mstcn_stream_step.argtypes = [c_void_p, c_void_p, c_size_t, c_int32, c_void_p, i32p, i64p, c_int32, c_void_p, c_void_p, c_void_p,
+                                         c_size_t, c_void_p]
+    lib.sv_trans_stream_state_bytes.argtypes = [c_void_p, c_int32]
+    lib.sv_trans_stream_state_bytes.restype = c_size_t
+    lib.sv_trans_stream_reset.argtypes = [c_void_p, c_void_p, c_size_t, c_int32, i32p, c_int32, c_void_p]
+    lib.sv_trans_stream_forward.argtypes = [c_void_p, c_void_p, c_size_t, c_int32, c_void_p, c_int64, c_void_p, i32p, i64p, c_int32, c_void_p,
+                                            c_void_p]
     lib.sv_prep_create.argtypes = [c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, f32p, f32p, POINTER(c_void_p)]
     lib.sv_prep_destroy.argtypes = [c_void_p]
     lib.sv_prep_workspace_bytes.argtypes = [c_void_p, c_int32]
@@ -150,7 +165,8 @@ def _declare(lib):
     for name in EXPORTED_SYMBOLS:
         fn = getattr(lib, name)
         if name not in ("sv_last_error", "sv_evp_workspace_bytes", "sv_mstcn_workspace_bytes", "sv_evp_last_launch_count",
-                        "sv_mstcn_last_launch_count", "sv_prep_workspace_bytes"):
+                        "sv_mstcn_last_launch_count", "sv_prep_workspace_bytes", "sv_mstcn_stream_state_bytes",
+                        "sv_mstcn_stream_workspace_bytes", "sv_trans_stream_state_bytes"):
             fn.restype = c_int32
 
 

@@ -137,12 +137,36 @@ __global__ void __launch_bounds__(128) mstcn_inproj_tf32x3_kernel(const float* _
   }
 }
 
+// ---- where a tap row that precedes its video's (or stream chunk's) first row in x comes from.  The layer kernels take one of these
+// as a template parameter; nothing else in them depends on it.
+//   OfflineTaps: x holds whole videos, so such a row is the causal zero padding.
+//   StreamTaps:  x holds one step of a stream (rows seen[s] .. seen[s]+count-1 of stream s); a row at stream position q >= 0 comes
+//                from the layer's ring in the stream state (slot q mod 2d), a row at q < 0 is the zero padding.
+struct OfflineTaps {
+  static constexpr bool kStream = false;
+};
+struct StreamTaps {
+  static constexpr bool kStream = true;
+  const int2* __restrict__ rowmap;   // [T]: (stream, stream position) of every row of x
+  const float* __restrict__ ring;    // this stage's / layer's ring of stream 0; ring rows = 2 * dilation (a power of two)
+  int64_t stream_stride;             // floats from one stream's state to the next
+  int ld;                            // floats per ring row (= F)
+  // the ring row `shift` positions before row tt, or null for the zero padding
+  __device__ __forceinline__ const float* row(int64_t tt, int64_t shift, int dilation) const {
+    const int2 m = rowmap[tt];
+    const int64_t q = static_cast<int64_t>(m.y) - shift;
+    if (q < 0) return nullptr;
+    return ring + m.x * stream_stride + (q & (2 * dilation - 1)) * ld;
+  }
+};
+
 // ---- one DilatedResidualLayer for every frame of every video.  One thread = NS consecutive time steps, all F channels
 // (NS = 2 for F = 32: every broadcast weight read from shared memory then feeds two FMAs per output channel).
 // smem: Wd [3][F_in][F_out], W1 [F_in][F_out], bd[F], b1[F] (weights broadcast-read, conflict-free).
-template <int F, int NS>
+template <int F, int NS, class Taps>
 __global__ void __launch_bounds__(128) mstcn_layer_kernel(const float* __restrict__ x, const int* __restrict__ frame_start,
-                                                          const float* __restrict__ wpack, int dilation, int64_t T, float* __restrict__ y) {
+                                                          const float* __restrict__ wpack, int dilation, int64_t T, float* __restrict__ y,
+                                                          const Taps taps) {
   extern __shared__ __align__(16) float sw[];
   constexpr int NW = 3 * F * F + F * F + 2 * F;
   for (int i = threadIdx.x; i < NW / 4; i += blockDim.x) reinterpret_cast<float4*>(sw)[i] = __ldg(reinterpret_cast<const float4*>(wpack) + i);
@@ -168,6 +192,10 @@ __global__ void __launch_bounds__(128) mstcn_layer_kernel(const float* __restric
       const int64_t ts = tt - static_cast<int64_t>(2 - tap) * dilation;
       ok[s] = tt < T && ts >= static_cast<int64_t>(frame_start[tt < T ? tt : T - 1]);  // zero left padding, never across a video boundary
       xp[s] = x + (ok[s] ? ts : 0) * F;
+      if constexpr (Taps::kStream) {
+        const float* hp = (!ok[s] && tt < T) ? taps.row(tt, tt - ts, dilation) : nullptr;
+        if (hp != nullptr) { ok[s] = true; xp[s] = hp; }
+      }
     }
 #pragma unroll
     for (int c4 = 0; c4 < F / 4; ++c4) {
@@ -243,8 +271,9 @@ __global__ void __launch_bounds__(128) mstcn_layer_kernel(const float* __restric
 // The fp32 SIMT kernel below it is bound by broadcast LDS of the weights (20 TFLOP/s); this one by the L2 stream of the activations.
 constexpr int kTcLdW = 40;                                                       // F + 8: conflict-free B fragments
 constexpr int kTcWpack = 2 * (96 * kTcLdW) + 2 * (32 * kTcLdW) + 64;             // Wd hi | Wd lo | W1 hi | W1 lo | bd | b1
+template <class Taps>
 __global__ void __launch_bounds__(128) mstcn_layer_tc_kernel(const float* __restrict__ x, const int* __restrict__ frame_start, const float* __restrict__ wpack,
-                                                             int dilation, int64_t T, float* __restrict__ y, int num_tiles) {
+                                                             int dilation, int64_t T, float* __restrict__ y, int num_tiles, const Taps taps) {
   constexpr int F = 32, BM = 128, LDA = F + 4, LDW = kTcLdW;
   extern __shared__ __align__(16) float sm[];
   float* Xs = sm;                         // [3 taps][BM][LDA]
@@ -267,7 +296,12 @@ __global__ void __launch_bounds__(128) mstcn_layer_tc_kernel(const float* __rest
       const int64_t tt = row0 + r;
       const int64_t ts = tt - static_cast<int64_t>(2 - tap) * dilation;
       const bool ok = tt < T && ts >= static_cast<int64_t>(frame_start[tt < T ? tt : T - 1]);   // zero left padding, never across a video boundary
-      cp_async_16(Xs + (tap * BM + r) * LDA + c4 * 4, ok ? x + ts * F + c4 * 4 : x, ok);
+      if constexpr (Taps::kStream) {
+        const float* hp = (!ok && tt < T) ? taps.row(tt, tt - ts, dilation) : nullptr;
+        cp_async_16(Xs + (tap * BM + r) * LDA + c4 * 4, ok ? x + ts * F + c4 * 4 : (hp != nullptr ? hp + c4 * 4 : x), ok || hp != nullptr);
+      } else {
+        cp_async_16(Xs + (tap * BM + r) * LDA + c4 * 4, ok ? x + ts * F + c4 * 4 : x, ok);
+      }
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
     asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -441,6 +475,54 @@ __global__ void frame_start_kernel(const int64_t* __restrict__ offsets, int n_vi
   frame_start[t] = static_cast<int>(offsets[lo]);
 }
 
+// ---- stream steps.  `tab` = the step's host tables: row offsets of the n_ids chunks [n_ids + 1], then their stream ids [n_ids].
+__device__ __forceinline__ int step_chunk(const int64_t* __restrict__ offsets, int n_ids, int64_t t) {
+  int lo = 0, hi = n_ids;  // chunk k with offsets[k] <= t < offsets[k+1]
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (offsets[mid] <= t) lo = mid; else hi = mid;
+  }
+  return lo;
+}
+
+// frame_start_kernel of a step: every row's chunk start (the first row the layer kernels read from x) and (stream, position).
+__global__ void stream_rowmap_kernel(const int64_t* __restrict__ tab, int n_ids, int64_t T, const int64_t* __restrict__ seen,
+                                     int* __restrict__ frame_start, int2* __restrict__ rowmap) {
+  const int64_t t = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (t >= T) return;
+  const int k = step_chunk(tab, n_ids, t);
+  const int s = static_cast<int>(tab[n_ids + 1 + k]);
+  frame_start[t] = static_cast<int>(tab[k]);
+  rowmap[t] = make_int2(s, static_cast<int>(seen[s] + (t - tab[k])));
+}
+
+// After the step: the last min(2 * 2^l, count) input rows of every layer l of every stage go to their ring slots, then seen advances.
+// act holds the layer inputs of the step, buffer g * (layers + 1) + l for stage g, layer l.  No kernel of this step reads a ring
+// after this one starts, so the ring writes cannot race a reader.
+template <int F>
+__global__ void mstcn_stream_commit_kernel(const float* __restrict__ act, int64_t T, int stages, int layers, const int64_t* __restrict__ tab,
+                                           int n_ids, const int2* __restrict__ rowmap, float* __restrict__ rings, int64_t stream_stride,
+                                           int64_t* __restrict__ seen) {
+  const int64_t ring_rows = 2 * ((int64_t{1} << layers) - 1);   // per stage
+  const int64_t total = T * (F / 4);
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int64_t r = i / (F / 4);
+    const int c4 = static_cast<int>(i % (F / 4));
+    const int64_t end = tab[step_chunk(tab, n_ids, r) + 1];
+    const int2 m = rowmap[r];
+    float* ring_s = rings + m.x * stream_stride;
+    for (int g = 0; g < stages; ++g) {
+      for (int l = 0; l < layers; ++l) {
+        const int64_t R = int64_t{2} << l;   // ring rows of layer l; its ring starts R - 2 rows into the stage's rings
+        if (end - r > R) continue;
+        const float4 v = __ldg(reinterpret_cast<const float4*>(act + ((static_cast<int64_t>(g) * (layers + 1) + l) * T + r) * F) + c4);
+        reinterpret_cast<float4*>(ring_s + (g * ring_rows + R - 2 + (m.y & (R - 1))) * F)[c4] = v;
+      }
+    }
+    if (r == end - 1 && c4 == 0) seen[m.x] = static_cast<int64_t>(m.y) + 1;
+  }
+}
+
 struct HostTensor {
   std::vector<float> data;
   std::vector<int64_t> shape;
@@ -460,6 +542,9 @@ struct sv_mstcn {
   std::vector<Stage> stages;
   int q_out = 0;  // rows of the optional query head `fc.weight` packed next to the stage-1 projection (0 = absent)
   int64_t launches = 0;
+  // host copy of the frame counters of every stream state reset through this handle, keyed by the state's address: the handle is the
+  // only writer of those counters, and the copy lets a step be refused before launch (unknown state, position past 2^31)
+  std::map<const void*, std::vector<int64_t>> stream_seen;
 };
 
 namespace sv {
@@ -488,55 +573,102 @@ int launch_inproj(sv_mstcn* h, const float* feats, int64_t T, float* out, float*
   return launch_status("mstcn_inproj_tf32x3_kernel");
 }
 
+// What a stream step adds to a forward: the state it reads history from and commits to.
+struct StreamStep {
+  const int64_t* tab;   // device copy of the step's tables (see stream_rowmap_kernel)
+  int n_ids;
+  int64_t* seen;        // state: [n_streams] frame counters
+  float* rings;         // state: rings of stream 0
+  int64_t stream_stride;
+};
+
+// Stream-state layout (documented in surgvid.h): int64 seen[n_streams], padded to 256 B, then per stream, per stage, per layer l a ring
+// of 2 * 2^l rows x f_maps floats (ring of layer l starts 2 * (2^l - 1) rows into the stage's 2 * (2^layers - 1) rows).
+size_t stream_seen_bytes(int32_t n_streams) { return (static_cast<size_t>(n_streams) * sizeof(int64_t) + 255) & ~static_cast<size_t>(255); }
+int64_t stream_ring_rows(const sv_mstcn_cfg& c) { return 2 * ((int64_t{1} << c.layers) - 1); }   // per stage
+int64_t stream_stride_floats(const sv_mstcn_cfg& c) { return c.stages * stream_ring_rows(c) * c.f_maps; }
+
+template <int F, int NS, class Taps>
+int launch_layer(bool tc, int tc_grid, int tc_tiles, size_t tc_smem, unsigned lb, size_t layer_smem, const float* x, const int* frame_start,
+                 const float* w, const float* w_tc, int dilation, int64_t T, float* y, const Taps& taps, cudaStream_t st) {
+  if (tc) {
+    mstcn_layer_tc_kernel<Taps><<<tc_grid, 128, tc_smem, st>>>(x, frame_start, w_tc, dilation, T, y, tc_tiles, taps);
+    return launch_status("mstcn_layer_tc_kernel");
+  }
+  mstcn_layer_kernel<F, NS, Taps><<<lb, 128, layer_smem, st>>>(x, frame_start, w, dilation, T, y, taps);
+  return launch_status("mstcn_layer_kernel");
+}
+
+// The whole-video forward (ss == null) or one stream step (ss != null) over T rows.  Offline, the activations ping-pong between two
+// buffers; a step keeps every layer's input (buffer g * (layers + 1) + l) for the commit at its end.
 template <int F>
 int run_forward(sv_mstcn* h, const float* feats, const int64_t* d_offsets, int n_videos, int64_t T, float* logits, float* query, void* ws,
-                cudaStream_t st) {
+                cudaStream_t st, const StreamStep* ss = nullptr) {
   const sv_mstcn_cfg& c = h->cfg;
   char* p = static_cast<char*>(ws);
-  float* bufA = reinterpret_cast<float*>(p);
-  float* bufB = bufA + T * F;
-  int* frame_start = reinterpret_cast<int*>(bufB + T * F);
+  const int64_t n_bufs = ss ? static_cast<int64_t>(c.stages) * (c.layers + 1) : 2;
+  float* act = reinterpret_cast<float*>(p);
+  int* frame_start = reinterpret_cast<int*>(act + n_bufs * T * F);
+  int2* rowmap = reinterpret_cast<int2*>(frame_start + ((T + 1) & ~int64_t{1}));
+  auto buf = [&](int64_t i) { return act + (ss ? i : (i & 1)) * T * F; };
   const unsigned tb = static_cast<unsigned>(ceil_div64(T, 128));
-  frame_start_kernel<<<tb, 128, 0, st>>>(d_offsets, n_videos, T, frame_start);
-  SV_TRY(launch_status("frame_start_kernel"));
+  if (ss) {
+    stream_rowmap_kernel<<<tb, 128, 0, st>>>(ss->tab, ss->n_ids, T, ss->seen, frame_start, rowmap);
+    SV_TRY(launch_status("stream_rowmap_kernel"));
+  } else {
+    frame_start_kernel<<<tb, 128, 0, st>>>(d_offsets, n_videos, T, frame_start);
+    SV_TRY(launch_status("frame_start_kernel"));
+  }
   h->launches = 1;
   const float* W = h->d_weights;
   const size_t layer_smem = (3 * F * F + F * F + 2 * F) * sizeof(float);
   constexpr int NS = 1;  // time steps per thread in the layer kernel (NS = 2 measured slower on B200: 167 registers, 92 vs 76 us)
   const unsigned lb = static_cast<unsigned>(ceil_div64(ceil_div64(T, NS), 128));
-  SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(mstcn_layer_kernel<F, NS>), static_cast<int>(layer_smem)));
   static const bool use_tc = [] { const char* e = getenv("SURGVID_MSTCN_TC"); return !(e && atoi(e) == 0); }();   // A/B switch
+  const bool tc = F == 32 && use_tc;
   const size_t tc_smem = (3 * 128 * (32 + 4) + kTcWpack + 4 * 32 * (32 + 4)) * sizeof(float);
   const int tc_tiles = static_cast<int>(ceil_div64(T, 128));
   const int tc_grid = std::min(tc_tiles, 2 * std::max(1, device_sm_count()));
-  if (F == 32 && use_tc) SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(mstcn_layer_tc_kernel), static_cast<int>(tc_smem)));
-  float* cur = bufA;  // current stage input / running activation
-  float* nxt = bufB;
+  if (ss) {
+    SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(mstcn_layer_kernel<F, NS, StreamTaps>), static_cast<int>(layer_smem)));
+    if (tc) SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(mstcn_layer_tc_kernel<StreamTaps>), static_cast<int>(tc_smem)));
+  } else {
+    SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(mstcn_layer_kernel<F, NS, OfflineTaps>), static_cast<int>(layer_smem)));
+    if (tc) SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(mstcn_layer_tc_kernel<OfflineTaps>), static_cast<int>(tc_smem)));
+  }
   for (int s = 0; s < c.stages; ++s) {
     const sv_mstcn::Stage& S = h->stages[s];
+    const int64_t b0 = static_cast<int64_t>(s) * (c.layers + 1);   // this stage's input buffer
     if (s == 0) {
-      if (h->q_out > 0) SV_TRY((launch_inproj<F, kQCols>(h, feats, T, cur, query, st)));
-      else SV_TRY((launch_inproj<F, 0>(h, feats, T, cur, nullptr, st)));
+      if (h->q_out > 0) SV_TRY((launch_inproj<F, kQCols>(h, feats, T, buf(0), query, st)));
+      else SV_TRY((launch_inproj<F, 0>(h, feats, T, buf(0), nullptr, st)));
       ++h->launches;
     }
     for (int l = 0; l < c.layers; ++l) {
-      if (F == 32 && use_tc) {
-        mstcn_layer_tc_kernel<<<tc_grid, 128, tc_smem, st>>>(cur, frame_start, W + S.layer_tc[l], 1 << l, T, nxt, tc_tiles);
-        SV_TRY(launch_status("mstcn_layer_tc_kernel"));
+      const float* w = W + S.layer[l];
+      const float* w_tc = tc ? W + S.layer_tc[l] : nullptr;
+      if (ss) {
+        const StreamTaps taps{rowmap, ss->rings + (s * stream_ring_rows(c) + (int64_t{2} << l) - 2) * F, ss->stream_stride, F};
+        SV_TRY((launch_layer<F, NS>(tc, tc_grid, tc_tiles, tc_smem, lb, layer_smem, buf(b0 + l), frame_start, w, w_tc, 1 << l, T, buf(b0 + l + 1), taps, st)));
       } else {
-        mstcn_layer_kernel<F, NS><<<lb, 128, layer_smem, st>>>(cur, frame_start, W + S.layer[l], 1 << l, T, nxt);
-        SV_TRY(launch_status("mstcn_layer_kernel"));
+        SV_TRY((launch_layer<F, NS>(tc, tc_grid, tc_tiles, tc_smem, lb, layer_smem, buf(b0 + l), frame_start, w, w_tc, 1 << l, T, buf(b0 + l + 1),
+                                    OfflineTaps{}, st)));
       }
       ++h->launches;
-      std::swap(cur, nxt);
     }
     const bool last = s == c.stages - 1;
-    // writes this stage's logits; unless last, also softmax + the next stage's conv_1x1 into `nxt`
-    mstcn_out_kernel<F><<<tb, 128, 0, st>>>(cur, W + S.w_out, W + S.b_out, c.out_features, T, logits + static_cast<int64_t>(s) * c.out_features * T,
-                                           last ? nullptr : W + S.w_next, last ? nullptr : W + S.b_next, nxt);
+    // writes this stage's logits; unless last, also softmax + the next stage's conv_1x1 into the next stage's input buffer
+    mstcn_out_kernel<F><<<tb, 128, 0, st>>>(buf(b0 + c.layers), W + S.w_out, W + S.b_out, c.out_features, T,
+                                           logits + static_cast<int64_t>(s) * c.out_features * T, last ? nullptr : W + S.w_next,
+                                           last ? nullptr : W + S.b_next, last ? nullptr : buf(b0 + c.layers + 1));
     SV_TRY(launch_status("mstcn_out_kernel"));
     ++h->launches;
-    std::swap(cur, nxt);
+  }
+  if (ss) {
+    const unsigned cb = static_cast<unsigned>(std::min<int64_t>(ceil_div64(T * (F / 4), 256), static_cast<int64_t>(device_sm_count()) * 8));
+    mstcn_stream_commit_kernel<F><<<cb, 256, 0, st>>>(act, T, c.stages, c.layers, ss->tab, ss->n_ids, rowmap, ss->rings, ss->stream_stride, ss->seen);
+    SV_TRY(launch_status("mstcn_stream_commit_kernel"));
+    ++h->launches;
   }
   return SV_OK;
 }
@@ -735,6 +867,98 @@ int sv_mstcn_forward_query(sv_mstcn_handle* h, const float* feats, const int64_t
   SV_CUDA_OK(cudaMemcpyAsync(d_offsets, video_offsets, (n_videos + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
   if (h->cfg.f_maps == 32) return run_forward<32>(h, feats, d_offsets, n_videos, T, logits, query, workspace, st);
   return run_forward<64>(h, feats, d_offsets, n_videos, T, logits, query, workspace, st);
+}
+
+size_t sv_mstcn_stream_state_bytes(const sv_mstcn_handle* h, int32_t n_streams) {
+  if (!h || n_streams < 1) return 0;
+  return sv::stream_seen_bytes(n_streams) + static_cast<size_t>(n_streams) * sv::stream_stride_floats(h->cfg) * sizeof(float);
+}
+
+size_t sv_mstcn_stream_workspace_bytes(const sv_mstcn_handle* h, int64_t rows) {
+  if (!h || rows <= 0) return 0;
+  const size_t T = static_cast<size_t>(rows), bufs = static_cast<size_t>(h->cfg.stages) * (h->cfg.layers + 1);
+  const size_t rowmap_end = bufs * T * h->cfg.f_maps * sizeof(float) + ((T + 1) & ~size_t{1}) * sizeof(int) + T * sizeof(int2);
+  return rowmap_end + 256 + (2 * T + 1) * sizeof(int64_t);
+}
+
+int sv_mstcn_stream_reset(sv_mstcn_handle* h, void* state, size_t state_bytes, int32_t n_streams, const int32_t* stream_ids, int32_t n_ids,
+                          void* stream) {
+  using namespace sv;
+  SV_CHECK(h && state, "null argument");
+  SV_CHECK(n_streams >= 1, "mstcn stream: n_streams >= 1");
+  SV_CHECK(state_bytes >= sv_mstcn_stream_state_bytes(h, n_streams), "mstcn stream: state too small");
+  SV_CHECK((reinterpret_cast<uintptr_t>(state) & 255) == 0, "mstcn stream: state must be 256-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int64_t* seen = static_cast<int64_t*>(state);
+  if (stream_ids == nullptr) {   // every stream: the whole state, so that no stale ring row is left behind
+    SV_CUDA_OK(cudaMemsetAsync(state, 0, sv_mstcn_stream_state_bytes(h, n_streams), st));
+    h->stream_seen[state].assign(n_streams, 0);
+    return SV_OK;
+  }
+  auto it = h->stream_seen.find(state);
+  if (it == h->stream_seen.end()) return fail(SV_ERR_STATE, "mstcn stream: reset every stream of a new state (stream_ids = NULL) first");
+  SV_CHECK(static_cast<int32_t>(it->second.size()) == n_streams, "mstcn stream: n_streams differs from the state's last full reset");
+  SV_CHECK(n_ids >= 1, "mstcn stream: n_ids >= 1");
+  std::vector<char> hit(n_streams, 0);
+  for (int i = 0; i < n_ids; ++i) {
+    SV_CHECK(stream_ids[i] >= 0 && stream_ids[i] < n_streams, "mstcn stream: stream id out of range");
+    SV_CHECK(!hit[stream_ids[i]], "mstcn stream: duplicate stream id");
+    hit[stream_ids[i]] = 1;
+  }
+  // only the counter: ring rows are read at positions [0, seen) alone, and those are rewritten before they are read again
+  for (int i = 0; i < n_ids; ++i) {
+    SV_CUDA_OK(cudaMemsetAsync(seen + stream_ids[i], 0, sizeof(int64_t), st));
+    it->second[stream_ids[i]] = 0;
+  }
+  return SV_OK;
+}
+
+int sv_mstcn_stream_step(sv_mstcn_handle* h, void* state, size_t state_bytes, int32_t n_streams, const float* feats, const int32_t* stream_ids,
+                         const int64_t* counts, int32_t n_ids, float* logits, float* query, void* workspace, size_t workspace_bytes, void* stream) {
+  using namespace sv;
+  SV_CHECK(h && state && feats && stream_ids && counts && logits && workspace, "null argument");
+  if (!h->packed) return fail(SV_ERR_STATE, "mstcn: pack_weights() has not been called");
+  if (query != nullptr && h->q_out == 0) return fail(SV_ERR_STATE, "mstcn: a query output was requested but no 'fc.weight' tensor was set");
+  SV_CHECK(n_streams >= 1, "mstcn stream: n_streams >= 1");
+  SV_CHECK(state_bytes >= sv_mstcn_stream_state_bytes(h, n_streams), "mstcn stream: state too small");
+  auto it = h->stream_seen.find(state);
+  if (it == h->stream_seen.end()) return fail(SV_ERR_STATE, "mstcn stream: the state was not reset through this handle (reset every stream first)");
+  SV_CHECK(static_cast<int32_t>(it->second.size()) == n_streams, "mstcn stream: n_streams differs from the state's last full reset");
+  SV_CHECK(n_ids >= 1 && n_ids <= n_streams, "mstcn stream: 1 <= n_ids <= n_streams");
+  std::vector<int64_t> tab(2 * static_cast<size_t>(n_ids) + 1);   // chunk row offsets [n_ids + 1], then stream ids [n_ids]
+  std::vector<char> hit(n_streams, 0);
+  for (int i = 0; i < n_ids; ++i) {
+    const int32_t s = stream_ids[i];
+    SV_CHECK(s >= 0 && s < n_streams, "mstcn stream: stream id out of range");
+    SV_CHECK(!hit[s], "mstcn stream: duplicate stream id");
+    hit[s] = 1;
+    SV_CHECK(counts[i] >= 1, "mstcn stream: counts must be >= 1");
+    SV_CHECK(counts[i] < (1LL << 31) - it->second[s], "mstcn stream: a stream position would pass 2^31");
+    tab[i + 1] = tab[i] + counts[i];
+    SV_CHECK(tab[i + 1] < (1LL << 31), "mstcn stream: too many rows in one step");
+    tab[n_ids + 1 + i] = s;
+  }
+  const int64_t T = tab[n_ids];
+  SV_CHECK(workspace_bytes >= sv_mstcn_stream_workspace_bytes(h, T), "mstcn stream: workspace too small");
+  SV_CHECK((reinterpret_cast<uintptr_t>(feats) & 15) == 0 && (reinterpret_cast<uintptr_t>(workspace) & 255) == 0 &&
+               (reinterpret_cast<uintptr_t>(state) & 255) == 0, "mstcn stream: alignment (feats 16 B, workspace and state 256 B)");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t bufs = static_cast<size_t>(h->cfg.stages) * (h->cfg.layers + 1);
+  char* tail = static_cast<char*>(workspace) + bufs * T * h->cfg.f_maps * sizeof(float) + ((T + 1) & ~int64_t{1}) * sizeof(int) + T * sizeof(int2);
+  tail = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(tail) + 255) & ~static_cast<uintptr_t>(255));
+  int64_t* d_tab = reinterpret_cast<int64_t*>(tail);
+  SV_CUDA_OK(cudaMemcpyAsync(d_tab, tab.data(), tab.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  StreamStep ss;
+  ss.tab = d_tab;
+  ss.n_ids = n_ids;
+  ss.seen = static_cast<int64_t*>(state);
+  ss.rings = reinterpret_cast<float*>(static_cast<char*>(state) + stream_seen_bytes(n_streams));
+  ss.stream_stride = stream_stride_floats(h->cfg);
+  const int rc = h->cfg.f_maps == 32 ? run_forward<32>(h, feats, nullptr, 0, T, logits, query, workspace, st, &ss)
+                                     : run_forward<64>(h, feats, nullptr, 0, T, logits, query, workspace, st, &ss);
+  if (rc != SV_OK) return rc;
+  for (int i = 0; i < n_ids; ++i) it->second[stream_ids[i]] += counts[i];
+  return SV_OK;
 }
 
 int sv_op_causal_windows(const float* x, int64_t ldx, int32_t C, const int64_t* video_offsets, int32_t n_videos, int32_t len_q, float* out,

@@ -59,9 +59,24 @@ constexpr int kGroups = 2;                                       // 128-thread g
 constexpr int kGroupFloats = 3 * kLMax * kLdS + 3 * kLMax * kDP + kDP;   // per-group tiles
 __device__ __forceinline__ void group_sync(int grp) { asm volatile("bar.sync %0, 128;" ::"r"(grp + 1) : "memory"); }
 
+// Where a window row that precedes its video's (or stream chunk's) first frame in `logits` comes from.
+//   OfflineWindow: logits hold whole videos, so such a row is the zero left padding.
+//   StreamWindow:  logits hold one step of the streams (chunk k = stream ids[k], frames seen[s] .. seen[s]+count-1); a row at stream
+//                  position q >= 0 comes from the stream's ring of the last len_q - 1 logits rows (slot q mod (len_q - 1)), q < 0 is zero.
+struct OfflineWindow {
+  static constexpr bool kStream = false;
+};
+struct StreamWindow {
+  static constexpr bool kStream = true;
+  const int64_t* __restrict__ ids;     // [n_ids] stream of each chunk
+  const int64_t* __restrict__ seen;    // [n_streams]
+  const float* __restrict__ ring;      // [n_streams][len_q - 1][D]
+};
+
+template <class Window>
 __global__ void __launch_bounds__(128 * kGroups) trans_head_kernel(const float* __restrict__ logits, int64_t ldx, const float* __restrict__ query,
                                                          const int64_t* __restrict__ offsets, int64_t T, const float* __restrict__ blob,
-                                                         float* __restrict__ out, const TransParams p) {
+                                                         float* __restrict__ out, const TransParams p, const Window win) {
   extern __shared__ __align__(16) float sm[];
   float* Wb = sm;                              // kBlobSize
   const int grp = threadIdx.x >> 7;
@@ -90,10 +105,22 @@ __global__ void __launch_bounds__(128 * kGroups) trans_head_kernel(const float* 
     }
     const int64_t start = offsets[lo];
     // ---- (1) window X [L, D] and the decoder query
-    for (int idx = tid; idx < L * kDP; idx += 128) {
-      const int i = idx / kDP, c = idx % kDP;
-      const int64_t src = t - (L - 1) + i;
-      Xs[idx] = (c < D && src >= start) ? __ldg(logits + static_cast<int64_t>(c) * ldx + src) : 0.f;
+    if constexpr (Window::kStream) {
+      const int64_t s = win.ids[lo], pos = win.seen[s] + (t - start);   // stream position of frame t
+      for (int idx = tid; idx < L * kDP; idx += 128) {
+        const int i = idx / kDP, c = idx % kDP;
+        const int64_t src = t - (L - 1) + i, q = pos - (L - 1) + i;
+        float v = 0.f;
+        if (c < D && src >= start) v = __ldg(logits + static_cast<int64_t>(c) * ldx + src);
+        else if (c < D && q >= 0) v = __ldg(win.ring + (s * (L - 1) + q % (L - 1)) * D + c);
+        Xs[idx] = v;
+      }
+    } else {
+      for (int idx = tid; idx < L * kDP; idx += 128) {
+        const int i = idx / kDP, c = idx % kDP;
+        const int64_t src = t - (L - 1) + i;
+        Xs[idx] = (c < D && src >= start) ? __ldg(logits + static_cast<int64_t>(c) * ldx + src) : 0.f;
+      }
     }
     if (tid < kDP) qv[tid] = tid < D ? __ldg(query + t * D + tid) : 0.f;
     group_sync(grp);
@@ -260,6 +287,21 @@ __global__ void __launch_bounds__(128 * kGroups) trans_head_kernel(const float* 
   }
 }
 
+// After a stream step: the last min(len_q - 1, count) logits rows of every chunk go to their ring slots, then seen advances.
+// One block per chunk; the block reads seen[s] before its thread 0 advances it.
+__global__ void trans_stream_commit_kernel(const float* __restrict__ logits, int64_t ldx, const int64_t* __restrict__ tab, int n_ids, int D, int L,
+                                           float* __restrict__ ring, int64_t* __restrict__ seen) {
+  const int k = blockIdx.x;
+  const int64_t s = tab[n_ids + 1 + k], r0 = tab[k], cnt = tab[k + 1] - r0, seen0 = seen[s], keep = cnt < L - 1 ? cnt : L - 1;
+  for (int64_t i = threadIdx.x; i < keep * D; i += blockDim.x) {
+    const int64_t j = cnt - keep + i / D;   // row in the chunk
+    const int c = static_cast<int>(i % D);
+    ring[(s * (L - 1) + (seen0 + j) % (L - 1)) * D + c] = __ldg(logits + static_cast<int64_t>(c) * ldx + r0 + j);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) seen[s] = seen0 + cnt;
+}
+
 struct HostTensor {
   std::vector<float> data;
   std::vector<int64_t> shape;
@@ -276,6 +318,8 @@ struct sv_trans {
   float* d_blob = nullptr;
   int64_t* d_offsets = nullptr;
   int offsets_cap = 0;
+  // host copy of the frame counters of every stream state reset through this handle (see sv_mstcn)
+  std::map<const void*, std::vector<int64_t>> stream_seen;
 };
 
 namespace sv {
@@ -392,10 +436,97 @@ int sv_trans_forward(sv_trans_handle* h, const float* logits, int64_t ldx, const
   p.D = h->cfg.d_model; p.L = h->cfg.len_q; p.FF = h->cfg.d_ff; p.n_videos = n_videos;
   p.scale = 1.0f / sqrtf(static_cast<float>(h->cfg.d_k));
   const int smem = (kBlobSize + kGroups * kGroupFloats) * static_cast<int>(sizeof(float));
-  SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(trans_head_kernel), smem));
+  SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(trans_head_kernel<OfflineWindow>), smem));
   const int grid = static_cast<int>(std::min<int64_t>((T + kGroups - 1) / kGroups, std::max(1, device_sm_count())));
-  trans_head_kernel<<<grid, 128 * kGroups, smem, st>>>(logits, ldx, query, h->d_offsets, T, h->d_blob, out, p);
+  trans_head_kernel<OfflineWindow><<<grid, 128 * kGroups, smem, st>>>(logits, ldx, query, h->d_offsets, T, h->d_blob, out, p, OfflineWindow{});
   return launch_status("trans_head_kernel");
+}
+
+size_t sv_trans_stream_state_bytes(const sv_trans_handle* h, int32_t n_streams) {
+  if (!h || n_streams < 1) return 0;
+  const size_t seen = (static_cast<size_t>(n_streams) * sizeof(int64_t) + 255) & ~static_cast<size_t>(255);
+  return seen + static_cast<size_t>(n_streams) * (h->cfg.len_q - 1) * h->cfg.d_model * sizeof(float);
+}
+
+int sv_trans_stream_reset(sv_trans_handle* h, void* state, size_t state_bytes, int32_t n_streams, const int32_t* stream_ids, int32_t n_ids,
+                          void* stream) {
+  using namespace sv;
+  SV_CHECK(h && state, "null argument");
+  SV_CHECK(n_streams >= 1, "trans stream: n_streams >= 1");
+  SV_CHECK(state_bytes >= sv_trans_stream_state_bytes(h, n_streams), "trans stream: state too small");
+  SV_CHECK((reinterpret_cast<uintptr_t>(state) & 255) == 0, "trans stream: state must be 256-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (stream_ids == nullptr) {
+    SV_CUDA_OK(cudaMemsetAsync(state, 0, sv_trans_stream_state_bytes(h, n_streams), st));
+    h->stream_seen[state].assign(n_streams, 0);
+    return SV_OK;
+  }
+  auto it = h->stream_seen.find(state);
+  if (it == h->stream_seen.end()) return fail(SV_ERR_STATE, "trans stream: reset every stream of a new state (stream_ids = NULL) first");
+  SV_CHECK(static_cast<int32_t>(it->second.size()) == n_streams, "trans stream: n_streams differs from the state's last full reset");
+  SV_CHECK(n_ids >= 1, "trans stream: n_ids >= 1");
+  std::vector<char> hit(n_streams, 0);
+  for (int i = 0; i < n_ids; ++i) {
+    SV_CHECK(stream_ids[i] >= 0 && stream_ids[i] < n_streams, "trans stream: stream id out of range");
+    SV_CHECK(!hit[stream_ids[i]], "trans stream: duplicate stream id");
+    hit[stream_ids[i]] = 1;
+  }
+  for (int i = 0; i < n_ids; ++i) {   // ring rows are read at positions [0, seen) alone
+    SV_CUDA_OK(cudaMemsetAsync(static_cast<int64_t*>(state) + stream_ids[i], 0, sizeof(int64_t), st));
+    it->second[stream_ids[i]] = 0;
+  }
+  return SV_OK;
+}
+
+int sv_trans_stream_forward(sv_trans_handle* h, void* state, size_t state_bytes, int32_t n_streams, const float* logits, int64_t ldx,
+                            const float* query, const int32_t* stream_ids, const int64_t* counts, int32_t n_ids, float* out, void* stream) {
+  using namespace sv;
+  SV_CHECK(h && state && logits && query && stream_ids && counts && out, "null argument");
+  if (!h->packed) return fail(SV_ERR_STATE, "trans: pack_weights() has not been called");
+  SV_CHECK(n_streams >= 1, "trans stream: n_streams >= 1");
+  SV_CHECK(state_bytes >= sv_trans_stream_state_bytes(h, n_streams), "trans stream: state too small");
+  SV_CHECK((reinterpret_cast<uintptr_t>(state) & 255) == 0, "trans stream: state must be 256-byte aligned");
+  auto it = h->stream_seen.find(state);
+  if (it == h->stream_seen.end()) return fail(SV_ERR_STATE, "trans stream: the state was not reset through this handle (reset every stream first)");
+  SV_CHECK(static_cast<int32_t>(it->second.size()) == n_streams, "trans stream: n_streams differs from the state's last full reset");
+  SV_CHECK(n_ids >= 1 && n_ids <= n_streams, "trans stream: 1 <= n_ids <= n_streams");
+  std::vector<int64_t> tab(2 * static_cast<size_t>(n_ids) + 1);   // chunk row offsets [n_ids + 1], then stream ids [n_ids]
+  std::vector<char> hit(n_streams, 0);
+  for (int i = 0; i < n_ids; ++i) {
+    const int32_t s = stream_ids[i];
+    SV_CHECK(s >= 0 && s < n_streams, "trans stream: stream id out of range");
+    SV_CHECK(!hit[s], "trans stream: duplicate stream id");
+    hit[s] = 1;
+    SV_CHECK(counts[i] >= 1, "trans stream: counts must be >= 1");
+    SV_CHECK(counts[i] < (1LL << 31) - it->second[s], "trans stream: a stream position would pass 2^31");
+    tab[i + 1] = tab[i] + counts[i];
+    SV_CHECK(tab[i + 1] < (1LL << 31), "trans stream: too many rows in one step");
+    tab[n_ids + 1 + i] = s;
+  }
+  const int64_t T = tab[n_ids];
+  SV_CHECK(ldx >= T, "trans: logits row stride");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (h->offsets_cap < static_cast<int>(tab.size())) {
+    if (h->d_offsets) cudaFree(h->d_offsets);
+    h->offsets_cap = std::max(128, 2 * static_cast<int>(tab.size()));
+    SV_CUDA_OK(cudaMalloc(&h->d_offsets, h->offsets_cap * sizeof(int64_t)));
+  }
+  SV_CUDA_OK(cudaMemcpyAsync(h->d_offsets, tab.data(), tab.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  TransParams p;
+  p.D = h->cfg.d_model; p.L = h->cfg.len_q; p.FF = h->cfg.d_ff; p.n_videos = n_ids;
+  p.scale = 1.0f / sqrtf(static_cast<float>(h->cfg.d_k));
+  int64_t* seen = static_cast<int64_t*>(state);
+  float* ring = reinterpret_cast<float*>(static_cast<char*>(state) + ((static_cast<size_t>(n_streams) * sizeof(int64_t) + 255) & ~static_cast<size_t>(255)));
+  const StreamWindow win{h->d_offsets + n_ids + 1, seen, ring};
+  const int smem = (kBlobSize + kGroups * kGroupFloats) * static_cast<int>(sizeof(float));
+  SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(trans_head_kernel<StreamWindow>), smem));
+  const int grid = static_cast<int>(std::min<int64_t>((T + kGroups - 1) / kGroups, std::max(1, device_sm_count())));
+  trans_head_kernel<StreamWindow><<<grid, 128 * kGroups, smem, st>>>(logits, ldx, query, h->d_offsets, T, h->d_blob, out, p, win);
+  SV_TRY(launch_status("trans_head_kernel"));
+  trans_stream_commit_kernel<<<n_ids, 128, 0, st>>>(logits, ldx, h->d_offsets, n_ids, p.D, p.L, ring, seen);
+  SV_TRY(launch_status("trans_stream_commit_kernel"));
+  for (int i = 0; i < n_ids; ++i) it->second[stream_ids[i]] += counts[i];
+  return SV_OK;
 }
 
 }  // extern "C"

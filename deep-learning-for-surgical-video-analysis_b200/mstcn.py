@@ -171,6 +171,16 @@ class MultiStageModel_S(nn.Module):
         st = self._state(feats.device)
         return torch.ops.surgvid.mstcn_forward_query(feats, offsets, st["id"])
 
+    def open_stream(self, n_streams: int, device=None) -> "MstcnStream":
+        """Online use: `n_streams` independent videos fed a few frames at a time (see `MstcnStream`).  `device` defaults to the
+        model's device, which must be a CUDA device."""
+        if self.training:
+            raise RuntimeError("surgvid_b200 models are inference-only: call model.eval() first (trans_SV_output.py:203)")
+        dev = torch.device(device) if device is not None else next(self.parameters()).device
+        if dev.type != "cuda":
+            raise RuntimeError("surgvid_b200 has no CPU path: open the stream on a CUDA (sm_100a) device")
+        return MstcnStream(self, int(n_streams), dev)
+
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         """x: [B, f_dim, T] -> [stages, B, out_features, T] (mstcn.py:122-130)."""
         self._check(x)
@@ -187,6 +197,99 @@ class MultiStageModel_S(nn.Module):
                 _native.lib().sv_mstcn_destroy(st["handle"])
         except (AttributeError, TypeError, ImportError):
             pass  # interpreter shutdown: module globals are already gone; anything else (a failing destroy) propagates as "ignored exception" text
+
+
+def _step_tables(stream_ids, counts, n_rows: int):
+    ids = np.ascontiguousarray(np.asarray(stream_ids, dtype=np.int64).reshape(-1))
+    cnt = np.ascontiguousarray(np.asarray(counts, dtype=np.int64).reshape(-1))
+    if ids.shape != cnt.shape or ids.size == 0:
+        raise ValueError("stream_ids and counts must be non-empty and of the same length")
+    if int(cnt.sum()) != n_rows:
+        raise ValueError(f"sum(counts) = {int(cnt.sum())} must equal the number of feature rows ({n_rows})")
+    if ids.min() < np.iinfo(np.int32).min or ids.max() > np.iinfo(np.int32).max:
+        raise ValueError("stream id out of range")
+    return np.ascontiguousarray(ids.astype(np.int32)), cnt
+
+
+class MstcnStream:
+    """Per-video state of `n_streams` videos on the GPU for online phase recognition (`MultiStageModel_S.open_stream`).
+
+    `step(feats, stream_ids, counts)` takes new feature rows for some of the streams (rows of stream_ids[k], counts[k] >= 1 of them,
+    grouped in that order) and returns their logits [stages, C, sum(counts)], bit-identical to `forward_videos` over each video's frames
+    so far.  The state holds what the causal layers still need of each video's past (the last 2 * 2^l inputs of layer l), so a step costs
+    the same whatever the history.  The state was computed with the weights of the last reset: after `load_state_dict` or `.to()`,
+    `step` raises until `reset()`."""
+
+    def __init__(self, model: MultiStageModel_S, n_streams: int, device: torch.device):
+        if n_streams < 1:
+            raise ValueError("n_streams >= 1")
+        self._model, self.n_streams = model, n_streams
+        self.device = torch.device("cuda", device.index if device.index is not None else torch.cuda.current_device())
+        lib = _native.lib()
+        st = model._state(self.device)
+        nbytes = int(lib.sv_mstcn_stream_state_bytes(st["handle"], n_streams))
+        self._state = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        self._ws = None
+        self._seen = np.zeros(n_streams, dtype=np.int64)
+        self.reset()
+
+    @property
+    def seen(self) -> torch.Tensor:
+        """Frames each stream has consumed since its last reset (a CPU copy)."""
+        return torch.from_numpy(self._seen.copy())
+
+    def _handle(self):
+        with torch.cuda.device(self.device):
+            return self._model._state(self.device)["handle"]
+
+    def reset(self, ids=None):
+        """Make the next frame of the listed streams (all when ids is None) frame 0 of a new video.  Resetting every stream also adopts
+        the model's current weights."""
+        h = self._handle()
+        cs = ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        lib = _native.lib()
+        if ids is None:
+            _native.check(lib.sv_mstcn_stream_reset(h, ctypes.c_void_p(self._state.data_ptr()), self._state.numel(), self.n_streams, None, 0, cs),
+                          "sv_mstcn_stream_reset")
+            self._seen[:] = 0
+            self._epoch = self._model._weights_epoch
+            return
+        a = np.ascontiguousarray(np.asarray(ids, dtype=np.int32).reshape(-1))
+        _native.check(lib.sv_mstcn_stream_reset(h, ctypes.c_void_p(self._state.data_ptr()), self._state.numel(), self.n_streams,
+                                                a.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), a.size, cs), "sv_mstcn_stream_reset")
+        self._seen[a] = 0
+
+    def step(self, feats: torch.Tensor, stream_ids, counts, query: bool = False):
+        """feats [sum(counts), f_dim] fp32 CUDA -> logits [stages, C, sum(counts)]; with query=True, (logits, query [sum(counts), q])
+        (needs `set_query_head`)."""
+        m = self._model
+        if m._weights_epoch != self._epoch:
+            raise RuntimeError("the model's weights changed since this stream state was computed: call reset() first")
+        m._check(feats)
+        feats = feats.to(torch.float32).contiguous()
+        if feats.dim() != 2 or feats.shape[1] != m.dim:
+            raise ValueError(f"feats must be [rows, {m.dim}], got {tuple(feats.shape)}")
+        n = feats.shape[0]
+        ids, cnt = _step_tables(stream_ids, counts, n)
+        lib = _native.lib()
+        h = self._handle()
+        nbytes = int(lib.sv_mstcn_stream_workspace_bytes(h, n))
+        if self._ws is None or self._ws.numel() < nbytes:
+            self._ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        out = torch.empty((m.num_stages, m.num_classes, n), dtype=torch.float32, device=self.device)
+        q = None
+        if query:
+            if m._fc_weight is None:
+                raise RuntimeError("no query head attached: call set_query_head(fc_weight) first")
+            q = torch.empty((n, m._fc_weight.shape[0]), dtype=torch.float32, device=self.device)
+        rc = lib.sv_mstcn_stream_step(h, ctypes.c_void_p(self._state.data_ptr()), self._state.numel(), self.n_streams, ctypes.c_void_p(feats.data_ptr()),
+                                      ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), ids.size,
+                                      ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(0 if q is None else q.data_ptr()),
+                                      ctypes.c_void_p(self._ws.data_ptr()), self._ws.numel(),
+                                      ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream))
+        _native.check(rc, "sv_mstcn_stream_step")
+        self._seen[ids] += cnt
+        return (out, q) if query else out
 
 
 class _MstcnOpOwner:

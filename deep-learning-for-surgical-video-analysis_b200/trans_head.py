@@ -223,3 +223,65 @@ class Transformer(TransformerInputs):
             self.attach(mstcn_model)
         logits, query = mstcn_model.forward_videos_query(long_feature, lengths)
         return logits, self.transformer.forward_fused(logits[-1], query, lengths)
+
+    def open_stream(self, mstcn_model: MultiStageModel_S, n_streams: int, device=None) -> "TransStream":
+        """Online use of MS-TCN + head for `n_streams` videos (see `TransStream`)."""
+        if self.training or self.transformer.training:
+            raise RuntimeError("surgvid_b200 models are inference-only: call .eval() first")
+        if self._attached_to is not mstcn_model:
+            self.attach(mstcn_model)
+        return TransStream(self, mstcn_model.open_stream(n_streams, device))
+
+
+class TransStream:
+    """`Transformer.open_stream`: an `MstcnStream` plus the head's own state (the last len_q - 1 last-stage logits rows of every stream).
+    `step(feats, stream_ids, counts)` returns (logits [stages, C, n], head_out [n, 1, C]) for the step's rows, bit-identical to
+    `Transformer.forward_videos` over each video's frames so far; `reset(ids)` resets both states together."""
+
+    def __init__(self, head: Transformer, mstcn_stream):
+        self._head, self.mstcn = head, mstcn_stream
+        self.n_streams, self.device = mstcn_stream.n_streams, mstcn_stream.device
+        nbytes = int(_native.lib().sv_trans_stream_state_bytes(self._handle(), self.n_streams))
+        self._state = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        self.reset()
+
+    @property
+    def seen(self) -> torch.Tensor:
+        return self.mstcn.seen
+
+    def _handle(self):
+        with torch.cuda.device(self.device):
+            return self._head.transformer._state(self.device)["handle"]
+
+    def reset(self, ids=None):
+        self.mstcn.reset(ids)
+        cs = ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        lib = _native.lib()
+        if ids is None:
+            _native.check(lib.sv_trans_stream_reset(self._handle(), ctypes.c_void_p(self._state.data_ptr()), self._state.numel(), self.n_streams,
+                                                    None, 0, cs), "sv_trans_stream_reset")
+            self._epoch = self._head.transformer._weights_epoch
+            return
+        a = np.ascontiguousarray(np.asarray(ids, dtype=np.int32).reshape(-1))
+        _native.check(lib.sv_trans_stream_reset(self._handle(), ctypes.c_void_p(self._state.data_ptr()), self._state.numel(), self.n_streams,
+                                                a.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), a.size, cs), "sv_trans_stream_reset")
+
+    @torch.no_grad()
+    def step(self, feats: torch.Tensor, stream_ids, counts):
+        if self._head.transformer._weights_epoch != self._epoch:
+            raise RuntimeError("the head's weights changed since this stream state was computed: call reset() first")
+        if self._head._attached_to is not self.mstcn._model:
+            raise RuntimeError("the head's query projection was attached to another MS-TCN model: open a new stream")
+        logits, query = self.mstcn.step(feats, stream_ids, counts, query=True)
+        n = logits.shape[2]
+        ids = np.ascontiguousarray(np.asarray(stream_ids, dtype=np.int32).reshape(-1))
+        cnt = np.ascontiguousarray(np.asarray(counts, dtype=np.int64).reshape(-1))
+        out = torch.empty((n, self._head.num_classes), dtype=torch.float32, device=self.device)
+        last = logits[-1]
+        rc = _native.lib().sv_trans_stream_forward(self._handle(), ctypes.c_void_p(self._state.data_ptr()), self._state.numel(), self.n_streams,
+                                                   ctypes.c_void_p(last.data_ptr()), last.stride(0), ctypes.c_void_p(query.data_ptr()),
+                                                   ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), cnt.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
+                                                   ids.size, ctypes.c_void_p(out.data_ptr()),
+                                                   ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream))
+        _native.check(rc, "sv_trans_stream_forward")
+        return logits, out.unsqueeze(1)

@@ -153,6 +153,27 @@ int sv_mstcn_forward_query(sv_mstcn_handle* h, const float* feats, const int64_t
 int sv_op_causal_windows(const float* x, int64_t ldx, int32_t C, const int64_t* video_offsets, int32_t n_videos, int32_t len_q,
                          float* out, void* stream);
 
+/* Online use: n_streams independent videos fed a few frames at a time, with what the causal layers need of each video's past kept in a
+ * caller-owned device STATE.  Streamed logits (and query) are bit-identical to sv_mstcn_forward_query over the same video's frames.
+ *   State layout (size it with sv_mstcn_stream_state_bytes, zero it with sv_mstcn_stream_reset, 256-byte aligned; nothing else writes it):
+ *     int64 seen[n_streams] (frames each stream has consumed), padded to 256 bytes; then per stream, per stage, per layer l a ring of
+ *     2 * 2^l rows x f_maps fp32 holding that layer's last inputs (position q in slot q mod 2 * 2^l); the ring of layer l starts
+ *     2 * (2^l - 1) rows into the stage's 2 * (2^layers - 1) rows (510 rows, 65 280 B per stage at layers 8, f_maps 32).
+ *   sv_mstcn_stream_reset: stream_ids NULL resets every stream (required once for a new state: the handle keeps a host copy of the
+ *     counters of the states it has reset, which is how a step is checked before launch); otherwise the n_ids listed streams, whose
+ *     next frame then behaves as frame 0 of a new video.
+ *   sv_mstcn_stream_step: feats [sum(counts), f_dim] fp32 device (16-byte aligned), the rows of stream stream_ids[k] (counts[k] >= 1,
+ *     no id twice) grouped in that order; logits [stages, out_features, sum(counts)], query [sum(counts), q] or NULL, as
+ *     sv_mstcn_forward_query.  Then each listed stream's seen advances by its count.  Launches 21 kernels at stages 2, layers 8.
+ *     Workspace: sv_mstcn_stream_workspace_bytes(h, sum(counts)), 256-byte aligned (it keeps every layer's inputs of the step). */
+size_t sv_mstcn_stream_state_bytes(const sv_mstcn_handle* h, int32_t n_streams);
+size_t sv_mstcn_stream_workspace_bytes(const sv_mstcn_handle* h, int64_t rows);
+int sv_mstcn_stream_reset(sv_mstcn_handle* h, void* state, size_t state_bytes, int32_t n_streams, const int32_t* stream_ids,
+                          int32_t n_ids, void* stream);
+int sv_mstcn_stream_step(sv_mstcn_handle* h, void* state, size_t state_bytes, int32_t n_streams, const float* feats,
+                         const int32_t* stream_ids, const int64_t* counts, int32_t n_ids, float* logits, float* query, void* workspace,
+                         size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Single kernels (unit-test surface; the two forwards above are built from exactly these).
  * bf16 tensors are passed as uint16_t*. All pointers are device pointers.
@@ -260,6 +281,17 @@ int sv_trans_pack_weights(sv_trans_handle* h);
  * the left and never cross a video boundary. */
 int sv_trans_forward(sv_trans_handle* h, const float* logits, int64_t ldx, const float* query, const int64_t* video_offsets,
                      int32_t n_videos, float* out, void* stream);
+/* Online use, the counterpart of sv_mstcn_stream_step: the head of the frames of one step, bit-identical to sv_trans_forward over the
+ * same video's frames.  State (sv_trans_stream_state_bytes, zeroed by sv_trans_stream_reset, 256-byte aligned): int64 seen[n_streams]
+ * padded to 256 bytes, then per stream a ring of len_q - 1 rows x d_model fp32 of the last logits rows (position q in slot
+ * q mod (len_q - 1)).  Reset works as sv_mstcn_stream_reset.  logits [d_model][ldx] = the last stage of the step's logits, query
+ * [sum(counts), d_model], out [sum(counts), d_model]; stream_ids / counts as in sv_mstcn_stream_step.  Only the step's frames are
+ * computed; two launches (head, ring commit). */
+size_t sv_trans_stream_state_bytes(const sv_trans_handle* h, int32_t n_streams);
+int sv_trans_stream_reset(sv_trans_handle* h, void* state, size_t state_bytes, int32_t n_streams, const int32_t* stream_ids,
+                          int32_t n_ids, void* stream);
+int sv_trans_stream_forward(sv_trans_handle* h, void* state, size_t state_bytes, int32_t n_streams, const float* logits, int64_t ldx,
+                            const float* query, const int32_t* stream_ids, const int64_t* counts, int32_t n_ids, float* out, void* stream);
 
 /* ---- on-GPU input transforms (SURVEY.md 8f-2): the reference's per-frame dataset transforms, applied to device copies of
  * the raw uint8 frames / float32 RAFT flow instead of on the CPU inside CholecFlowDataset.__getitem__ (data_process.py:409-483).
