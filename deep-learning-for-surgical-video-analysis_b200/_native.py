@@ -16,7 +16,7 @@ CSRC_DIR = os.path.join(_PKG_DIR, "csrc")
 # SURGVID_LIB: load another build of the same native library (same-box A/B of two builds); never a non-native path
 LIB_PATH = os.environ.get("SURGVID_LIB") or os.path.join(_PKG_DIR, "lib", "libsurgvid.so")
 INCLUDE_DIR = os.path.join(os.path.dirname(_PKG_DIR), "include")
-SOURCES = ["api.cu", "gemm_tcgen05.cu", "elementwise.cu", "attention.cu", "attention_tc.cu", "dwconv_tma.cu", "stem.cu", "mixffn.cu", "mstcn.cu", "trans_head.cu", "evp.cu", "preprocess.cu"]
+SOURCES = ["api.cu", "gemm_tcgen05.cu", "elementwise.cu", "attention.cu", "attention_tc.cu", "attention_probs.cu", "dwconv_tma.cu", "stem.cu", "mixffn.cu", "mstcn.cu", "trans_head.cu", "evp.cu", "preprocess.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
 
 SV_OK = 0
@@ -32,6 +32,7 @@ EXPORTED_SYMBOLS = [
     "sv_trans_create", "sv_trans_destroy", "sv_trans_set_tensor", "sv_trans_pack_weights", "sv_trans_forward",
     "sv_mstcn_stream_state_bytes", "sv_mstcn_stream_workspace_bytes", "sv_mstcn_stream_reset", "sv_mstcn_stream_step",
     "sv_trans_stream_state_bytes", "sv_trans_stream_reset", "sv_trans_stream_forward",
+    "sv_evp_attention_maps_layout", "sv_evp_forward_attention", "sv_op_attention_probs",
 ]
 
 
@@ -156,6 +157,11 @@ def _declare(lib):
     lib.sv_trans_stream_reset.argtypes = [c_void_p, c_void_p, c_size_t, c_int32, i32p, c_int32, c_void_p]
     lib.sv_trans_stream_forward.argtypes = [c_void_p, c_void_p, c_size_t, c_int32, c_void_p, c_int64, c_void_p, i32p, i64p, c_int32, c_void_p,
                                             c_void_p]
+    lib.sv_evp_attention_maps_layout.argtypes = [POINTER(EvpCfg), c_int32, c_int32, c_int32, i64p, i32p, c_int32, i32p]
+    lib.sv_evp_forward_attention.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32,
+                                             c_int32, c_void_p, c_size_t, c_void_p]
+    lib.sv_op_attention_probs.argtypes = [c_void_p, c_int64, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_int32, c_float, c_void_p,
+                                          c_void_p]
     lib.sv_prep_create.argtypes = [c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, f32p, f32p, POINTER(c_void_p)]
     lib.sv_prep_destroy.argtypes = [c_void_p]
     lib.sv_prep_workspace_bytes.argtypes = [c_void_p, c_int32]

@@ -67,6 +67,7 @@ struct Op {
   bool dw_tma = false;
   AttnTcPlan attn_tc;
   bool attn_tc_on = false;
+  bool probs = false;  // OP_ATTN that writes the attention maps of encoder block i[5] (capture plans only)
   // generic arguments (meaning depends on kind)
   const void* src = nullptr;
   const void* src2 = nullptr;
@@ -433,6 +434,27 @@ void stage_geometry(const sv_evp_cfg& c, int H, int W, StageGeom (&g)[4]) {
   }
 }
 
+// Where each encoder block's attention maps [B, heads, N, N_kv] (fp32) go in one buffer, in call order (stage 1 blocks first).
+// off has n_blocks + 1 entries (element offsets; the last is the total), dims 3 per block.
+int maps_layout(const sv_evp_cfg& c, int B, int H, int W, std::vector<int64_t>* off, std::vector<int32_t>* dims) {
+  if (B <= 0 || H <= 0 || W <= 0) return fail(SV_ERR_INVALID, "evp: B, H and W must be positive");
+  for (int s = 0; s < 4; ++s)
+    if (c.embed_dims[s] <= 0 || c.num_heads[s] <= 0 || c.depths[s] <= 0 || c.sr_ratios[s] <= 0 || c.embed_dims[s] % c.num_heads[s] != 0)
+      return fail(SV_ERR_INVALID, "evp: bad config (non-positive entry or dim not divisible by heads)");
+  StageGeom g[4];
+  stage_geometry(c, H, W, g);
+  for (int s = 0; s < 4; ++s)
+    if (g[s].H < 1 || g[s].W < 1 || g[s].Hk < 1 || g[s].Wk < 1) return fail(SV_ERR_INVALID, "evp: input too small for the 4-stage pyramid");
+  off->assign(1, 0);
+  dims->clear();
+  for (int s = 0; s < 4; ++s)
+    for (int i = 0; i < c.depths[s]; ++i) {
+      off->push_back(off->back() + static_cast<int64_t>(B) * g[s].heads * g[s].N * g[s].Nkv);
+      dims->insert(dims->end(), {g[s].heads, g[s].N, g[s].Nkv});
+    }
+  return SV_OK;
+}
+
 // --------------------------------------------------------------------------------------------- plan building
 struct Builder {
   sv_evp* h;
@@ -509,6 +531,13 @@ struct Builder {
     }
     push(op);
   }
+  // P = softmax(Q K^T * scale) of encoder block `block` into the caller's maps buffer (resolved per call, see run_plan)
+  void probs(const bf16* q, int64_t ldq, const bf16* k, int64_t ldk, int B, int heads, int Nq, int Nkv, int hd, int block) {
+    Op op; op.kind = OP_ATTN; op.probs = true; op.src = q; op.src2 = k; op.l0 = ldq; op.l1 = ldk;
+    op.i[0] = B; op.i[1] = heads; op.i[2] = Nq; op.i[3] = Nkv; op.i[4] = hd; op.i[5] = block; op.f0 = 1.0f / sqrtf(static_cast<float>(hd));
+    op.alg_bytes = 2.0 * B * heads * hd * (static_cast<double>(Nq) + Nkv) + 4.0 * B * heads * static_cast<double>(Nq) * Nkv;
+    push(op);
+  }
   void gauss(float* out, int planes, int H, int W) {
     Op op; op.kind = OP_GAUSS; op.dst = out; op.i[0] = planes; op.i[1] = H; op.i[2] = W; op.ext_src = EXT_SEG;
     op.alg_bytes = 8.0 * planes * H * W;
@@ -535,7 +564,7 @@ struct Builder {
 };
 
 // Builds (or only sizes, when plan == nullptr) the launch schedule for n frames of HxW.
-int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, size_t* bytes_out) {
+int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, bool capture, size_t* bytes_out) {
   const sv_evp_cfg& c = h->cfg;
   Builder b(h, plan, ws);
   Arena& A = b.arena;
@@ -627,6 +656,7 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
   // ---- 1. encoder stages
   {
     int hh = H, ww = W;
+    int block = 0;  // encoder block index over all stages (capture plans)
     for (int s = 0; s < 4; ++s) {
       const StageGeom& G = g[s];
       const StageW& S = h->st[s];
@@ -665,6 +695,8 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
           b.gemm(xn, C, Bk.kv, M, ACT_NONE, nullptr, 0, kvb, 2 * C, 0);
         }
         b.attn(qb, C, kvb, 2 * C, kvb + C, 2 * C, ob, C, n, G.heads, G.N, G.Nkv, C / G.heads);
+        if (capture) b.probs(qb, C, kvb, 2 * C, n, G.heads, G.N, G.Nkv, C / G.heads, block);
+        ++block;
         b.gemm(ob, C, Bk.proj, M, ACT_NONE, x, C, x, C, 1);
         // MixFFN (:60-67)
         b.ln(x, Bk.n2, 1e-6f, M, nullptr, xn);
@@ -751,7 +783,8 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
   return b.status;
 }
 
-int run_plan(sv_evp* h, const Plan& p, const float* x, const float* seg, const float* flow, float* out, cudaStream_t st) {
+// maps: per encoder block, where this micro-batch's attention maps go (capture plans only)
+int run_plan(sv_evp* h, const Plan& p, const float* x, const float* seg, const float* flow, float* out, float* const* maps, cudaStream_t st) {
   const bool prof = h->profile;
   if (prof) {
     while (h->prof_events.size() < 2 * p.ops.size()) {
@@ -783,6 +816,11 @@ int run_plan(sv_evp* h, const Plan& p, const float* x, const float* seg, const f
         rc = launch_dwconv3x3_gelu(static_cast<const bf16*>(op.src), op.p0, op.p1, op.i[0], op.i[1], op.i[2], op.i[3], static_cast<bf16*>(op.dst), op.l0, st);
         break;
       case OP_ATTN:
+        if (op.probs) {
+          rc = launch_attention_probs(static_cast<const bf16*>(op.src), op.l0, static_cast<const bf16*>(op.src2), op.l1, op.i[0], op.i[1], op.i[2],
+                                      op.i[3], op.i[4], op.f0, maps[op.i[5]], st);
+          break;
+        }
         if (op.attn_tc_on) { rc = attention_tc_launch(op.attn_tc, st); break; }
         rc = launch_attention(static_cast<const bf16*>(op.src), op.l0, static_cast<const bf16*>(op.src2), op.l1, static_cast<const bf16*>(op.src3),
                               op.l2, static_cast<bf16*>(op.dst), op.l3, op.i[0], op.i[1], op.i[2], op.i[3], op.i[4], op.f0, st);
@@ -916,13 +954,19 @@ size_t sv_evp_workspace_bytes(const sv_evp_handle* h, int32_t micro_batch, int32
     }
     return true;
   }();
-  if (sv::build(const_cast<sv_evp*>(h), nullptr, nullptr, micro_batch, H, W, flow_ok, &bytes) != SV_OK) return 0;
+  if (sv::build(const_cast<sv_evp*>(h), nullptr, nullptr, micro_batch, H, W, flow_ok, false, &bytes) != SV_OK) return 0;
   return bytes;
 }
 
-int sv_evp_forward(sv_evp_handle* h, const float* x, const float* seg, const float* flow, float* out_features, int32_t B, int32_t H,
-                   int32_t W, int32_t micro_batch, void* workspace, size_t workspace_bytes, void* stream) {
-  using namespace sv;
+}  // extern "C"
+
+namespace sv {
+namespace {
+// maps == nullptr: the plain forward.  Otherwise the capture plans run, and block k's maps of frames [b0, b0 + n) go to
+// maps + off[k] + b0 * heads_k * N_k * Nkv_k.
+int evp_forward(sv_evp_handle* h, const float* x, const float* seg, const float* flow, float* out_features, float* maps, const std::vector<int64_t>& off,
+                const std::vector<int32_t>& dims, int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace, size_t workspace_bytes,
+                void* stream) {
   SV_CHECK(h && x && seg && out_features && workspace, "null argument");
   if (!h->packed) return fail(SV_ERR_STATE, "evp: pack_weights() has not been called");
   SV_CHECK(B > 0 && micro_batch > 0, "evp: B and micro_batch must be positive");
@@ -932,14 +976,16 @@ int sv_evp_forward(sv_evp_handle* h, const float* x, const float* seg, const flo
   const bool with_flow = flow != nullptr;
   h->launches = 0;
   const int E = h->cfg.embedding_dim;
+  const bool capture = maps != nullptr;
+  std::vector<float*> block_maps(capture ? off.size() - 1 : 0);
   for (int b0 = 0; b0 < B; b0 += micro_batch) {
     const int n = std::min<int>(micro_batch, B - b0);
-    const long long key = (static_cast<long long>(n) << 40) ^ (static_cast<long long>(H) << 24) ^ (static_cast<long long>(W) << 8) ^ (with_flow ? 1 : 0);
+    const long long key = (static_cast<long long>(n) << 40) ^ (static_cast<long long>(H) << 24) ^ (static_cast<long long>(W) << 8) ^ (with_flow ? 1 : 0) ^ (capture ? 2 : 0);
     auto it = h->plans.find(key);
     if (it == h->plans.end() || it->second->ws != workspace) {
       std::unique_ptr<Plan> p(new Plan());
       p->n = n; p->H = H; p->W = W; p->with_flow = with_flow; p->ws = workspace;
-      SV_TRY(build(h, p.get(), workspace, n, H, W, with_flow, &p->need));
+      SV_TRY(build(h, p.get(), workspace, n, H, W, with_flow, capture, &p->need));
       if (it == h->plans.end() && h->plans.size() >= kMaxPlans) {  // evict the least recently used plan (never the one just run)
         auto victim = h->plans.end();
         for (auto jt = h->plans.begin(); jt != h->plans.end(); ++jt)
@@ -955,11 +1001,54 @@ int sv_evp_forward(sv_evp_handle* h, const float* x, const float* seg, const flo
     it->second->last_use = ++h->plan_clock;
     const Plan& plan = *it->second;
     const size_t in_off = static_cast<size_t>(b0) * 3 * H * W;
+    for (size_t k = 0; k < block_maps.size(); ++k)
+      block_maps[k] = maps + off[k] + static_cast<int64_t>(b0) * dims[3 * k] * dims[3 * k + 1] * dims[3 * k + 2];
     SV_TRY(run_plan(h, plan, x + in_off, seg + in_off, with_flow ? flow + static_cast<size_t>(b0) * 2 * H * W : nullptr,
-                    out_features + static_cast<size_t>(b0) * E, st));
+                    out_features + static_cast<size_t>(b0) * E, block_maps.data(), st));
     h->last_plan = it->second.get();
   }
   return SV_OK;
+}
+}  // namespace
+}  // namespace sv
+
+extern "C" {
+
+int sv_evp_forward(sv_evp_handle* h, const float* x, const float* seg, const float* flow, float* out_features, int32_t B, int32_t H,
+                   int32_t W, int32_t micro_batch, void* workspace, size_t workspace_bytes, void* stream) {
+  return sv::evp_forward(h, x, seg, flow, out_features, nullptr, {}, {}, B, H, W, micro_batch, workspace, workspace_bytes, stream);
+}
+
+int sv_evp_attention_maps_layout(const sv_evp_cfg* cfg, int32_t B, int32_t H, int32_t W, int64_t* block_offsets, int32_t* block_dims,
+                                 int32_t max_blocks, int32_t* n_blocks) {
+  using namespace sv;
+  SV_CHECK(cfg && n_blocks, "null argument");
+  std::vector<int64_t> off;
+  std::vector<int32_t> dims;
+  SV_TRY(maps_layout(*cfg, B, H, W, &off, &dims));
+  const int nb = static_cast<int>(off.size()) - 1;
+  *n_blocks = nb;
+  if (!block_offsets && !block_dims) return SV_OK;  // size query
+  SV_CHECK(block_offsets && block_dims, "evp: block_offsets and block_dims must both be given (or both NULL to query n_blocks)");
+  SV_CHECK(max_blocks >= nb, "evp: max_blocks is smaller than n_blocks = sum(depths)");
+  std::copy(off.begin(), off.end(), block_offsets);
+  std::copy(dims.begin(), dims.end(), block_dims);
+  return SV_OK;
+}
+
+int sv_evp_forward_attention(sv_evp_handle* h, const float* x, const float* seg, const float* flow, float* out_features, float* maps,
+                             int64_t maps_elems, int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace, size_t workspace_bytes,
+                             void* stream) {
+  using namespace sv;
+  SV_CHECK(h && maps, "null argument");
+  std::vector<int64_t> off;
+  std::vector<int32_t> dims;
+  SV_TRY(maps_layout(h->cfg, B, H, W, &off, &dims));
+  SV_CHECK((reinterpret_cast<uintptr_t>(maps) & 15) == 0, "evp: maps must be 16-byte aligned");
+  if (maps_elems < off.back())
+    return fail(SV_ERR_INVALID, "evp: maps buffer too small: " + std::to_string(maps_elems) + " elements given, " + std::to_string(off.back()) +
+                                    " needed (sv_evp_attention_maps_layout)");
+  return evp_forward(h, x, seg, flow, out_features, maps, off, dims, B, H, W, micro_batch, workspace, workspace_bytes, stream);
 }
 
 int sv_evp_classify(sv_evp_handle* h, const float* feats, float* y, float* y_ant, int32_t B, void* stream) {

@@ -18,6 +18,9 @@ int launch_token_mean(const float* x, int B, int tokens, int C, float* out, cuda
 int launch_bf16_to_f32(const bf16* x, float* out, int64_t n, cudaStream_t st);
 int launch_attention(const bf16* q, int64_t ldq, const bf16* k, int64_t ldk, const bf16* v, int64_t ldv, bf16* o, int64_t ldo, int B,
                      int heads, int Nq, int Nkv, int hd, float scale, cudaStream_t st);
+// P = softmax(Q K^T * scale) -> fp32 [B, heads, Nq, Nkv] (attention_probs.cu); hd 32 or 64
+int launch_attention_probs(const bf16* q, int64_t ldq, const bf16* k, int64_t ldk, int B, int heads, int Nq, int Nkv, int hd, float scale,
+                           float* p, cudaStream_t st);
 
 // tcgen05/TMEM attention for head_dim 64, N_kv <= 448 (attention_tc.cu); the plan owns the four 3-D tensor maps
 struct AttnTcPlan {

@@ -25,7 +25,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from .. import _native, ops
+from .. import _native, ops, visualizer
 from .segformer_head import SegFormerHead, _Holder
 
 
@@ -235,6 +235,27 @@ class MixVisionTransformerEVP(nn.Module):
         """Call after modifying parameters in place (anything other than load_state_dict / .to()): forces a re-pack."""
         self._weights_epoch = getattr(self, "_weights_epoch", 0) + 1
 
+    def _cfg(self) -> _native.EvpCfg:
+        cfg = _native.EvpCfg()
+        for s in range(4):
+            cfg.embed_dims[s], cfg.num_heads[s] = self.embed_dims[s], self.num_heads[s]
+            cfg.depths[s], cfg.sr_ratios[s] = self.depths[s], self.sr_ratios[s]
+        cfg.mlp_ratio, cfg.embedding_dim, cfg.fold_head = self.mlp_ratio, self.embedding_dim, int(self.fold_head)
+        return cfg
+
+    def attention_maps_layout(self, B: int, H: int, W: int):
+        """Host only: ([n_blocks + 1] element offsets of each encoder block's [B, heads, N, N_kv] fp32 maps in one buffer, the last being
+        the total, [(heads, N, N_kv)] per block), blocks in call order (sv_evp_attention_maps_layout)."""
+        lib = _native.lib()
+        cfg = self._cfg()
+        nb = ctypes.c_int32(0)
+        _native.check(lib.sv_evp_attention_maps_layout(ctypes.byref(cfg), B, H, W, None, None, 0, ctypes.byref(nb)), "sv_evp_attention_maps_layout")
+        off = (ctypes.c_int64 * (nb.value + 1))()
+        dims = (ctypes.c_int32 * (3 * nb.value))()
+        _native.check(lib.sv_evp_attention_maps_layout(ctypes.byref(cfg), B, H, W, off, dims, nb.value, ctypes.byref(nb)),
+                      "sv_evp_attention_maps_layout")
+        return list(off), [tuple(dims[3 * i:3 * i + 3]) for i in range(nb.value)]
+
     def _state(self, device: torch.device):
         """Per-device native handle with packed weights; re-packed after load_state_dict / .to() / refresh_weights()."""
         idx = device.index if device.index is not None else torch.cuda.current_device()
@@ -245,11 +266,7 @@ class MixVisionTransformerEVP(nn.Module):
         lib = _native.lib()
         with torch.cuda.device(idx):
             if st is None:
-                cfg = _native.EvpCfg()
-                for s in range(4):
-                    cfg.embed_dims[s], cfg.num_heads[s] = self.embed_dims[s], self.num_heads[s]
-                    cfg.depths[s], cfg.sr_ratios[s] = self.depths[s], self.sr_ratios[s]
-                cfg.mlp_ratio, cfg.embedding_dim, cfg.fold_head = self.mlp_ratio, self.embedding_dim, int(self.fold_head)
+                cfg = self._cfg()
                 h = ctypes.c_void_p()
                 _native.check(lib.sv_evp_create(ctypes.byref(cfg), ctypes.byref(h)), "sv_evp_create")
                 st = {"handle": h, "workspace": {}, "fold_head": self.fold_head, "id": None}
@@ -266,7 +283,8 @@ class MixVisionTransformerEVP(nn.Module):
             st["id"] = ops.register_handle(_EvpOpOwner(self, idx))
         return st
 
-    def _native_forward(self, idx: int, x, seg, flow, micro_batch):
+    def _native_forward(self, idx: int, x, seg, flow, micro_batch, maps=None):
+        """maps: None, or an fp32 buffer of the layout's total element count (then the capture forward also fills it)."""
         st = self._native[idx]
         lib = _native.lib()
         B, _, H, W = x.shape
@@ -284,10 +302,14 @@ class MixVisionTransformerEVP(nn.Module):
             ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
             st["workspace"][key] = ws
         out = torch.empty((B, self.embedding_dim), dtype=torch.float32, device=x.device)
-        rc = lib.sv_evp_forward(st["handle"], ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(seg.data_ptr()),
-                                ctypes.c_void_p(0 if flow is None else flow.data_ptr()), ctypes.c_void_p(out.data_ptr()), B, H, W, mb,
-                                ctypes.c_void_p(ws.data_ptr()), ws.numel(), ctypes.c_void_p(torch.cuda.current_stream(x.device).cuda_stream))
-        _native.check(rc, "sv_evp_forward")
+        args = (ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(seg.data_ptr()), ctypes.c_void_p(0 if flow is None else flow.data_ptr()),
+                ctypes.c_void_p(out.data_ptr()))
+        tail = (B, H, W, mb, ctypes.c_void_p(ws.data_ptr()), ws.numel(), ctypes.c_void_p(torch.cuda.current_stream(x.device).cuda_stream))
+        if maps is None:
+            _native.check(lib.sv_evp_forward(st["handle"], *args, *tail), "sv_evp_forward")
+        else:
+            _native.check(lib.sv_evp_forward_attention(st["handle"], *args, ctypes.c_void_p(maps.data_ptr()), maps.numel(), *tail),
+                          "sv_evp_forward_attention")
         return out
 
     def last_launch_count(self, device=None) -> int:
@@ -316,7 +338,7 @@ class MixVisionTransformerEVP(nn.Module):
         raise RuntimeError("forward_features is fused into torch.ops.surgvid.evp_lfb_forward; per-stage tensors are available "
                            "through model.read_tap('stage{1..4}_tokens') after a forward")
 
-    def extract_features(self, x, y, flow=None) -> torch.Tensor:
+    def _inputs(self, x, y, flow):
         if self.training:
             raise RuntimeError("surgvid_b200 models are inference-only: call model.eval() first (generate_evp_LFB.py:437)")
         if not x.is_cuda:
@@ -326,11 +348,36 @@ class MixVisionTransformerEVP(nn.Module):
         y = y.reshape(-1, 3, H, W).to(device=x.device, dtype=torch.float32).contiguous()
         if flow is not None:
             flow = flow.reshape(-1, 2, H, W).to(device=x.device, dtype=torch.float32).contiguous()
+        return x, y, flow
+
+    def extract_features(self, x, y, flow=None) -> torch.Tensor:
+        x, y, flow = self._inputs(x, y, flow)
         st = self._state(x.device)
         return torch.ops.surgvid.evp_lfb_forward(x, y, flow, st["id"], self.micro_batch)
 
+    def attention_maps(self, x, y, flow=None):
+        """-> (features [B, E] as `extract_features`, maps): maps is a list of sum(depths) fp32 CUDA tensors [B, heads, N, N_kv], the
+        post-softmax attention of each encoder block in call order (stage 1's blocks first), views into one buffer.  The features are
+        bit-identical to `extract_features` on the same inputs.  Flow cross-attention maps are not captured."""
+        x, y, flow = self._inputs(x, y, flow)
+        B, _, H, W = x.shape
+        off, dims = self.attention_maps_layout(B, H, W)
+        buf = torch.empty(off[-1], dtype=torch.float32, device=x.device)
+        self._state(x.device)
+        idx = x.device.index if x.device.index is not None else torch.cuda.current_device()
+        feats = self._native_forward(idx, x, y, flow, self.micro_batch, maps=buf)
+        maps = [buf[off[i]:off[i + 1]].view(B, *dims[i]) for i in range(len(dims))]
+        return feats, maps
+
     def forward(self, x, y, flow=None, return_features=False):
-        feats = self.extract_features(x, y, flow)
+        caches = visualizer.active_caches()
+        if caches:  # visualizer.get_local.activate(): record what the reference's decorated Attention.forward would
+            feats, maps = self.attention_maps(x, y, flow)
+            arrays = [m.cpu().numpy() for m in maps]
+            for cache in caches:
+                cache.setdefault(visualizer.QUALNAME, []).extend(arrays)
+        else:
+            feats = self.extract_features(x, y, flow)
         if return_features:
             return feats
         return self.head.classify(self, feats)

@@ -194,6 +194,22 @@ def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, B: int, heads: 
     return out
 
 
+def attention_probs(q: torch.Tensor, k: torch.Tensor, B: int, heads: int, Nq: int, Nkv: int, hd: int, scale: float,
+                    out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """softmax(Q K^T * scale) as fp32 [B, heads, Nq, Nkv]: q [B*Nq, >=heads*hd] bf16, k [B*Nkv, >=heads*hd] bf16 (row-strided views
+    allowed, as for `attention`); written into `out` (contiguous fp32) when given."""
+    _require_cuda(q, k, out)
+    assert q.dtype == torch.bfloat16 and k.dtype == torch.bfloat16 and q.stride(1) == 1 and k.stride(1) == 1
+    assert q.shape[0] == B * Nq and k.shape[0] == B * Nkv
+    if out is None:
+        out = torch.empty((B, heads, Nq, Nkv), dtype=torch.float32, device=q.device)
+    assert out.dtype == torch.float32 and tuple(out.shape) == (B, heads, Nq, Nkv) and out.is_contiguous()
+    rc = _native.lib().sv_op_attention_probs(_ptr(q), q.stride(0), _ptr(k), k.stride(0), B, heads, Nq, Nkv, hd, scale, _ptr(out),
+                                             _stream_ptr(q.device))
+    _native.check(rc, "sv_op_attention_probs")
+    return out
+
+
 def gauss5x5(x: torch.Tensor) -> torch.Tensor:
     _require_cuda(x)
     B, C, H, W = x.shape

@@ -85,6 +85,22 @@ int sv_evp_forward(sv_evp_handle* h, const float* x, const float* seg, const flo
                    int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace, size_t workspace_bytes,
                    void* stream);
 
+/* Attention maps of the encoder blocks: the post-softmax P = softmax(Q K^T * head_dim^-0.5) of every block's spatial-reduction
+ * attention (mix_transformer_evp.py:123-125; what the reference's `get_local('attn')` records from Attention.forward), fp32.
+ *   sv_evp_attention_maps_layout: host only (needs no device and no handle, only the config).  *n_blocks = sum(depths).
+ *     block_offsets[n_blocks + 1]: element offsets of block k's [B, heads, N, N_kv] array in one buffer, in call order (stage 1's
+ *     blocks, then stage 2's, ...), the last entry is the total; block_dims[3 * n_blocks]: (heads, N, N_kv) per block.  With both
+ *     arrays NULL only *n_blocks is set; otherwise max_blocks must be >= n_blocks.  Bad config, B, H or W -> SV_ERR_INVALID.
+ *   sv_evp_forward_attention: sv_evp_forward (same arguments, same features bit for bit, same workspace size) that also writes every
+ *     block's maps to `maps` (device, 16-byte aligned, >= block_offsets[n_blocks] fp32 elements, else SV_ERR_INVALID).  It runs its
+ *     own launch plans (one attention_probs_kernel launch after each block's attention); the plans of sv_evp_forward are unchanged.
+ *     Flow cross-attention maps are not captured.  Cost: 6.76 MB per frame for mit_b3_evp at 224x224, 452 MB at 480x854. */
+int sv_evp_attention_maps_layout(const sv_evp_cfg* cfg, int32_t B, int32_t H, int32_t W, int64_t* block_offsets, int32_t* block_dims,
+                                 int32_t max_blocks, int32_t* n_blocks);
+int sv_evp_forward_attention(sv_evp_handle* h, const float* x, const float* seg, const float* flow, float* out_features, float* maps,
+                             int64_t maps_elems, int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace,
+                             size_t workspace_bytes, void* stream);
+
 /* head.fc / head.fc_ant on extracted features (segformer_head.py:101-106,176-179):
  * feats [B,2048] fp32 device -> y [B,7], y_ant [B,7] fp32 device. */
 int sv_evp_classify(sv_evp_handle* h, const float* feats, float* y, float* y_ant, int32_t B, void* stream);
@@ -217,6 +233,12 @@ int sv_op_attention(const uint16_t* q, int64_t ldq, const uint16_t* k, int64_t l
 #define SV_ATTN_STREAM 4         /* attention_kernel: mma.sync, streamed key tiles, online softmax */
 int sv_op_attention_kernel(const uint16_t* q, int64_t ldq, const uint16_t* k, int64_t ldk, const uint16_t* v, int64_t ldv,
                            const uint16_t* o, int64_t ldo, int32_t Nkv, int32_t hd);
+
+/* Attention probabilities p[b, h, i, j] = softmax_j(q_i . k_j * scale), fp32, written to a contiguous [B, heads, Nq, Nkv] array
+ * (64-bit offsets).  q, k as for sv_op_attention (head h = columns [h*hd, (h+1)*hd); ldq, ldk % 8 == 0; q, k 16-byte aligned);
+ * p 4-byte aligned.  hd 32 or 64 (else SV_ERR_UNSUPPORTED); any Nq, Nkv >= 1.  Every row sums to 1 within fp32 rounding. */
+int sv_op_attention_probs(const uint16_t* q, int64_t ldq, const uint16_t* k, int64_t ldk, int32_t B, int32_t heads, int32_t Nq,
+                          int32_t Nkv, int32_t hd, float scale, float* p, void* stream);
 
 /* reflect-pad-2 + 5x5 binomial/256 depthwise filter on fp32 NCHW (mix_transformer_evp.py:500-514). */
 int sv_op_gauss5x5(const float* x, float* out, int32_t planes, int32_t H, int32_t W, void* stream);
