@@ -32,7 +32,7 @@ EXPORTED_SYMBOLS = [
     "sv_trans_create", "sv_trans_destroy", "sv_trans_set_tensor", "sv_trans_pack_weights", "sv_trans_forward",
     "sv_mstcn_stream_state_bytes", "sv_mstcn_stream_workspace_bytes", "sv_mstcn_stream_reset", "sv_mstcn_stream_step",
     "sv_trans_stream_state_bytes", "sv_trans_stream_reset", "sv_trans_stream_forward",
-    "sv_evp_attention_maps_layout", "sv_evp_forward_attention", "sv_op_attention_probs",
+    "sv_evp_attention_maps_layout", "sv_evp_forward_attention", "sv_op_attention_probs", "sv_op_gemm_plan_info",
 ]
 
 
@@ -126,6 +126,7 @@ def _declare(lib):
                                     c_void_p, c_int64, c_int32, c_void_p]
     lib.sv_op_gemm_bf16_cat.argtypes = [c_void_p, c_int64, c_void_p, c_int64, c_int32, c_void_p, c_int64, c_int32, c_int32, c_int32, c_void_p, c_int32,
                                         c_void_p, c_int64, c_void_p, c_int64, c_int32, c_void_p]
+    lib.sv_op_gemm_plan_info.argtypes = [c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, POINTER(c_int32)]
     lib.sv_op_layernorm.argtypes = [c_void_p, c_void_p, c_void_p, c_float, c_int64, c_int32, c_void_p, c_void_p, c_void_p]
     lib.sv_op_im2col.argtypes = [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int64, c_void_p]
     lib.sv_op_dwconv3x3_gelu.argtypes = [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]

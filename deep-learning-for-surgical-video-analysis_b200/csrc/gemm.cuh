@@ -61,6 +61,8 @@ struct GemmPlan {
 };
 
 int gemm_plan(const GemmDesc& d, GemmPlan* plan);
+// the shape-only part of gemm_plan (no device, no driver): fills plan->p except the pointers and act, plan->grid, plan->smem_bytes
+int gemm_plan_shape(int M, int N, int K, int K2, int out_fp32, bool has_residual, int pair_request, int sms, GemmPlan* plan);
 int gemm_launch(const GemmPlan& plan, cudaStream_t stream);
 // pick the UMMA N for a problem (exposed for tests)
 int gemm_pick_block_n(int M, int N, int K, int num_sms, int step = 16);

@@ -635,25 +635,17 @@ int gemm_pick_block_n(int M, int N, int K, int num_sms, int step) {
   return best;
 }
 
-int gemm_plan(const GemmDesc& d, GemmPlan* plan) {
-  SV_CHECK(d.M > 0 && d.N > 0 && d.K > 0, "GEMM dims must be positive");
-  SV_CHECK(d.K % 8 == 0 && d.N % 8 == 0, "GEMM needs K%8==0 and N%8==0");
-  SV_CHECK(d.K2 >= 0 && d.K2 < d.K && (d.K2 == 0 || (d.A2 != nullptr && (d.K - d.K2) % kBlockK == 0 && d.K2 % 8 == 0 && d.lda2 >= d.K2)),
-           "GEMM second A segment: K-K2 must be a multiple of 64, K2 % 8 == 0");
-  SV_CHECK(d.lda >= d.K - d.K2 && d.ldw >= d.K && d.ldc >= d.N, "GEMM leading dimensions too small");
-  SV_CHECK(d.A && d.W && d.out, "GEMM null operand");
-  SV_CHECK((reinterpret_cast<uintptr_t>(d.out) & 15) == 0 && d.ldc % (d.out_fp32 ? 4 : 8) == 0, "GEMM output must be 16B-aligned rows");
-  if (d.residual) SV_CHECK((reinterpret_cast<uintptr_t>(d.residual) & 15) == 0 && d.ldr % 4 == 0 && d.ldr >= d.N, "GEMM residual alignment");
-  if (d.bias) SV_CHECK((reinterpret_cast<uintptr_t>(d.bias) & 15) == 0, "GEMM bias alignment");
-  const int sms = device_sm_count();
-  SV_CHECK(sms > 0, "no CUDA device");
+// Every decision of the plan that depends only on the problem's shape, the SM count and the A/B switches: tile width, pair mode,
+// epilogue form, ring depth, epilogue buffers, tiles and grid.  Host only (no device, no driver); gemm_plan launches by it and
+// sv_op_gemm_plan_info reports it.
+int gemm_plan_shape(int M, int N, int K, int K2, int out_fp32, bool has_residual, int pair_request, int sms, GemmPlan* plan) {
   GemmParams& p = plan->p;
-  p.M = d.M; p.N = d.N; p.K = d.K;
+  p.M = M; p.N = N; p.K = K;
   static const int tma_out_env = getenv("SURGVID_GEMM_TMA_OUT") ? atoi(getenv("SURGVID_GEMM_TMA_OUT")) : 1;   // A/B switch
-  // bf16 result without residual, or fp32 result with / without an fp32 residual (the bf16 + residual combination keeps the transposing epilogue)
-  p.tma_out = ((d.out_fp32 || d.residual == nullptr) && tma_out_env) ? 1 : 0;
-  if (p.tma_out && d.out_fp32 && ((d.ldc * 4) % 16 != 0 || (d.residual && (d.ldr * 4) % 16 != 0))) p.tma_out = 0;
-  p.block_n = gemm_pick_block_n(d.M, d.N, d.K, sms, (p.tma_out && !d.out_fp32) ? 32 : 16);
+  // bf16 result without residual, or fp32 result with / without an fp32 residual (the bf16 + residual combination keeps the transposing
+  // epilogue).  The fp32 TMA maps need 16-byte row strides, which the argument checks (ldc, ldr % 4 == 0) already guarantee.
+  p.tma_out = ((out_fp32 || !has_residual) && tma_out_env) ? 1 : 0;
+  p.block_n = gemm_pick_block_n(M, N, K, sms, (p.tma_out && !out_fp32) ? 32 : 16);
   // CTA-pair mode (cta_group::2): each CTA stages half of the B tile, so the ring holds more k-blocks per byte of shared memory
   // and the L2 -> shared-memory traffic of the weights halves.  Measured on B200 (profiles/r02/gemm_pair_relaxed_arrive.log, after
   // (1) the MMA issue moved to a converged warp + elect.sync and (2) the accumulator hand-back stopped using a .release.cluster
@@ -664,9 +656,9 @@ int gemm_plan(const GemmDesc& d, GemmPlan* plan) {
   // GemmDesc::pair / SURGVID_GEMM_PAIR force it on (1) or off (0).  Results are bit-identical to single-CTA tiles.
   {
     static const int pair_env = getenv("SURGVID_GEMM_PAIR") ? atoi(getenv("SURGVID_GEMM_PAIR")) : -1;
-    const int want = d.pair >= 0 ? d.pair : pair_env;
-    const long long pair_tiles = static_cast<long long>(ceil_div(d.M, 2 * kBlockM)) * ceil_div(d.N, p.block_n);
-    const bool pays = d.K >= 512 || (!d.out_fp32 && d.N >= 320);
+    const int want = pair_request >= 0 ? pair_request : pair_env;
+    const long long pair_tiles = static_cast<long long>(ceil_div(M, 2 * kBlockM)) * ceil_div(N, p.block_n);
+    const bool pays = K >= 512 || (!out_fp32 && N >= 320);
     p.pair = want >= 0 ? (want > 0 ? 1 : 0) : ((pays && pair_tiles >= sms / 2) ? 1 : 0);
   }
   if (p.pair && (p.block_n % 32 != 0)) p.block_n = round_up(p.block_n, 32);  // each CTA stages block_n/2 rows of B (multiple of 16)
@@ -686,18 +678,37 @@ int gemm_plan(const GemmDesc& d, GemmPlan* plan) {
   const int ring_budget = kSmemTotal - 1024 - kBiasBytes - p.staging_bytes;
   p.num_stages = std::min(kMaxStages, ring_budget / stage_bytes_eff);
   SV_CHECK(p.num_stages >= 2, "GEMM shared-memory plan");
-  p.num_n_tiles = ceil_div(d.N, p.block_n);
-  p.num_tiles = ceil_div(d.M, p.pair ? 2 * kBlockM : kBlockM) * p.num_n_tiles;
+  p.num_n_tiles = ceil_div(N, p.block_n);
+  p.num_tiles = ceil_div(M, p.pair ? 2 * kBlockM : kBlockM) * p.num_n_tiles;
   {
     static const int pf_env = getenv("SURGVID_GEMM_PREFETCH") ? atoi(getenv("SURGVID_GEMM_PREFETCH")) : 0;  // measured: no gain (0 = off)
     p.prefetch = pf_env;
   }
-  p.act = d.act; p.out_fp32 = d.out_fp32;
-  p.bias = d.bias; p.residual = d.residual; p.ldr = d.ldr; p.out = d.out; p.ldc = d.ldc;
+  p.out_fp32 = out_fp32;
+  p.kb_split = ceil_div(K - K2, kBlockK);
   plan->grid = p.pair ? 2 * std::min(p.num_tiles, sms / 2) : std::min(p.num_tiles, sms);
   plan->smem_bytes = static_cast<size_t>(p.num_stages) * stage_bytes_eff + p.staging_bytes + kBiasBytes + 1024;
-  plan->flops = 2.0 * d.M * static_cast<double>(d.N) * d.K;
-  p.kb_split = ceil_div(d.K - d.K2, kBlockK);
+  plan->flops = 2.0 * M * static_cast<double>(N) * K;
+  return SV_OK;
+}
+
+int gemm_plan(const GemmDesc& d, GemmPlan* plan) {
+  SV_CHECK(d.M > 0 && d.N > 0 && d.K > 0, "GEMM dims must be positive");
+  SV_CHECK(d.K % 8 == 0 && d.N % 8 == 0, "GEMM needs K%8==0 and N%8==0");
+  SV_CHECK(d.K2 >= 0 && d.K2 < d.K && (d.K2 == 0 || (d.A2 != nullptr && (d.K - d.K2) % kBlockK == 0 && d.K2 % 8 == 0 && d.lda2 >= d.K2)),
+           "GEMM second A segment: K-K2 must be a multiple of 64, K2 % 8 == 0");
+  SV_CHECK(d.lda >= d.K - d.K2 && d.ldw >= d.K && d.ldc >= d.N, "GEMM leading dimensions too small");
+  SV_CHECK(d.A && d.W && d.out, "GEMM null operand");
+  SV_CHECK((reinterpret_cast<uintptr_t>(d.out) & 15) == 0 && d.ldc % (d.out_fp32 ? 4 : 8) == 0, "GEMM output must be 16B-aligned rows");
+  if (d.residual) SV_CHECK((reinterpret_cast<uintptr_t>(d.residual) & 15) == 0 && d.ldr % 4 == 0 && d.ldr >= d.N, "GEMM residual alignment");
+  if (d.bias) SV_CHECK((reinterpret_cast<uintptr_t>(d.bias) & 15) == 0, "GEMM bias alignment");
+  const int sms = device_sm_count();
+  SV_CHECK(sms > 0, "no CUDA device");
+  SV_TRY(gemm_plan_shape(d.M, d.N, d.K, d.K2, d.out_fp32, d.residual != nullptr, d.pair, sms, plan));
+  GemmParams& p = plan->p;
+  const int b_rows = p.pair ? p.block_n / 2 : p.block_n;
+  p.act = d.act;
+  p.bias = d.bias; p.residual = d.residual; p.ldr = d.ldr; p.out = d.out; p.ldc = d.ldc;
   SV_TRY(encode_operand_map(&plan->tmap_a, d.A, d.M, d.K - d.K2, d.lda, kBlockM));
   if (d.K2 > 0) SV_TRY(encode_operand_map(&plan->tmap_a2, d.A2, d.M, d.K2, d.lda2, kBlockM));
   else plan->tmap_a2 = plan->tmap_a;
@@ -795,6 +806,23 @@ extern "C" int sv_op_gemm_bf16(const uint16_t* A, int64_t lda, const uint16_t* W
   sv::GemmPlan plan;
   SV_TRY(sv::gemm_plan(d, &plan));
   return sv::gemm_launch(plan, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int sv_op_gemm_plan_info(int32_t M, int32_t N, int32_t K, int32_t K2, int32_t out_fp32, int32_t has_residual, int32_t pair_request,
+                                    int32_t num_sms, int32_t* info) {
+  SV_CHECK(info != nullptr, "GEMM plan info: null output");
+  SV_CHECK(M > 0 && N > 0 && K > 0 && num_sms > 0, "GEMM plan info: dims and SM count must be positive");
+  SV_CHECK(K % 8 == 0 && N % 8 == 0, "GEMM needs K%8==0 and N%8==0");
+  SV_CHECK(K2 >= 0 && K2 < K && (K2 == 0 || ((K - K2) % 64 == 0 && K2 % 8 == 0)), "GEMM second A segment: K-K2 must be a multiple of 64, K2 % 8 == 0");
+  sv::GemmPlan plan;
+  SV_TRY(sv::gemm_plan_shape(M, N, K, K2, out_fp32 ? 1 : 0, has_residual != 0, pair_request, num_sms, &plan));
+  const sv::GemmParams& p = plan.p;
+  const int epi = !p.tma_out ? SV_GEMM_EPI_TRANSPOSE : (!out_fp32 ? SV_GEMM_EPI_BF16_TMA : (has_residual ? SV_GEMM_EPI_F32_TMA_RESID : SV_GEMM_EPI_F32_TMA));
+  const int32_t v[SV_GEMM_PLAN_INFO_LEN] = {p.block_n, p.pair, p.tma_out, p.num_stages, p.epi_bufs, p.epi_lag, p.prefetch, p.num_tiles, plan.grid,
+                                            epi, (out_fp32 ? 1 : 0) | (has_residual ? 2 : 0) | (p.pair ? 4 : 0), p.num_n_tiles,
+                                            static_cast<int32_t>(plan.smem_bytes)};
+  std::copy(v, v + SV_GEMM_PLAN_INFO_LEN, info);
+  return SV_OK;
 }
 
 extern "C" int sv_op_gemm_bf16_cat(const uint16_t* A, int64_t lda, const uint16_t* A2, int64_t lda2, int32_t K2, const uint16_t* W, int64_t ldw,

@@ -124,6 +124,24 @@ def gemm_bf16(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = N
     return out
 
 
+GEMM_PLAN_FIELDS = ("block_n", "pair", "tma_out", "num_stages", "epi_bufs", "epi_lag", "prefetch", "num_tiles", "grid", "epilogue", "kernel",
+                    "num_n_tiles", "smem_bytes")
+GEMM_EPILOGUES = ("bf16_tma", "f32_tma", "f32_tma_resid", "transpose")   # SV_GEMM_EPI_* in include/surgvid.h
+
+
+def gemm_plan_info(M: int, N: int, K: int, K2: int = 0, out_fp32: bool = False, residual: bool = False, pair: int = -1,
+                   num_sms: Optional[int] = None) -> dict:
+    """The launch plan gemm_bf16 / gemm_bf16_cat choose for this problem (sv_op_gemm_plan_info; host only).  `num_sms` defaults to
+    the current device's SM count; `epilogue` is named by GEMM_EPILOGUES."""
+    if num_sms is None:
+        num_sms = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+    info = (ctypes.c_int32 * len(GEMM_PLAN_FIELDS))()
+    _native.check(_native.lib().sv_op_gemm_plan_info(M, N, K, K2, int(out_fp32), int(residual), pair, num_sms, info), "sv_op_gemm_plan_info")
+    d = dict(zip(GEMM_PLAN_FIELDS, info))
+    d["epilogue"] = GEMM_EPILOGUES[d["epilogue"]]
+    return d
+
+
 def gemm_bf16_cat(a: torch.Tensor, a2: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None, act: int = 0,
                   residual: Optional[torch.Tensor] = None, out_dtype: torch.dtype = torch.bfloat16, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """out = act(cat([a, a2], 1) @ w.T + bias) (+ residual) without building the concatenation; a [M,K1] (K1 % 64 == 0), a2 [M,K2] bf16

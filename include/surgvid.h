@@ -203,6 +203,22 @@ int sv_op_gemm_bf16(const uint16_t* A, int64_t lda, const uint16_t* W, int64_t l
                     const float* bias, int32_t act, const float* residual, int64_t ldr, void* out, int64_t ldc,
                     int32_t out_fp32, void* stream);
 
+/* The launch plan sv_op_gemm_bf16 / sv_op_gemm_bf16_cat choose for a problem on a device with num_sms SMs (the same function decides
+ * both).  Host only: touches neither device nor driver.  It depends on M, N, K, K2 (0 without a second A segment), the output type,
+ * whether there is a residual, pair_request (-1 auto, 0 off, 1 on; the ops take it from SURGVID_GEMM_PAIR when set) and the
+ * switches SURGVID_GEMM_TMA_OUT / _EPI_BUFS / _EPI_LAG / _PREFETCH / _PAIR, read once per process.  info[SV_GEMM_PLAN_INFO_LEN]:
+ *   0 block_n (UMMA N), 1 pair (2-CTA clusters), 2 tma_out, 3 num_stages (operand ring depth), 4 epi_bufs, 5 epi_lag, 6 prefetch,
+ *   7 num_tiles, 8 grid (CTAs), 9 epilogue form (SV_GEMM_EPI_*), 10 kernel instantiation gemm_bf16_tcgen05_kernel<act, OUT_F32, RESID,
+ *   PAIR> as OUT_F32 | RESID << 1 | PAIR << 2, 11 num_n_tiles, 12 dynamic shared memory bytes.
+ * Shape errors (as sv_op_gemm_bf16 reports them) -> SV_ERR_INVALID. */
+#define SV_GEMM_EPI_BF16_TMA 0       /* bf16 result, no residual: 2-D TMA stores of 32x32 boxes */
+#define SV_GEMM_EPI_F32_TMA 1        /* fp32 result, no residual: 2-D TMA stores of 16x32 boxes */
+#define SV_GEMM_EPI_F32_TMA_RESID 2  /* fp32 result + fp32 residual: TMA residual loads into a per-warp ring, TMA stores */
+#define SV_GEMM_EPI_TRANSPOSE 3      /* bf16 result + residual, or SURGVID_GEMM_TMA_OUT=0: transposed through shared memory, plain stores */
+#define SV_GEMM_PLAN_INFO_LEN 13
+int sv_op_gemm_plan_info(int32_t M, int32_t N, int32_t K, int32_t K2, int32_t out_fp32, int32_t has_residual, int32_t pair_request,
+                         int32_t num_sms, int32_t* info);
+
 /* LayerNorm over the last dim of fp32 [rows, C] -> optional fp32 and/or bf16 outputs (either may be NULL). */
 int sv_op_layernorm(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int32_t C,
                     float* out_f32, uint16_t* out_bf16, void* stream);
