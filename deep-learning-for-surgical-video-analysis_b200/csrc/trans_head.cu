@@ -8,8 +8,12 @@
 // residual + LayerNorm, position-wise FFN with ReLU, residual + LayerNorm), one decoder layer whose single query cross-attends the
 // encoder output (same blocks).  fp32 throughout (d_model = 14: nothing here is tensor-core shaped).
 //
-// One persistent CTA = two groups of 128 threads (4 warps = 4 heads each); every group walks its own frames t with its own Q/K/V tiles
-// and named barriers, and both share the weights (86 KB, d_model padded to 16) in shared memory.
+// d_k = d_v is a template parameter (32: mstcn_f_maps 32; 64: mstcn_f_maps >= 64, adapter_transformer.py:315), see HeadCfg.
+//   d_k = 32: one persistent CTA = two groups of 128 threads (4 warps = 4 heads each); every group walks its own frames t with its own
+//             Q/K/V tiles and named barriers, and both share the weights (86 KB, d_model padded to 16) in shared memory.
+//   d_k = 64: the weights alone take 155 KB, so a CTA is one group, and it keeps no Q tile: a lane computes its window row's Q of its
+//             head in registers right before the scores, and the self-attention context overwrites the head's own K columns, which no
+//             other warp reads (228 936 B of shared memory in all).
 #include <string.h>
 
 #include <map>
@@ -23,19 +27,31 @@ namespace {
 
 constexpr int kDP = 16;      // d_model padded
 constexpr int kH = 4;        // heads
-constexpr int kDK = 32;      // d_k = d_v
-constexpr int kHD = kH * kDK;
 constexpr int kLMax = 32;    // len_q <= 32
 constexpr int kFFMax = 64;   // d_ff <= 64
-constexpr int kLdS = kHD + 1;  // row stride of the Q/K/V tiles (conflict-free row-wise reads)
 
-// blob layout of one attention block / one FFN block (floats)
-constexpr int kAttnWQ = 0, kAttnBQ = kHD * kDP, kAttnWK = kAttnBQ + kHD, kAttnBK = kAttnWK + kHD * kDP, kAttnWV = kAttnBK + kHD,
-              kAttnBV = kAttnWV + kHD * kDP, kAttnWO = kAttnBV + kHD, kAttnBO = kAttnWO + kDP * kHD, kAttnG = kAttnBO + kDP, kAttnB = kAttnG + kDP,
-              kAttnSize = kAttnB + kDP;
+// blob layout of one FFN block (floats)
 constexpr int kFfnW1 = 0, kFfnB1 = kFFMax * kDP, kFfnW2 = kFfnB1 + kFFMax, kFfnB2 = kFfnW2 + kDP * kFFMax, kFfnG = kFfnB2 + kDP, kFfnB = kFfnG + kDP,
               kFfnSize = kFfnB + kDP;
-constexpr int kBlobSize = 2 * (kAttnSize + kFfnSize);   // encoder attn | encoder ffn | decoder attn | decoder ffn
+
+template <int DK>   // d_k = d_v
+struct HeadCfg {
+  static_assert(DK == 32 || DK == 64, "d_k = d_v = 32 or 64");
+  static constexpr int kDK = DK;
+  static constexpr int kHD = kH * kDK;
+  static constexpr int kLdS = kHD + 1;  // row stride of the Q/K/V tiles (conflict-free row-wise reads)
+  // blob layout of one attention block (floats)
+  static constexpr int kAttnWQ = 0, kAttnBQ = kHD * kDP, kAttnWK = kAttnBQ + kHD, kAttnBK = kAttnWK + kHD * kDP, kAttnWV = kAttnBK + kHD,
+                       kAttnBV = kAttnWV + kHD * kDP, kAttnWO = kAttnBV + kHD, kAttnBO = kAttnWO + kDP * kHD, kAttnG = kAttnBO + kDP,
+                       kAttnB = kAttnG + kDP, kAttnSize = kAttnB + kDP;
+  static constexpr int kBlobSize = 2 * (kAttnSize + kFfnSize);   // encoder attn | encoder ffn | decoder attn | decoder ffn
+  static constexpr int kGroups = DK == 32 ? 2 : 1;               // 128-thread groups per CTA
+  // per-group tiles: Q (d_k = 32 only), K, V [kLMax][kLdS]; X, Y, E [kLMax][kDP]; the decoder query [kDP]; d_k = 64 adds the decoder's
+  // Q row and context row [2][kLdS] (d_k = 32 keeps both in the Q tile)
+  static constexpr int kGroupFloats = (DK == 32 ? 3 : 2) * kLMax * kLdS + 3 * kLMax * kDP + kDP + (DK == 32 ? 0 : 2 * kLdS);
+  static constexpr int kSmemBytes = (kBlobSize + kGroups * kGroupFloats) * static_cast<int>(sizeof(float));
+};
+static_assert(HeadCfg<32>::kSmemBytes <= 227 * 1024 && HeadCfg<64>::kSmemBytes <= 227 * 1024, "shared memory per block");
 
 struct TransParams {
   int D, L, FF, n_videos;
@@ -55,8 +71,6 @@ __device__ __forceinline__ void layer_norm_inplace(float (&v)[kDP], int D, const
   for (int c = 0; c < kDP; ++c) v[c] = (c < D) ? (v[c] - m) * r * g[c] + b[c] : 0.f;
 }
 
-constexpr int kGroups = 2;                                       // 128-thread groups per CTA
-constexpr int kGroupFloats = 3 * kLMax * kLdS + 3 * kLMax * kDP + kDP;   // per-group tiles
 __device__ __forceinline__ void group_sync(int grp) { asm volatile("bar.sync %0, 128;" ::"r"(grp + 1) : "memory"); }
 
 // Where a window row that precedes its video's (or stream chunk's) first frame in `logits` comes from.
@@ -73,20 +87,26 @@ struct StreamWindow {
   const float* __restrict__ ring;      // [n_streams][len_q - 1][D]
 };
 
-template <class Window>
-__global__ void __launch_bounds__(128 * kGroups) trans_head_kernel(const float* __restrict__ logits, int64_t ldx, const float* __restrict__ query,
+template <int DK, class Window>
+__global__ void __launch_bounds__(128 * HeadCfg<DK>::kGroups) trans_head_kernel(const float* __restrict__ logits, int64_t ldx, const float* __restrict__ query,
                                                          const int64_t* __restrict__ offsets, int64_t T, const float* __restrict__ blob,
                                                          float* __restrict__ out, const TransParams p, const Window win) {
+  using C = HeadCfg<DK>;
+  constexpr int kDK = C::kDK, kHD = C::kHD, kLdS = C::kLdS, kGroups = C::kGroups, kBlobSize = C::kBlobSize;
+  constexpr int kAttnWQ = C::kAttnWQ, kAttnBQ = C::kAttnBQ, kAttnWK = C::kAttnWK, kAttnBK = C::kAttnBK, kAttnWV = C::kAttnWV, kAttnBV = C::kAttnBV,
+                kAttnWO = C::kAttnWO, kAttnBO = C::kAttnBO, kAttnG = C::kAttnG, kAttnB = C::kAttnB, kAttnSize = C::kAttnSize;
   extern __shared__ __align__(16) float sm[];
   float* Wb = sm;                              // kBlobSize
   const int grp = threadIdx.x >> 7;
-  float* Qs = Wb + kBlobSize + grp * kGroupFloats;   // [kLMax][kLdS]  Q, then the attention context
-  float* Ks = Qs + kLMax * kLdS;
+  float* Qs = Wb + kBlobSize + grp * C::kGroupFloats;   // d_k = 32: [kLMax][kLdS]  Q, then the attention context
+  float* Ks = Qs + (DK == 32 ? kLMax * kLdS : 0);       // d_k = 64: the attention context overwrites K (head h's columns by warp h)
   float* Vs = Ks + kLMax * kLdS;
   float* Xs = Vs + kLMax * kLdS;               // [kLMax][kDP]  window
   float* Ys = Xs + kLMax * kDP;                // [kLMax][kDP]
   float* Es = Ys + kLMax * kDP;                // [kLMax][kDP]  encoder output
   float* qv = Es + kLMax * kDP;                // [kDP] decoder query
+  float* Cs = DK == 32 ? Qs : Ks;              // self-attention context [kLMax][kLdS]
+  float* Qd = DK == 32 ? Qs : qv + kDP;        // decoder: row 0 its Q, row 1 the cross-attention context
   const int tid = threadIdx.x & 127, warp = tid >> 5, lane = tid & 31;
   const int D = p.D, L = p.L, FF = p.FF;
   for (int i = threadIdx.x; i < kBlobSize / 4; i += 128 * kGroups) reinterpret_cast<float4*>(Wb)[i] = __ldg(reinterpret_cast<const float4*>(blob) + i);
@@ -124,55 +144,124 @@ __global__ void __launch_bounds__(128 * kGroups) trans_head_kernel(const float* 
     }
     if (tid < kDP) qv[tid] = tid < D ? __ldg(query + t * D + tid) : 0.f;
     group_sync(grp);
-    // ---- (2) encoder Q, K, V: thread = one of the 128 projection columns
-    {
-      float wq[kDP], wk[kDP], wv[kDP];
+    if constexpr (DK == 32) {
+      // ---- (2) encoder Q, K, V: thread = one of the 128 projection columns
+      {
+        float wq[kDP], wk[kDP], wv[kDP];
 #pragma unroll
-      for (int c = 0; c < kDP; ++c) { wq[c] = EA[kAttnWQ + tid * kDP + c]; wk[c] = EA[kAttnWK + tid * kDP + c]; wv[c] = EA[kAttnWV + tid * kDP + c]; }
-      const float bq = EA[kAttnBQ + tid], bk = EA[kAttnBK + tid], bv = EA[kAttnBV + tid];
-      for (int i = 0; i < L; ++i) {
-        float q = bq, k = bk, v = bv;
+        for (int c = 0; c < kDP; ++c) { wq[c] = EA[kAttnWQ + tid * kDP + c]; wk[c] = EA[kAttnWK + tid * kDP + c]; wv[c] = EA[kAttnWV + tid * kDP + c]; }
+        const float bq = EA[kAttnBQ + tid], bk = EA[kAttnBK + tid], bv = EA[kAttnBV + tid];
+        for (int i = 0; i < L; ++i) {
+          float q = bq, k = bk, v = bv;
 #pragma unroll
-        for (int c = 0; c < kDP; ++c) { const float x = Xs[i * kDP + c]; q = fmaf(x, wq[c], q); k = fmaf(x, wk[c], k); v = fmaf(x, wv[c], v); }
-        Qs[i * kLdS + tid] = q; Ks[i * kLdS + tid] = k; Vs[i * kLdS + tid] = v;
-      }
-    }
-    group_sync(grp);
-    // ---- (3) self-attention: warp = head, lane = query row
-    if (lane < L) {
-      float q[kDK];
-#pragma unroll
-      for (int d = 0; d < kDK; ++d) q[d] = Qs[lane * kLdS + warp * kDK + d];
-      float s[kLMax];
-      float m = -INFINITY;
-#pragma unroll
-      for (int j = 0; j < kLMax; ++j) {
-        float a = 0.f;
-        if (j < L) {
-#pragma unroll
-          for (int d = 0; d < kDK; ++d) a = fmaf(q[d], Ks[j * kLdS + warp * kDK + d], a);
-          a *= p.scale;
-          m = fmaxf(m, a);
-        }
-        s[j] = a;
-      }
-      float den = 0.f;
-#pragma unroll
-      for (int j = 0; j < kLMax; ++j) { s[j] = (j < L) ? __expf(s[j] - m) : 0.f; den += s[j]; }
-      const float inv = 1.0f / den;
-      float ctx[kDK];
-#pragma unroll
-      for (int d = 0; d < kDK; ++d) ctx[d] = 0.f;
-#pragma unroll
-      for (int j = 0; j < kLMax; ++j) {
-        if (j < L) {
-          const float pj = s[j] * inv;
-#pragma unroll
-          for (int d = 0; d < kDK; ++d) ctx[d] = fmaf(pj, Vs[j * kLdS + warp * kDK + d], ctx[d]);
+          for (int c = 0; c < kDP; ++c) { const float x = Xs[i * kDP + c]; q = fmaf(x, wq[c], q); k = fmaf(x, wk[c], k); v = fmaf(x, wv[c], v); }
+          Qs[i * kLdS + tid] = q; Ks[i * kLdS + tid] = k; Vs[i * kLdS + tid] = v;
         }
       }
+      group_sync(grp);
+      // ---- (3) self-attention: warp = head, lane = query row
+      if (lane < L) {
+        float q[kDK];
 #pragma unroll
-      for (int d = 0; d < kDK; ++d) Qs[lane * kLdS + warp * kDK + d] = ctx[d];   // only this lane ever read this Q row
+        for (int d = 0; d < kDK; ++d) q[d] = Qs[lane * kLdS + warp * kDK + d];
+        float s[kLMax];
+        float m = -INFINITY;
+#pragma unroll
+        for (int j = 0; j < kLMax; ++j) {
+          float a = 0.f;
+          if (j < L) {
+#pragma unroll
+            for (int d = 0; d < kDK; ++d) a = fmaf(q[d], Ks[j * kLdS + warp * kDK + d], a);
+            a *= p.scale;
+            m = fmaxf(m, a);
+          }
+          s[j] = a;
+        }
+        float den = 0.f;
+#pragma unroll
+        for (int j = 0; j < kLMax; ++j) { s[j] = (j < L) ? __expf(s[j] - m) : 0.f; den += s[j]; }
+        const float inv = 1.0f / den;
+        float ctx[kDK];
+#pragma unroll
+        for (int d = 0; d < kDK; ++d) ctx[d] = 0.f;
+#pragma unroll
+        for (int j = 0; j < kLMax; ++j) {
+          if (j < L) {
+            const float pj = s[j] * inv;
+#pragma unroll
+            for (int d = 0; d < kDK; ++d) ctx[d] = fmaf(pj, Vs[j * kLdS + warp * kDK + d], ctx[d]);
+          }
+        }
+#pragma unroll
+        for (int d = 0; d < kDK; ++d) Qs[lane * kLdS + warp * kDK + d] = ctx[d];   // only this lane ever read this Q row
+      }
+    } else {
+      // ---- (2) encoder K, V: thread = projection columns tid and tid + 128
+#pragma unroll 1
+      for (int col = tid; col < kHD; col += 128) {
+        float wk[kDP], wv[kDP];
+#pragma unroll
+        for (int c = 0; c < kDP; ++c) { wk[c] = EA[kAttnWK + col * kDP + c]; wv[c] = EA[kAttnWV + col * kDP + c]; }
+        const float bk = EA[kAttnBK + col], bv = EA[kAttnBV + col];
+        for (int i = 0; i < L; ++i) {
+          float k = bk, v = bv;
+#pragma unroll
+          for (int c = 0; c < kDP; ++c) { const float x = Xs[i * kDP + c]; k = fmaf(x, wk[c], k); v = fmaf(x, wv[c], v); }
+          Ks[i * kLdS + col] = k; Vs[i * kLdS + col] = v;
+        }
+      }
+      group_sync(grp);
+      // ---- (3) self-attention: warp = head, lane = query row (lanes past L repeat row L - 1 and store nothing)
+      {
+        const int r = lane < L ? lane : L - 1;
+        float s[kLMax];
+        float m = -INFINITY;
+        {
+          float x[kDP];
+#pragma unroll
+          for (int c = 0; c < kDP; ++c) x[c] = Xs[r * kDP + c];
+          float q[kDK];   // this row's Q of head `warp`, summed in the order of the projection above
+#pragma unroll
+          for (int d = 0; d < kDK; ++d) {
+            const int col = warp * kDK + d;
+            float a = EA[kAttnBQ + col];
+#pragma unroll
+            for (int c = 0; c < kDP; ++c) a = fmaf(x[c], EA[kAttnWQ + col * kDP + c], a);
+            q[d] = a;
+          }
+#pragma unroll
+          for (int j = 0; j < kLMax; ++j) {
+            float a = 0.f;
+            if (j < L) {
+#pragma unroll
+              for (int d = 0; d < kDK; ++d) a = fmaf(q[d], Ks[j * kLdS + warp * kDK + d], a);
+              a *= p.scale;
+              m = fmaxf(m, a);
+            }
+            s[j] = a;
+          }
+        }
+        float den = 0.f;
+#pragma unroll
+        for (int j = 0; j < kLMax; ++j) { s[j] = (j < L) ? __expf(s[j] - m) : 0.f; den += s[j]; }
+        const float inv = 1.0f / den;
+        float ctx[kDK];
+#pragma unroll
+        for (int d = 0; d < kDK; ++d) ctx[d] = 0.f;
+#pragma unroll
+        for (int j = 0; j < kLMax; ++j) {
+          if (j < L) {
+            const float pj = s[j] * inv;
+#pragma unroll
+            for (int d = 0; d < kDK; ++d) ctx[d] = fmaf(pj, Vs[j * kLdS + warp * kDK + d], ctx[d]);
+          }
+        }
+        __syncwarp();   // every lane of this head is done reading its K columns
+        if (lane < L) {
+#pragma unroll
+          for (int d = 0; d < kDK; ++d) Cs[lane * kLdS + warp * kDK + d] = ctx[d];
+        }
+      }
     }
     group_sync(grp);
     // ---- (4) output projection + residual: warp = group of 4 channels, lane = row
@@ -181,7 +270,7 @@ __global__ void __launch_bounds__(128 * kGroups) trans_head_kernel(const float* 
 #pragma unroll
       for (int u = 0; u < 4; ++u) { const int c = warp * 4 + u; acc[u] = (c < D) ? EA[kAttnBO + c] + Xs[lane * kDP + c] : 0.f; }
       for (int k = 0; k < kHD; ++k) {
-        const float cv = Qs[lane * kLdS + k];
+        const float cv = Cs[lane * kLdS + k];
 #pragma unroll
         for (int u = 0; u < 4; ++u) acc[u] = fmaf(cv, EA[kAttnWO + (warp * 4 + u) * kHD + k], acc[u]);
       }
@@ -211,47 +300,51 @@ __global__ void __launch_bounds__(128 * kGroups) trans_head_kernel(const float* 
       for (int c = 0; c < kDP; ++c) Es[lane * kDP + c] = o[c];
     }
     group_sync(grp);
-    // ---- (5) decoder: K, V of the encoder output, Q of the query: thread = projection column
-    {
+    // ---- (5) decoder: K, V of the encoder output, Q of the query: thread = projection column (d_k = 64: columns tid and tid + 128)
+#pragma unroll 1
+    for (int col = tid; col < kHD; col += 128) {
       float wk[kDP], wv[kDP];
-      float qd = DA[kAttnBQ + tid];
+      float qd = DA[kAttnBQ + col];
 #pragma unroll
       for (int c = 0; c < kDP; ++c) {
-        wk[c] = DA[kAttnWK + tid * kDP + c]; wv[c] = DA[kAttnWV + tid * kDP + c];
-        qd = fmaf(qv[c], DA[kAttnWQ + tid * kDP + c], qd);
+        wk[c] = DA[kAttnWK + col * kDP + c]; wv[c] = DA[kAttnWV + col * kDP + c];
+        qd = fmaf(qv[c], DA[kAttnWQ + col * kDP + c], qd);
       }
-      const float bk = DA[kAttnBK + tid], bv = DA[kAttnBV + tid];
+      const float bk = DA[kAttnBK + col], bv = DA[kAttnBV + col];
       for (int i = 0; i < L; ++i) {
         float k = bk, v = bv;
 #pragma unroll
         for (int c = 0; c < kDP; ++c) { const float e = Es[i * kDP + c]; k = fmaf(e, wk[c], k); v = fmaf(e, wv[c], v); }
-        Ks[i * kLdS + tid] = k; Vs[i * kLdS + tid] = v;
+        Ks[i * kLdS + col] = k; Vs[i * kLdS + col] = v;
       }
-      Qs[tid] = qd;   // row 0 of Qs
+      Qd[col] = qd;   // row 0 of Qd
     }
     group_sync(grp);
-    {  // cross-attention: warp = head, lane = key; softmax across the warp; context: lane = channel of the head
+    {  // cross-attention: warp = head, lane = key; softmax across the warp; context: lane = channel of the head (d_k = 64: two)
       float a = -INFINITY;
       if (lane < L) {
         a = 0.f;
 #pragma unroll
-        for (int d = 0; d < kDK; ++d) a = fmaf(Qs[warp * kDK + d], Ks[lane * kLdS + warp * kDK + d], a);
+        for (int d = 0; d < kDK; ++d) a = fmaf(Qd[warp * kDK + d], Ks[lane * kLdS + warp * kDK + d], a);
         a *= p.scale;
       }
       const float m = warp_max(a);
       const float e = (lane < L) ? __expf(a - m) : 0.f;
       const float pj = e / warp_sum(e);
-      float ctx = 0.f;
-      for (int j = 0; j < L; ++j) ctx = fmaf(__shfl_sync(0xffffffffu, pj, j), Vs[j * kLdS + warp * kDK + lane], ctx);
-      __syncwarp();
-      Qs[kLdS + warp * kDK + lane] = ctx;   // row 1 of Qs
+#pragma unroll
+      for (int d0 = 0; d0 < kDK; d0 += 32) {
+        float ctx = 0.f;
+        for (int j = 0; j < L; ++j) ctx = fmaf(__shfl_sync(0xffffffffu, pj, j), Vs[j * kLdS + warp * kDK + d0 + lane], ctx);
+        __syncwarp();
+        Qd[kLdS + warp * kDK + d0 + lane] = ctx;   // row 1 of Qd
+      }
     }
     group_sync(grp);
     if (warp == 0) {  // output projection + residual + LayerNorm + FFN + LayerNorm for the single decoder row: lane = channel
       float o = 0.f;
       if (lane < D) {
         o = DA[kAttnBO + lane] + qv[lane];
-        for (int k = 0; k < kHD; ++k) o = fmaf(Qs[kLdS + k], DA[kAttnWO + lane * kHD + k], o);
+        for (int k = 0; k < kHD; ++k) o = fmaf(Qd[kLdS + k], DA[kAttnWO + lane * kHD + k], o);
       }
       const float fD = static_cast<float>(D);
       float mean = warp_sum(lane < D ? o : 0.f) / fD;
@@ -347,6 +440,46 @@ int put_norm(const sv_trans* h, const std::string& p, int D, std::vector<float>*
   return SV_OK;
 }
 
+template <int DK>
+int pack_blob(const sv_trans* h, std::vector<float>* blob) {
+  using C = HeadCfg<DK>;
+  const int D = h->cfg.d_model, FF = h->cfg.d_ff;
+  blob->assign(C::kBlobSize, 0.f);
+  const char* attn_name[2] = {"encoder.layers.0.enc_self_attn", "decoder.layers.0.dec_enc_attn"};
+  const char* ffn_name[2] = {"encoder.layers.0.pos_ffn", "decoder.layers.0.pos_ffn"};
+  for (int s = 0; s < 2; ++s) {
+    const int a0 = s * (C::kAttnSize + kFfnSize), f0 = a0 + C::kAttnSize;
+    const std::string ap = attn_name[s], fp = ffn_name[s];
+    SV_TRY(put_linear(h, ap + ".W_Q", C::kHD, D, kDP, blob, a0 + C::kAttnWQ, a0 + C::kAttnBQ));
+    SV_TRY(put_linear(h, ap + ".W_K", C::kHD, D, kDP, blob, a0 + C::kAttnWK, a0 + C::kAttnBK));
+    SV_TRY(put_linear(h, ap + ".W_V", C::kHD, D, kDP, blob, a0 + C::kAttnWV, a0 + C::kAttnBV));
+    SV_TRY(put_linear(h, ap + ".fc", D, C::kHD, C::kHD, blob, a0 + C::kAttnWO, a0 + C::kAttnBO));
+    SV_TRY(put_norm(h, ap + ".layer_norm", D, blob, a0 + C::kAttnG, a0 + C::kAttnB));
+    SV_TRY(put_linear(h, fp + ".fc1", FF, D, kDP, blob, f0 + kFfnW1, f0 + kFfnB1));
+    SV_TRY(put_linear(h, fp + ".fc2", D, FF, kFFMax, blob, f0 + kFfnW2, f0 + kFfnB2));
+    SV_TRY(put_norm(h, fp + ".layer_norm", D, blob, f0 + kFfnG, f0 + kFfnB));
+  }
+  return SV_OK;
+}
+
+// One launch of the head kernel over T rows: a persistent grid of at most one CTA per SM, kGroups rows in flight per CTA.
+template <int DK, class Window>
+int launch_head(const float* logits, int64_t ldx, const float* query, const int64_t* offsets, int64_t T, const float* blob, float* out,
+                const TransParams& p, const Window& win, cudaStream_t st) {
+  using C = HeadCfg<DK>;
+  SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(trans_head_kernel<DK, Window>), C::kSmemBytes));
+  const int grid = static_cast<int>(std::min<int64_t>((T + C::kGroups - 1) / C::kGroups, std::max(1, device_sm_count())));
+  trans_head_kernel<DK, Window><<<grid, 128 * C::kGroups, C::kSmemBytes, st>>>(logits, ldx, query, offsets, T, blob, out, p, win);
+  return launch_status("trans_head_kernel");
+}
+
+template <class Window>
+int launch_head(int d_k, const float* logits, int64_t ldx, const float* query, const int64_t* offsets, int64_t T, const float* blob, float* out,
+                const TransParams& p, const Window& win, cudaStream_t st) {
+  return d_k == 64 ? launch_head<64>(logits, ldx, query, offsets, T, blob, out, p, win, st)
+                   : launch_head<32>(logits, ldx, query, offsets, T, blob, out, p, win, st);
+}
+
 }  // namespace
 }  // namespace sv
 
@@ -358,8 +491,8 @@ int sv_trans_create(const sv_trans_cfg* cfg, sv_trans_handle** out) {
   SV_CHECK(cfg->d_model >= 1 && cfg->d_model <= kDP, "trans: 1 <= d_model <= 16");
   SV_CHECK(cfg->len_q >= 1 && cfg->len_q <= kLMax, "trans: 1 <= len_q <= 32");
   SV_CHECK(cfg->d_ff >= 1 && cfg->d_ff <= kFFMax, "trans: 1 <= d_ff <= 64");
-  if (cfg->n_heads != kH || cfg->d_k != kDK || cfg->d_v != kDK)
-    return fail(SV_ERR_UNSUPPORTED, "trans: n_heads = 4 and d_k = d_v = 32 are supported (the reference's mstcn_f_maps = 32 configuration)");
+  if (cfg->n_heads != kH || cfg->d_k != cfg->d_v || (cfg->d_k != 32 && cfg->d_k != 64))
+    return fail(SV_ERR_UNSUPPORTED, "trans: n_heads = 4 and d_k = d_v = 32 or 64 are supported (the reference's mstcn_f_maps = 32 and >= 64 configurations)");
   if (cfg->n_layers != 1) return fail(SV_ERR_UNSUPPORTED, "trans: n_layers must be 1 (adapter_transformer.py:322)");
   int dev = 0;
   SV_CUDA_OK(cudaGetDevice(&dev));
@@ -393,25 +526,11 @@ int sv_trans_set_tensor(sv_trans_handle* h, const char* name, const float* host_
 int sv_trans_pack_weights(sv_trans_handle* h) {
   using namespace sv;
   SV_CHECK(h, "null handle");
-  const int D = h->cfg.d_model, FF = h->cfg.d_ff;
-  std::vector<float> blob(kBlobSize, 0.f);
-  const char* attn_name[2] = {"encoder.layers.0.enc_self_attn", "decoder.layers.0.dec_enc_attn"};
-  const char* ffn_name[2] = {"encoder.layers.0.pos_ffn", "decoder.layers.0.pos_ffn"};
-  for (int s = 0; s < 2; ++s) {
-    const int a0 = s * (kAttnSize + kFfnSize), f0 = a0 + kAttnSize;
-    const std::string ap = attn_name[s], fp = ffn_name[s];
-    SV_TRY(put_linear(h, ap + ".W_Q", kHD, D, kDP, &blob, a0 + kAttnWQ, a0 + kAttnBQ));
-    SV_TRY(put_linear(h, ap + ".W_K", kHD, D, kDP, &blob, a0 + kAttnWK, a0 + kAttnBK));
-    SV_TRY(put_linear(h, ap + ".W_V", kHD, D, kDP, &blob, a0 + kAttnWV, a0 + kAttnBV));
-    SV_TRY(put_linear(h, ap + ".fc", D, kHD, kHD, &blob, a0 + kAttnWO, a0 + kAttnBO));
-    SV_TRY(put_norm(h, ap + ".layer_norm", D, &blob, a0 + kAttnG, a0 + kAttnB));
-    SV_TRY(put_linear(h, fp + ".fc1", FF, D, kDP, &blob, f0 + kFfnW1, f0 + kFfnB1));
-    SV_TRY(put_linear(h, fp + ".fc2", D, FF, kFFMax, &blob, f0 + kFfnW2, f0 + kFfnB2));
-    SV_TRY(put_norm(h, fp + ".layer_norm", D, &blob, f0 + kFfnG, f0 + kFfnB));
-  }
+  std::vector<float> blob;
+  SV_TRY(h->cfg.d_k == 64 ? pack_blob<64>(h, &blob) : pack_blob<32>(h, &blob));
   SV_CUDA_OK(cudaSetDevice(h->device));
-  if (!h->d_blob) SV_CUDA_OK(cudaMalloc(&h->d_blob, kBlobSize * sizeof(float)));
-  SV_CUDA_OK(cudaMemcpy(h->d_blob, blob.data(), kBlobSize * sizeof(float), cudaMemcpyHostToDevice));
+  if (!h->d_blob) SV_CUDA_OK(cudaMalloc(&h->d_blob, blob.size() * sizeof(float)));
+  SV_CUDA_OK(cudaMemcpy(h->d_blob, blob.data(), blob.size() * sizeof(float), cudaMemcpyHostToDevice));
   h->packed = true;
   return SV_OK;
 }
@@ -435,11 +554,7 @@ int sv_trans_forward(sv_trans_handle* h, const float* logits, int64_t ldx, const
   TransParams p;
   p.D = h->cfg.d_model; p.L = h->cfg.len_q; p.FF = h->cfg.d_ff; p.n_videos = n_videos;
   p.scale = 1.0f / sqrtf(static_cast<float>(h->cfg.d_k));
-  const int smem = (kBlobSize + kGroups * kGroupFloats) * static_cast<int>(sizeof(float));
-  SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(trans_head_kernel<OfflineWindow>), smem));
-  const int grid = static_cast<int>(std::min<int64_t>((T + kGroups - 1) / kGroups, std::max(1, device_sm_count())));
-  trans_head_kernel<OfflineWindow><<<grid, 128 * kGroups, smem, st>>>(logits, ldx, query, h->d_offsets, T, h->d_blob, out, p, OfflineWindow{});
-  return launch_status("trans_head_kernel");
+  return launch_head(h->cfg.d_k, logits, ldx, query, h->d_offsets, T, h->d_blob, out, p, OfflineWindow{}, st);
 }
 
 size_t sv_trans_stream_state_bytes(const sv_trans_handle* h, int32_t n_streams) {
@@ -518,11 +633,7 @@ int sv_trans_stream_forward(sv_trans_handle* h, void* state, size_t state_bytes,
   int64_t* seen = static_cast<int64_t*>(state);
   float* ring = reinterpret_cast<float*>(static_cast<char*>(state) + ((static_cast<size_t>(n_streams) * sizeof(int64_t) + 255) & ~static_cast<size_t>(255)));
   const StreamWindow win{h->d_offsets + n_ids + 1, seen, ring};
-  const int smem = (kBlobSize + kGroups * kGroupFloats) * static_cast<int>(sizeof(float));
-  SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(trans_head_kernel<StreamWindow>), smem));
-  const int grid = static_cast<int>(std::min<int64_t>((T + kGroups - 1) / kGroups, std::max(1, device_sm_count())));
-  trans_head_kernel<StreamWindow><<<grid, 128 * kGroups, smem, st>>>(logits, ldx, query, h->d_offsets, T, h->d_blob, out, p, win);
-  SV_TRY(launch_status("trans_head_kernel"));
+  SV_TRY(launch_head(h->cfg.d_k, logits, ldx, query, h->d_offsets, T, h->d_blob, out, p, win, st));
   trans_stream_commit_kernel<<<n_ids, 128, 0, st>>>(logits, ldx, h->d_offsets, n_ids, p.D, p.L, ring, seen);
   SV_TRY(launch_status("trans_stream_commit_kernel"));
   for (int i = 0; i < n_ids; ++i) it->second[stream_ids[i]] += counts[i];

@@ -302,8 +302,8 @@ int sv_op_token_mean(const float* x, int32_t B, int32_t tokens, int32_t C, float
  *   {encoder,decoder}.layers.0.pos_ffn.{fc1,fc2}.{weight[,bias]}, .layer_norm.{weight,bias}   (missing biases = 0). */
 typedef struct sv_trans_cfg {
   int32_t d_model;   /* out_features (14) */
-  int32_t d_ff;      /* mstcn_f_maps (32) */
-  int32_t d_k, d_v;  /* min(64, mstcn_f_maps); 32 supported */
+  int32_t d_ff;      /* mstcn_f_maps (32 or 64), <= 64 */
+  int32_t d_k, d_v;  /* min(64, mstcn_f_maps); d_k = d_v = 32 or 64 supported, anything else is SV_ERR_UNSUPPORTED */
   int32_t n_layers;  /* 1 */
   int32_t n_heads;   /* 4 */
   int32_t len_q;     /* sequence_length (30), <= 32 */

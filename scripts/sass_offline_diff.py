@@ -2,8 +2,9 @@
 
     python scripts/sass_offline_diff.py <earlier libsurgvid.so, e.g. from scripts/build_prev_lib.sh> <mstcn.o | libsurgvid.so> [...]
 
-The stream path gave these kernels a template parameter (`OfflineTaps` / `StreamTaps`, `OfflineWindow` / `StreamWindow`); the offline
-instantiations must not change.  Instructions are compared with addresses and symbol names stripped.  Needs cuobjdump, no GPU."""
+The stream path gave these kernels a template parameter (`OfflineTaps` / `StreamTaps`, `OfflineWindow` / `StreamWindow`), and d_k = 64
+gave the head kernel another (`trans_head_kernel<DK, Window>`); the offline instantiations and both d_k = 32 head instantiations must not
+change.  Instructions are compared with addresses and symbol names stripped.  Needs cuobjdump, no GPU."""
 import difflib
 import re
 import subprocess
@@ -25,10 +26,13 @@ def funcs(path):
     return res
 
 
-PAIRS = [("mstcn_layer_tc_kernelEPKf", "mstcn_layer_tc_kernelINS0_11OfflineTaps"),
-         ("mstcn_layer_kernelILi64ELi1EEE", "mstcn_layer_kernelILi64ELi1ENS0_11OfflineTaps"),
-         ("mstcn_layer_kernelILi32ELi1EEE", "mstcn_layer_kernelILi32ELi1ENS0_11OfflineTaps"),
-         ("trans_head_kernelEPKf", "trans_head_kernelINS0_13OfflineWindow")]
+# (earlier build, this build): regular expressions, each matching one kernel name.  The earlier side matches both the names from before
+# the stream path and those from before the d_k template parameter of the head kernel.
+PAIRS = [("mstcn_layer_tc_kernel(EPKf|INS0_11OfflineTaps)", "mstcn_layer_tc_kernelINS0_11OfflineTaps"),
+         ("mstcn_layer_kernelILi64ELi1E(EE|NS0_11OfflineTaps)", "mstcn_layer_kernelILi64ELi1ENS0_11OfflineTaps"),
+         ("mstcn_layer_kernelILi32ELi1E(EE|NS0_11OfflineTaps)", "mstcn_layer_kernelILi32ELi1ENS0_11OfflineTaps"),
+         ("trans_head_kernel(EPKf|INS0_13OfflineWindow)", "trans_head_kernelILi32ENS0_13OfflineWindow"),
+         ("trans_head_kernelINS0_12StreamWindow", "trans_head_kernelILi32ENS0_12StreamWindow")]
 
 
 def main():
@@ -37,7 +41,7 @@ def main():
         new.update(funcs(p))
     same = True
     for a, b in PAIRS:
-        fa, fb = [k for k in old if a in k], [k for k in new if b in k]
+        fa, fb = [k for k in old if re.search(a, k)], [k for k in new if re.search(b, k)]
         assert len(fa) == 1 and len(fb) == 1, (a, fa, b, fb)
         A, B = old[fa[0]], new[fb[0]]
         print(f"{b}: {len(A)} vs {len(B)} instructions, identical={A == B}")
