@@ -33,7 +33,12 @@ EXPORTED_SYMBOLS = [
     "sv_mstcn_stream_state_bytes", "sv_mstcn_stream_workspace_bytes", "sv_mstcn_stream_reset", "sv_mstcn_stream_step",
     "sv_trans_stream_state_bytes", "sv_trans_stream_reset", "sv_trans_stream_forward",
     "sv_evp_attention_maps_layout", "sv_evp_forward_attention", "sv_op_attention_probs", "sv_op_gemm_plan_info",
+    "sv_op_conv_gemm_bf16", "sv_op_conv_gemm_plan_info",
 ]
+
+# entry points an earlier build of the library, loaded through SURGVID_LIB for a same-box A/B run, may not have (build() still requires
+# every EXPORTED_SYMBOLS entry of the library it builds)
+_ABSENT_IN_EARLIER_BUILDS = ("sv_op_conv_gemm_bf16", "sv_op_conv_gemm_plan_info")
 
 
 class EvpCfg(Structure):
@@ -127,6 +132,10 @@ def _declare(lib):
     lib.sv_op_gemm_bf16_cat.argtypes = [c_void_p, c_int64, c_void_p, c_int64, c_int32, c_void_p, c_int64, c_int32, c_int32, c_int32, c_void_p, c_int32,
                                         c_void_p, c_int64, c_void_p, c_int64, c_int32, c_void_p]
     lib.sv_op_gemm_plan_info.argtypes = [c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, POINTER(c_int32)]
+    if hasattr(lib, "sv_op_conv_gemm_bf16"):   # see _ABSENT_IN_EARLIER_BUILDS
+        lib.sv_op_conv_gemm_bf16.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int64, c_int32,
+                                             c_void_p, c_int32, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_void_p]
+        lib.sv_op_conv_gemm_plan_info.argtypes = [c_int32] * 12 + [POINTER(c_int32), POINTER(c_int32)]
     lib.sv_op_layernorm.argtypes = [c_void_p, c_void_p, c_void_p, c_float, c_int64, c_int32, c_void_p, c_void_p, c_void_p]
     lib.sv_op_im2col.argtypes = [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int64, c_void_p]
     lib.sv_op_dwconv3x3_gelu.argtypes = [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]
@@ -170,6 +179,8 @@ def _declare(lib):
     lib.sv_prep_images.argtypes = [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_size_t, c_void_p]
     lib.sv_prep_flow.argtypes = [c_void_p, c_void_p, c_int32, c_void_p, c_void_p]
     for name in EXPORTED_SYMBOLS:
+        if name in _ABSENT_IN_EARLIER_BUILDS and not hasattr(lib, name):
+            continue
         fn = getattr(lib, name)
         if name not in ("sv_last_error", "sv_evp_workspace_bytes", "sv_mstcn_workspace_bytes", "sv_evp_last_launch_count",
                         "sv_mstcn_last_launch_count", "sv_prep_workspace_bytes", "sv_mstcn_stream_state_bytes",

@@ -498,6 +498,31 @@ struct Builder {
     op.alg_bytes = 2.0 * M * d.K + 2.0 * l.N * d.K + static_cast<double>(M) * l.N * (out_fp32 ? 4 : 2) + (resid ? 4.0 * M * l.N : 0.0);
     push(op);
   }
+  // convolution of an NHWC bf16 input with (kh, kw, cin)-packed weights: an implicit GEMM whose A tiles the TMA gathers through an
+  // im2col-mode map when the geometry allows (conv_gemm_im2col_ok), else an im2col gather into `col` and a GEMM over it
+  void conv(const bf16* x, const ConvGeom& cg, const Lin& l, int act, void* out, int64_t ldc, int out_fp32, bf16* col) {
+    const int M = cg.B * cg.Ho() * cg.Wo();
+    if (!conv_gemm_im2col_ok(cg)) {
+      im2col(nullptr, x, cg.B, cg.C, cg.H, cg.W, cg.k, cg.stride, cg.pad, col, l.ldw);
+      gemm(col, l.ldw, l, M, act, nullptr, 0, out, ldc, out_fp32);
+      return;
+    }
+    if (dry() || status != SV_OK) return;
+    const size_t x_bytes = static_cast<size_t>(cg.B) * cg.H * cg.W * cg.C * 2;
+    if (!arena.contains(out, (static_cast<size_t>(M - 1) * ldc + l.N) * (out_fp32 ? 4 : 2)) || !arena.contains(x, x_bytes)) {
+      status = fail(SV_ERR_STATE, "evp: internal error: a conv GEMM of the plan addresses memory outside its workspace buffer");
+      return;
+    }
+    GemmDesc d;
+    d.A = x; d.conv = cg; d.W = W(l); d.ldw = l.ldw; d.M = M; d.N = l.N; d.K = l.ldw; d.bias = Bf(l); d.act = act;
+    d.out = out; d.ldc = ldc; d.out_fp32 = out_fp32;
+    Op op;
+    op.kind = OP_GEMM;
+    status = gemm_plan(d, &op.gemm);
+    plan->gemm_flops += op.gemm.flops;
+    op.alg_bytes = static_cast<double>(x_bytes) + 2.0 * l.N * d.K + static_cast<double>(M) * l.N * (out_fp32 ? 4 : 2);
+    push(op);
+  }
   void ln(const float* x, const Norm& n, float eps, int64_t rows, float* of, bf16* ob, bf16* patch = nullptr, int pH = 0, int pW = 0, int psr = 0) {
     Op op; op.kind = OP_LN; op.src = x; op.p0 = F(n.g); op.p1 = F(n.b); op.f0 = eps; op.l0 = rows; op.i[0] = n.C; op.dst = of; op.dst2 = ob;
     op.dst3 = patch; op.i[1] = pH; op.i[2] = pW; op.i[3] = psr;
@@ -582,6 +607,18 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
   }
   const int E = c.embedding_dim;
   const int ks[4] = {7, 3, 3, 3}, strd[4] = {4, 2, 2, 2};
+  const int fch[5] = {2, 64, 128, c.embed_dims[2], c.embed_dims[3]};
+  auto geom = [&](int B, int Hi, int Wi, int C, int k, int st, int pad) {
+    ConvGeom cg;
+    cg.B = B; cg.H = Hi; cg.W = Wi; cg.C = C; cg.k = k; cg.stride = st; cg.pad = pad;
+    return cg;
+  };
+  // does the stage-s conv (patch embed / handcrafted prompt / flow conv, input width cin) gather an im2col buffer?  Stage 0 runs the
+  // fused stem when it can (the same test as below, on the packed shapes), stages 1-3 read their input through an im2col map when they can
+  auto needs_col = [&](int s, int cin, int cout) {
+    if (s == 0) return !stem_conv_supported(cin, cout, round_up(49 * cin, 8));
+    return !conv_gemm_im2col_ok(geom(n, g[s - 1].H, g[s - 1].W, cin, 3, 2, 1));
+  };
 
   // ---- sizes of stage-scoped buffers (max over stages)
   size_t max_tok_c = 0, max_tok_cp = 0, max_tok_hid = 0, max_tok_tall = 0, max_kv_c = 0, max_sr_k = 0, max_col = 0, max_conv_out = 0;
@@ -592,23 +629,24 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
     max_tok_hid = std::max(max_tok_hid, M * g[s].hidden);
     max_tok_tall = std::max(max_tok_tall, M * static_cast<size_t>(c.depths[s]) * g[s].Cp);
     max_kv_c = std::max(max_kv_c, Mk * g[s].C);
-    if (g[s].sr > 1) max_sr_k = std::max(max_sr_k, Mk * static_cast<size_t>(g[s].sr * g[s].sr * g[s].C));
+    if (g[s].sr > 1 && !conv_gemm_im2col_ok(geom(n, g[s].H, g[s].W, g[s].C, g[s].sr, g[s].sr, 0)))   // LN1's sr-patch copy
+      max_sr_k = std::max(max_sr_k, Mk * static_cast<size_t>(g[s].sr * g[s].sr * g[s].C));
     const int cin = s == 0 ? 3 : c.embed_dims[s - 1];
     const int cinp = s == 0 ? 3 : c.embed_dims[s - 1] / 4;
-    max_col = std::max(max_col, M * static_cast<size_t>(round_up(ks[s] * ks[s] * cin, 8)));
-    max_col = std::max(max_col, M * static_cast<size_t>(round_up(ks[s] * ks[s] * cinp, 8)));
+    if (needs_col(s, cin, g[s].C)) max_col = std::max(max_col, M * static_cast<size_t>(round_up(ks[s] * ks[s] * cin, 8)));
+    if (needs_col(s, cinp, g[s].Cp)) max_col = std::max(max_col, M * static_cast<size_t>(round_up(ks[s] * ks[s] * cinp, 8)));
     max_conv_out = std::max(max_conv_out, M * g[s].C);
   }
-  const int fch[5] = {2, 64, 128, c.embed_dims[2], c.embed_dims[3]};
   // the flow cross-attention keys/values cover the stage's FULL token grid (no spatial reduction): [n*N, 2C] in `kvb`
   if (with_flow)
     for (int s = 2; s < 4; ++s) max_kv_c = std::max(max_kv_c, static_cast<size_t>(n) * g[s].N * g[s].C);
   if (with_flow)
-    for (int i = 0; i < 4; ++i) max_col = std::max(max_col, static_cast<size_t>(n) * g[i].N * round_up((i == 0 ? 49 : 9) * fch[i], 8));
+    for (int i = 0; i < 4; ++i)
+      if (needs_col(i, fch[i], fch[i + 1])) max_col = std::max(max_col, static_cast<size_t>(n) * g[i].N * round_up((i == 0 ? 49 : 9) * fch[i], 8));
 
   // ---- buffers
   float* seg_g = A.get<float>(static_cast<size_t>(n) * 3 * H * W);
-  bf16* col = A.get<bf16>(max_col);
+  bf16* col = max_col > 0 ? A.get<bf16>(max_col) : nullptr;
   float* conv_out = A.get<float>(max_conv_out);
   float* hc_f32[4];
   bf16* hc_b16[4];
@@ -626,7 +664,7 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
   bf16* qb = A.get<bf16>(max_tok_c);
   bf16* ob = A.get<bf16>(max_tok_c);
   bf16* Pb = A.get<bf16>(max_tok_cp);
-  bf16* a_sr = A.get<bf16>(std::max<size_t>(max_sr_k, 8));
+  bf16* a_sr = max_sr_k > 0 ? A.get<bf16>(max_sr_k) : nullptr;   // sr-patch copy of LN1, only for sr convs without an im2col map
   float* sr_out = A.get<float>(max_kv_c);
   bf16* srn = A.get<bf16>(max_kv_c);
   bf16* kvb = A.get<bf16>(2 * max_kv_c);
@@ -645,9 +683,12 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
       if (s == 0 && stem_conv_supported(cinp, S.hc.N, S.hc.ldw)) {
         b.stem(seg_g, EXT_NONE, S.hc, &S.hc_norm, n, cinp, hh, ww, hc_f32[s], hc_b16[s]);
       } else {
-        if (s == 0) b.im2col(seg_g, nullptr, n, cinp, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.hc.ldw);
-        else b.im2col(nullptr, hc_b16[s - 1], n, cinp, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.hc.ldw);
-        b.gemm(col, S.hc.ldw, S.hc, M, ACT_NONE, nullptr, 0, conv_out, g[s].Cp, 1);
+        if (s == 0) {
+          b.im2col(seg_g, nullptr, n, cinp, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.hc.ldw);
+          b.gemm(col, S.hc.ldw, S.hc, M, ACT_NONE, nullptr, 0, conv_out, g[s].Cp, 1);
+        } else {
+          b.conv(hc_b16[s - 1], geom(n, hh, ww, cinp, ks[s], strd[s], ks[s] / 2), S.hc, ACT_NONE, conv_out, g[s].Cp, 1, col);
+        }
         b.ln(conv_out, S.hc_norm, 1e-5f, M, hc_f32[s], hc_b16[s]);
       }
       hh = g[s].H; ww = g[s].W;
@@ -665,9 +706,12 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
       if (s == 0 && stem_conv_supported(cin, S.pe.N, S.pe.ldw)) {
         b.stem(nullptr, EXT_X, S.pe, &S.pe_norm, n, cin, hh, ww, x, xn);
       } else {
-        if (s == 0) b.im2col(nullptr, nullptr, n, cin, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.pe.ldw, EXT_X);
-        else b.im2col(nullptr, c_b16[s - 1], n, cin, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.pe.ldw);
-        b.gemm(col, S.pe.ldw, S.pe, M, ACT_NONE, nullptr, 0, conv_out, C, 1);
+        if (s == 0) {
+          b.im2col(nullptr, nullptr, n, cin, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.pe.ldw, EXT_X);
+          b.gemm(col, S.pe.ldw, S.pe, M, ACT_NONE, nullptr, 0, conv_out, C, 1);
+        } else {
+          b.conv(c_b16[s - 1], geom(n, hh, ww, cin, ks[s], strd[s], ks[s] / 2), S.pe, ACT_NONE, conv_out, C, 1, col);
+        }
         b.ln(conv_out, S.pe_norm, 1e-5f, M, x, xn);
       }
       // init_prompt (:749-756): P = handcrafted_s + embedding_generator_s(x)   (constant over depth)
@@ -682,11 +726,15 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
         // get_prompt (:776-815): x += shared_mlp(T_i).  Only block 0 does this as its own GEMM; for i >= 1 the term was already
         // added by block i-1's K-concatenated fc2 GEMM (see pack_all).
         if (i == 0) b.gemm(T_all, ldt, S.shared, M, ACT_NONE, x, C, x, C, 1);
-        // attention (:110-131); LN1 also emits the sr-conv's A operand (non-overlapping sr x sr patches) directly
+        // attention (:110-131).  The sr conv (k = stride = sr, no padding) reads LN1's output through an im2col map; where it cannot,
+        // LN1 also emits the conv's A operand (non-overlapping sr x sr patches) as a second bf16 copy
         if (G.sr > 1) {
-          b.ln(x, Bk.n1, 1e-6f, M, nullptr, xn, a_sr, G.H, G.W, G.sr);
+          const ConvGeom srg = geom(n, G.H, G.W, C, G.sr, G.sr, 0);
+          const bool sr_map = conv_gemm_im2col_ok(srg);
+          b.ln(x, Bk.n1, 1e-6f, M, nullptr, xn, sr_map ? nullptr : a_sr, G.H, G.W, G.sr);
           b.gemm(xn, C, Bk.q, M, ACT_NONE, nullptr, 0, qb, C, 0);
-          b.gemm(a_sr, Bk.sr.ldw, Bk.sr, Mk, ACT_NONE, nullptr, 0, sr_out, C, 1);
+          if (sr_map) b.conv(xn, srg, Bk.sr, ACT_NONE, sr_out, C, 1, nullptr);
+          else b.gemm(a_sr, Bk.sr.ldw, Bk.sr, Mk, ACT_NONE, nullptr, 0, sr_out, C, 1);
           b.ln(sr_out, Bk.srn, 1e-5f, Mk, nullptr, srn);
           b.gemm(srn, C, Bk.kv, Mk, ACT_NONE, nullptr, 0, kvb, 2 * C, 0);
         } else {
@@ -726,9 +774,12 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
       if (i == 0 && stem_conv_supported(2, L.N, L.ldw)) {
         b.stem(nullptr, EXT_FLOW, L, nullptr, n, 2, hh, ww, nullptr, fl[i]);
       } else {
-        if (i == 0) b.im2col(nullptr, nullptr, n, 2, hh, ww, 7, 4, 3, col, L.ldw, EXT_FLOW);
-        else b.im2col(nullptr, fl[i - 1], n, fch[i], hh, ww, 3, 2, 1, col, L.ldw);
-        b.gemm(col, L.ldw, L, M, ACT_RELU, nullptr, 0, fl[i], fch[i + 1], 0);
+        if (i == 0) {
+          b.im2col(nullptr, nullptr, n, 2, hh, ww, 7, 4, 3, col, L.ldw, EXT_FLOW);
+          b.gemm(col, L.ldw, L, M, ACT_RELU, nullptr, 0, fl[i], fch[i + 1], 0);
+        } else {
+          b.conv(fl[i - 1], geom(n, hh, ww, fch[i], 3, 2, 1), L, ACT_RELU, fl[i], fch[i + 1], 0, col);
+        }
       }
       hh = g[i].H; ww = g[i].W;
     }

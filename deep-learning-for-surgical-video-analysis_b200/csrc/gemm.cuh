@@ -4,6 +4,18 @@
 
 namespace sv {
 
+// Geometry of a convolution computed as an implicit GEMM: input NHWC bf16 [B, H, W, C], k x k taps, stride, symmetric zero padding.
+// Output pixel m = (b, oh, ow) is GEMM row m (M = B * Ho * Wo); the GEMM's K index is (kh, kw, cin), the order conv weights are packed in.
+struct ConvGeom {
+  int B = 0, H = 0, W = 0, C = 0, k = 0, stride = 1, pad = 0;   // k == 0: no convolution
+  int Ho() const { return (H + 2 * pad - k) / stride + 1; }
+  int Wo() const { return (W + 2 * pad - k) / stride + 1; }
+};
+// Can the GEMM read this conv's A operand straight from the NHWC input through an im2col-mode tensor map?  Whole 64-channel k-blocks
+// (C % 64 == 0, so a k-block never straddles two taps), element strides <= 8 and bounding-box corners in [-128, 127] (4-D maps).
+// Host only.
+bool conv_gemm_im2col_ok(const ConvGeom& g);
+
 // out[M,N] = act(A[M,K] * W[N,K]^T + bias[N]) (+ residual[M,N])
 struct GemmDesc {
   const bf16* A = nullptr;   // [M, K] row-major, row stride lda (elements)
@@ -24,6 +36,9 @@ struct GemmDesc {
   int64_t ldc = 0;
   int out_fp32 = 0;
   int pair = -1;  // CTA-pair mode (tcgen05 cta_group::2, 256-row tiles, B split across the pair): -1 auto, 0 off, 1 on
+  // conv.k > 0: implicit-GEMM convolution, A is the NHWC input [conv.B, conv.H, conv.W, conv.C] (lda unused), read through an
+  // im2col-mode tensor map (conv_gemm_im2col_ok must hold); M = B * Ho * Wo, K = k * k * C, no second A segment.
+  ConvGeom conv;
 };
 
 struct GemmParams {
@@ -46,6 +61,9 @@ struct GemmParams {
   long long ldr;
   void* out;
   long long ldc;
+  // implicit-GEMM convolution (GemmDesc::conv): A tiles come from the im2col-mode map; k-block kb = ((kh * k + kw) * C + c0) / 64
+  int conv;         // 1: A is read through an im2col map
+  int conv_k, conv_c, conv_stride, conv_pad, conv_ho, conv_wo;
 };
 
 struct GemmPlan {

@@ -55,7 +55,10 @@ constexpr int kSmemTotal = 230400;                // dynamic shared memory per C
 // the B tile (block_n/2 rows); the leader CTA (cluster rank 0) issues one M=256 MMA per k-step that reads both CTAs' shared
 // memory and writes 128 accumulator rows into each CTA's TMEM.  Shared-memory fill traffic per MAC drops by 1/4..1/3, which is
 // what bounds the K >= 256 GEMMs of stages 3/4 (operands come from L2, not HBM).
-template <int ACT, bool OUT_F32, bool RESID, bool PAIR>
+// CONV = true: implicit-GEMM convolution.  tmap_a is an im2col-mode map of the NHWC input (128 pixels x 64 channels per load, same
+// 128B-swizzled tile as the 2-D map), and k-block kb is tap (kh, kw), channels c0 .. c0 + 63 — the (kh, kw, cin) order of the packed
+// conv weights, so the MMAs see exactly the tiles a materialised im2col buffer would give them.
+template <int ACT, bool OUT_F32, bool RESID, bool PAIR, bool CONV>
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_a2,
                          const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ CUtensorMap tmap_out,
@@ -135,10 +138,20 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
         if (ptx::elect_one()) ptx::tma_prefetch_l2_2d(&tmap_a, pf_kb * kBlockK, pm0);
         if (++pf_kb == num_kb) { pf_kb = 0; pf_tile += tile_step; }
       };
-      for (int i = 0; i < p.prefetch; ++i) prefetch_next();
+      for (int i = 0; i < p.prefetch; ++i) prefetch_next();   // 2-D maps only: gemm_plan sets prefetch = 0 for convolutions
       for (int tile = first_tile; tile < p.num_tiles; tile += tile_step) {
         const int m0 = (tile / p.num_n_tiles) * (PAIR ? 2 * kBlockM : kBlockM) + static_cast<int>(cta_rank) * kBlockM;
         const int n0 = (tile % p.num_n_tiles) * p.block_n + static_cast<int>(cta_rank) * b_rows;
+        // CONV: input pixel (cw, ch, cn) under output pixel m0 with the window's top-left tap, and the tap / channel cursor of k-block kb
+        int cw = 0, ch = 0, cn = 0, tap_w = 0, tap_h = 0, c0 = 0;
+        if constexpr (CONV) {
+          const int hw = p.conv_ho * p.conv_wo;
+          cn = m0 / hw;
+          const int r = m0 - cn * hw;
+          const int oh = r / p.conv_wo;
+          ch = oh * p.conv_stride - p.conv_pad;
+          cw = (r - oh * p.conv_wo) * p.conv_stride - p.conv_pad;
+        }
         for (int kb = 0; kb < num_kb; ++kb) {
           if (p.prefetch > 0) prefetch_next();
           ptx::mbar_wait(&empty_bar[stage], phase ^ 1u);
@@ -152,15 +165,24 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
             if (PAIR) {
               // the leader's barrier collects the bytes of both CTAs; only the leader posts the expectation
               if (cta_rank == 0) ptx::mbar_arrive_expect_tx(&full_bar[stage], static_cast<uint32_t>(2 * stage_bytes));
-              ptx::tma_load_2d_pair(sa, ma, &full_bar[stage], ka, m0);
+              if constexpr (CONV) ptx::tma_load_im2col_4d_pair(sa, &tmap_a, &full_bar[stage], c0, cw, ch, cn, static_cast<uint16_t>(tap_w), static_cast<uint16_t>(tap_h));
+              else ptx::tma_load_2d_pair(sa, ma, &full_bar[stage], ka, m0);
               ptx::tma_load_2d_pair(sb, &tmap_w, &full_bar[stage], kb * kBlockK, n0);
             } else {
               ptx::mbar_arrive_expect_tx(&full_bar[stage], static_cast<uint32_t>(stage_bytes));
-              ptx::tma_load_2d(sa, ma, &full_bar[stage], ka, m0);
+              if constexpr (CONV) ptx::tma_load_im2col_4d(sa, &tmap_a, &full_bar[stage], c0, cw, ch, cn, static_cast<uint16_t>(tap_w), static_cast<uint16_t>(tap_h));
+              else ptx::tma_load_2d(sa, ma, &full_bar[stage], ka, m0);
               ptx::tma_load_2d(sb, &tmap_w, &full_bar[stage], kb * kBlockK, n0);
             }
           }
           __syncwarp();
+          if constexpr (CONV) {
+            c0 += kBlockK;
+            if (c0 == p.conv_c) {
+              c0 = 0;
+              if (++tap_w == p.conv_k) { tap_w = 0; ++tap_h; }
+            }
+          }
           if (++stage == S) { stage = 0; phase ^= 1u; }
         }
       }
@@ -603,7 +625,69 @@ int encode_operand_map(CUtensorMap* map, const bf16* base, int64_t rows, int64_t
   return SV_OK;
 }
 
+typedef CUresult (*EncodeIm2colFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const int*,
+                                  const int*, cuuint32_t, cuuint32_t, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+EncodeIm2colFn get_encode_im2col_fn() {
+  static EncodeIm2colFn fn = nullptr;
+  static std::once_flag once;
+  std::call_once(once, [] {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
+      fn = reinterpret_cast<EncodeIm2colFn>(p);
+  });
+  return fn;
+}
+
+// im2col-mode map of an NHWC bf16 conv input: each load is one 128-pixel column of one tap, 64 channels (128 B) per pixel, 128B swizzle —
+// the tile a 2-D map with box [128 rows, 64 cols] writes.  The bounding box [-pad, W - 1 + pad - (k - 1)] (and the same along H), walked
+// with the conv stride, holds exactly the Ho x Wo window origins; zero OOB fill is the conv's padding and the rows past M.
+int encode_im2col_map(CUtensorMap* map, const bf16* base, const ConvGeom& g) {
+  EncodeIm2colFn fn = get_encode_im2col_fn();
+  if (fn == nullptr) return fail(SV_ERR_CUDA, "cuTensorMapEncodeIm2col driver entry point unavailable (no CUDA driver?)");
+  if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return fail(SV_ERR_INVALID, "conv GEMM input must be 16-byte aligned");
+  const cuuint64_t es = 2;
+  cuuint64_t gdim[4] = {static_cast<cuuint64_t>(g.C), static_cast<cuuint64_t>(g.W), static_cast<cuuint64_t>(g.H), static_cast<cuuint64_t>(g.B)};
+  cuuint64_t gstride[3] = {gdim[0] * es, gdim[0] * gdim[1] * es, gdim[0] * gdim[1] * gdim[2] * es};
+  const int lower[2] = {-g.pad, -g.pad};
+  const int upper[2] = {g.pad - (g.k - 1), g.pad - (g.k - 1)};
+  cuuint32_t estr[4] = {1, static_cast<cuuint32_t>(g.stride), static_cast<cuuint32_t>(g.stride), 1};
+  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<bf16*>(base), gdim, gstride, lower, upper, kBlockK, kBlockM, estr,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    char buf[256];
+    snprintf(buf, sizeof(buf), "cuTensorMapEncodeIm2col failed (CUresult %d) B=%d H=%d W=%d C=%d k=%d stride=%d pad=%d", static_cast<int>(r), g.B, g.H,
+             g.W, g.C, g.k, g.stride, g.pad);
+    return fail(SV_ERR_CUDA, buf);
+  }
+  return SV_OK;
+}
+
+// Host-side checks of a convolution's geometry; no device access.
+int check_conv_args(const ConvGeom& g) {
+  SV_CHECK(g.B > 0 && g.H > 0 && g.W > 0 && g.C > 0 && g.k > 0 && g.stride > 0 && g.pad >= 0, "conv GEMM: B, H, W, C, k, stride must be positive, pad >= 0");
+  SV_CHECK(g.Ho() > 0 && g.Wo() > 0 && g.H + 2 * g.pad >= g.k && g.W + 2 * g.pad >= g.k, "conv GEMM: the kernel window does not fit the padded input");
+  SV_CHECK(static_cast<int64_t>(g.B) * g.Ho() * g.Wo() < (1LL << 31) && static_cast<int64_t>(g.k) * g.k * g.C < (1LL << 31), "conv GEMM: M or K too large");
+  return SV_OK;
+}
+// argument errors -> SV_ERR_INVALID, geometry the im2col map cannot express -> SV_ERR_UNSUPPORTED
+int check_conv(const ConvGeom& g) {
+  SV_TRY(check_conv_args(g));
+  if (!conv_gemm_im2col_ok(g))
+    return fail(SV_ERR_UNSUPPORTED, "conv GEMM: needs C % 64 == 0, stride <= 8 and padding corners -pad, pad - (k - 1) within [-128, 127] (got C=" +
+                                        std::to_string(g.C) + " k=" + std::to_string(g.k) + " stride=" + std::to_string(g.stride) + " pad=" +
+                                        std::to_string(g.pad) + "); gather with sv_op_im2col and use sv_op_gemm_bf16");
+  return SV_OK;
+}
+
 }  // namespace
+
+bool conv_gemm_im2col_ok(const ConvGeom& g) {
+  const int upper = g.pad - (g.k - 1);
+  return g.k > 0 && g.C % kBlockK == 0 && g.stride >= 1 && g.stride <= 8 && g.pad >= 0 && g.pad <= 128 && upper >= -128 && upper <= 127;
+}
 
 int gemm_pick_block_n(int M, int N, int K, int num_sms, int step) {
   // Candidates are legal UMMA N for M=128 (multiples of 16, <= 256).  Model: time ~ waves * (per-tile cost),
@@ -697,7 +781,13 @@ int gemm_plan(const GemmDesc& d, GemmPlan* plan) {
   SV_CHECK(d.K % 8 == 0 && d.N % 8 == 0, "GEMM needs K%8==0 and N%8==0");
   SV_CHECK(d.K2 >= 0 && d.K2 < d.K && (d.K2 == 0 || (d.A2 != nullptr && (d.K - d.K2) % kBlockK == 0 && d.K2 % 8 == 0 && d.lda2 >= d.K2)),
            "GEMM second A segment: K-K2 must be a multiple of 64, K2 % 8 == 0");
-  SV_CHECK(d.lda >= d.K - d.K2 && d.ldw >= d.K && d.ldc >= d.N, "GEMM leading dimensions too small");
+  const bool conv = d.conv.k > 0;
+  if (conv) {
+    SV_TRY(check_conv(d.conv));
+    SV_CHECK(d.K2 == 0 && d.M == d.conv.B * d.conv.Ho() * d.conv.Wo() && d.K == d.conv.k * d.conv.k * d.conv.C,
+             "conv GEMM: M must be B*Ho*Wo and K k*k*C, no second A segment");
+  }
+  SV_CHECK((conv || d.lda >= d.K - d.K2) && d.ldw >= d.K && d.ldc >= d.N, "GEMM leading dimensions too small");
   SV_CHECK(d.A && d.W && d.out, "GEMM null operand");
   SV_CHECK((reinterpret_cast<uintptr_t>(d.out) & 15) == 0 && d.ldc % (d.out_fp32 ? 4 : 8) == 0, "GEMM output must be 16B-aligned rows");
   if (d.residual) SV_CHECK((reinterpret_cast<uintptr_t>(d.residual) & 15) == 0 && d.ldr % 4 == 0 && d.ldr >= d.N, "GEMM residual alignment");
@@ -709,7 +799,15 @@ int gemm_plan(const GemmDesc& d, GemmPlan* plan) {
   const int b_rows = p.pair ? p.block_n / 2 : p.block_n;
   p.act = d.act;
   p.bias = d.bias; p.residual = d.residual; p.ldr = d.ldr; p.out = d.out; p.ldc = d.ldc;
-  SV_TRY(encode_operand_map(&plan->tmap_a, d.A, d.M, d.K - d.K2, d.lda, kBlockM));
+  p.conv = conv ? 1 : 0;
+  p.conv_k = d.conv.k; p.conv_c = d.conv.C; p.conv_stride = d.conv.stride; p.conv_pad = d.conv.pad;
+  p.conv_ho = conv ? d.conv.Ho() : 0; p.conv_wo = conv ? d.conv.Wo() : 0;
+  if (conv) {
+    p.prefetch = 0;
+    SV_TRY(encode_im2col_map(&plan->tmap_a, d.A, d.conv));
+  } else {
+    SV_TRY(encode_operand_map(&plan->tmap_a, d.A, d.M, d.K - d.K2, d.lda, kBlockM));
+  }
   if (d.K2 > 0) SV_TRY(encode_operand_map(&plan->tmap_a2, d.A2, d.M, d.K2, d.lda2, kBlockM));
   else plan->tmap_a2 = plan->tmap_a;
   SV_TRY(encode_operand_map(&plan->tmap_w, d.W, d.N, d.K, d.ldw, b_rows));
@@ -740,27 +838,30 @@ namespace {
 
 typedef void (*GemmKernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const GemmParams);
 
-template <int ACT, bool PAIR>
+template <int ACT, bool PAIR, bool CONV>
 GemmKernelFn pick_kernel(int out_fp32, bool resid) {
-  if (out_fp32) return resid ? gemm_bf16_tcgen05_kernel<ACT, true, true, PAIR> : gemm_bf16_tcgen05_kernel<ACT, true, false, PAIR>;
-  return resid ? gemm_bf16_tcgen05_kernel<ACT, false, true, PAIR> : gemm_bf16_tcgen05_kernel<ACT, false, false, PAIR>;
+  if (out_fp32) return resid ? gemm_bf16_tcgen05_kernel<ACT, true, true, PAIR, CONV> : gemm_bf16_tcgen05_kernel<ACT, true, false, PAIR, CONV>;
+  return resid ? gemm_bf16_tcgen05_kernel<ACT, false, true, PAIR, CONV> : gemm_bf16_tcgen05_kernel<ACT, false, false, PAIR, CONV>;
 }
 
-GemmKernelFn kernel_for(const GemmParams& p) {
+template <bool CONV>
+GemmKernelFn kernel_for_a(const GemmParams& p) {
   const bool resid = p.residual != nullptr;
   if (p.pair) {
     switch (p.act) {
-      case ACT_GELU: return pick_kernel<ACT_GELU, true>(p.out_fp32, resid);
-      case ACT_RELU: return pick_kernel<ACT_RELU, true>(p.out_fp32, resid);
-      default: return pick_kernel<ACT_NONE, true>(p.out_fp32, resid);
+      case ACT_GELU: return pick_kernel<ACT_GELU, true, CONV>(p.out_fp32, resid);
+      case ACT_RELU: return pick_kernel<ACT_RELU, true, CONV>(p.out_fp32, resid);
+      default: return pick_kernel<ACT_NONE, true, CONV>(p.out_fp32, resid);
     }
   }
   switch (p.act) {
-    case ACT_GELU: return pick_kernel<ACT_GELU, false>(p.out_fp32, resid);
-    case ACT_RELU: return pick_kernel<ACT_RELU, false>(p.out_fp32, resid);
-    default: return pick_kernel<ACT_NONE, false>(p.out_fp32, resid);
+    case ACT_GELU: return pick_kernel<ACT_GELU, false, CONV>(p.out_fp32, resid);
+    case ACT_RELU: return pick_kernel<ACT_RELU, false, CONV>(p.out_fp32, resid);
+    default: return pick_kernel<ACT_NONE, false, CONV>(p.out_fp32, resid);
   }
 }
+
+GemmKernelFn kernel_for(const GemmParams& p) { return p.conv ? kernel_for_a<true>(p) : kernel_for_a<false>(p); }
 
 }  // namespace
 
@@ -823,6 +924,38 @@ extern "C" int sv_op_gemm_plan_info(int32_t M, int32_t N, int32_t K, int32_t K2,
                                             static_cast<int32_t>(plan.smem_bytes)};
   std::copy(v, v + SV_GEMM_PLAN_INFO_LEN, info);
   return SV_OK;
+}
+
+extern "C" int sv_op_conv_gemm_bf16(const uint16_t* x, int32_t B, int32_t H, int32_t W, int32_t C, int32_t k, int32_t stride, int32_t pad,
+                                    const uint16_t* Wt, int64_t ldw, int32_t N, const float* bias, int32_t act, const float* residual, int64_t ldr,
+                                    void* out, int64_t ldc, int32_t out_fp32, void* stream) {
+  sv::GemmDesc d;
+  d.conv.B = B; d.conv.H = H; d.conv.W = W; d.conv.C = C; d.conv.k = k; d.conv.stride = stride; d.conv.pad = pad;
+  SV_CHECK(x && Wt && out, "conv GEMM: null input, weight or output");
+  SV_TRY(sv::check_conv(d.conv));
+  SV_CHECK(N > 0 && N % 8 == 0 && ldw >= static_cast<int64_t>(k) * k * C && ldc >= N, "conv GEMM: N % 8 == 0, ldw >= k*k*C and ldc >= N");
+  SV_CHECK(act == sv::ACT_NONE || act == sv::ACT_GELU || act == sv::ACT_RELU, "conv GEMM: act must be 0 (none), 1 (GELU) or 2 (ReLU)");
+  d.A = reinterpret_cast<const sv::bf16*>(x);
+  d.W = reinterpret_cast<const sv::bf16*>(Wt); d.ldw = ldw;
+  d.M = B * d.conv.Ho() * d.conv.Wo(); d.N = N; d.K = k * k * C; d.bias = bias; d.act = act; d.residual = residual; d.ldr = ldr;
+  d.out = out; d.ldc = ldc; d.out_fp32 = out_fp32;
+  if (const char* e = getenv("SURGVID_GEMM_PAIR")) d.pair = atoi(e);  // test hook, as in sv_op_gemm_bf16
+  sv::GemmPlan plan;
+  SV_TRY(sv::gemm_plan(d, &plan));
+  return sv::gemm_launch(plan, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int sv_op_conv_gemm_plan_info(int32_t B, int32_t H, int32_t W, int32_t C, int32_t k, int32_t stride, int32_t pad, int32_t N, int32_t out_fp32,
+                                         int32_t has_residual, int32_t pair_request, int32_t num_sms, int32_t* conv_info, int32_t* gemm_info) {
+  SV_CHECK(conv_info != nullptr, "conv GEMM plan info: null output");
+  sv::ConvGeom g;
+  g.B = B; g.H = H; g.W = W; g.C = C; g.k = k; g.stride = stride; g.pad = pad;
+  SV_TRY(sv::check_conv_args(g));
+  const int32_t K = k * k * C, M = B * g.Ho() * g.Wo();
+  const int32_t v[SV_CONV_PLAN_INFO_LEN] = {sv::conv_gemm_im2col_ok(g) ? SV_GEMM_A_IM2COL : SV_GEMM_A_TILED, g.Ho(), g.Wo(), M, K};
+  std::copy(v, v + SV_CONV_PLAN_INFO_LEN, conv_info);
+  if (gemm_info == nullptr) return SV_OK;
+  return sv_op_gemm_plan_info(M, N, (K + 7) / 8 * 8, 0, out_fp32, has_residual, pair_request, num_sms, gemm_info);
 }
 
 extern "C" int sv_op_gemm_bf16_cat(const uint16_t* A, int64_t lda, const uint16_t* A2, int64_t lda2, int32_t K2, const uint16_t* W, int64_t ldw,

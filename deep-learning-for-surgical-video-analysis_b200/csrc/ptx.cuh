@@ -104,6 +104,18 @@ __device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* m
       : "memory");
 }
 
+// im2col-mode load from an NHWC tensor (map from cuTensorMapEncodeIm2col): pixelsPerColumn pixels, channelsPerPixel channels from c,
+// starting at pixel (w, h, n) and walking the map's bounding box with its element strides (row by row, then image by image); each
+// pixel is read at (w + off_w, h + off_h).  Pixels outside the tensor (conv padding, images past the last) are zero-filled.
+__device__ __forceinline__ void tma_load_im2col_4d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int32_t c, int32_t w, int32_t h, int32_t n,
+                                                   uint16_t off_w, uint16_t off_h) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.shared::cluster.global.im2col.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2], {%7, %8};"
+      :
+      : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c), "r"(w), "r"(h), "r"(n), "h"(off_w), "h"(off_h)
+      : "memory");
+}
+
 // ---------------------------------------------------------------- tcgen05 / TMEM
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_result, uint32_t ncols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)), "r"(ncols) : "memory");
@@ -181,6 +193,15 @@ __device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const CUtensorM
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       :
       : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0), "r"(c1)
+      : "memory");
+}
+__device__ __forceinline__ void tma_load_im2col_4d_pair(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int32_t c, int32_t w, int32_t h,
+                                                        int32_t n, uint16_t off_w, uint16_t off_h) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.im2col.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2], {%7, %8};"
+      :
+      : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar) & kPeerBitMask), "r"(c), "r"(w), "r"(h), "r"(n),
+        "h"(off_w), "h"(off_h)
       : "memory");
 }
 __device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_result, uint32_t ncols) {

@@ -142,6 +142,45 @@ def gemm_plan_info(M: int, N: int, K: int, K2: int = 0, out_fp32: bool = False, 
     return d
 
 
+def conv_gemm(x: torch.Tensor, w: torch.Tensor, k: int, stride: int, pad: int, bias: Optional[torch.Tensor] = None, act: int = 0,
+              residual: Optional[torch.Tensor] = None, out_dtype: torch.dtype = torch.bfloat16, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Convolution as an implicit GEMM (sv_op_conv_gemm_bf16): x [B,H,W,C] bf16 NHWC (C % 64 == 0), w [N, k*k*C] bf16 in (kh, kw, cin)
+    order (row stride may exceed k*k*C) -> out [B*Ho*Wo, N] = act(im2col(x) @ w.T + bias) (+ residual), rows in (b, oh, ow) order.
+    Bit-identical to gemm_bf16(im2col(x, k, stride, pad), w, ...) without the im2col buffer."""
+    _require_cuda(x, w, bias, residual, out)
+    assert x.dtype == torch.bfloat16 and w.dtype == torch.bfloat16 and x.is_contiguous() and w.stride(1) == 1
+    B, H, W, C = x.shape
+    M = B * ((H + 2 * pad - k) // stride + 1) * ((W + 2 * pad - k) // stride + 1)
+    N = w.shape[0]
+    if out is None:
+        out = torch.empty((M, N), dtype=out_dtype, device=x.device)
+    assert out.stride(1) == 1 and out.dtype in (torch.bfloat16, torch.float32)
+    rc = _native.lib().sv_op_conv_gemm_bf16(_ptr(x), B, H, W, C, k, stride, pad, _ptr(w), w.stride(0), N, _ptr(bias), act, _ptr(residual),
+                                            0 if residual is None else residual.stride(0), _ptr(out), out.stride(0), int(out.dtype == torch.float32),
+                                            _stream_ptr(x.device))
+    _native.check(rc, "sv_op_conv_gemm_bf16")
+    return out
+
+
+CONV_A_FORMS = ("tiled", "im2col")   # SV_GEMM_A_* in include/surgvid.h
+
+
+def conv_gemm_plan_info(B: int, H: int, W: int, C: int, k: int, stride: int, pad: int, N: int, out_fp32: bool = False, residual: bool = False,
+                        pair: int = -1, num_sms: int = 148) -> dict:
+    """How a convolution runs (sv_op_conv_gemm_plan_info; host only): `a_form` "im2col" (conv_gemm reads the NHWC input through an
+    im2col-mode TMA map) or "tiled" (not eligible: im2col buffer + gemm_bf16), Ho, Wo, M, K, and under "gemm" the GEMM's plan
+    (gemm_plan_info's fields)."""
+    ci = (ctypes.c_int32 * 5)()
+    gi = (ctypes.c_int32 * len(GEMM_PLAN_FIELDS))()
+    _native.check(_native.lib().sv_op_conv_gemm_plan_info(B, H, W, C, k, stride, pad, N, int(out_fp32), int(residual), pair, num_sms, ci, gi),
+                  "sv_op_conv_gemm_plan_info")
+    d = dict(zip(("a_form", "Ho", "Wo", "M", "K"), ci))
+    d["a_form"] = CONV_A_FORMS[d["a_form"]]
+    d["gemm"] = dict(zip(GEMM_PLAN_FIELDS, gi))
+    d["gemm"]["epilogue"] = GEMM_EPILOGUES[d["gemm"]["epilogue"]]
+    return d
+
+
 def gemm_bf16_cat(a: torch.Tensor, a2: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None, act: int = 0,
                   residual: Optional[torch.Tensor] = None, out_dtype: torch.dtype = torch.bfloat16, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """out = act(cat([a, a2], 1) @ w.T + bias) (+ residual) without building the concatenation; a [M,K1] (K1 % 64 == 0), a2 [M,K2] bf16

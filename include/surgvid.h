@@ -219,6 +219,27 @@ int sv_op_gemm_bf16(const uint16_t* A, int64_t lda, const uint16_t* W, int64_t l
 int sv_op_gemm_plan_info(int32_t M, int32_t N, int32_t K, int32_t K2, int32_t out_fp32, int32_t has_residual, int32_t pair_request,
                          int32_t num_sms, int32_t* info);
 
+/* Convolution as an implicit GEMM: out[M,N] = act(im2col(x) * W[N,K]^T + bias) (+ residual) with no im2col buffer.  x is the NHWC bf16
+ * input [B, H, W, C] (16-byte aligned, rows of C contiguous), k x k taps, stride, symmetric zero padding pad; M = B * Ho * Wo with
+ * Ho = (H + 2 pad - k) / stride + 1 (Wo likewise), output row m = (b, oh, ow); K = k * k * C in (kh, kw, cin) order, the layout
+ * sv_op_im2col gathers and packed conv weights use.  The GEMM reads its A tiles through an im2col-mode TMA map (one tap and 64 channels
+ * per k-block); the result is bit-identical to sv_op_im2col + sv_op_gemm_bf16.  Epilogue options (bias, act, residual, out_fp32, ldc,
+ * ldr) as sv_op_gemm_bf16; ldw >= K.  Needs C % 64 == 0, stride <= 8 and -pad, pad - (k - 1) within [-128, 127]: other geometries ->
+ * SV_ERR_UNSUPPORTED (gather with sv_op_im2col instead).  Bad arguments -> SV_ERR_INVALID, checked before the device is touched. */
+int sv_op_conv_gemm_bf16(const uint16_t* x, int32_t B, int32_t H, int32_t W, int32_t C, int32_t k, int32_t stride, int32_t pad,
+                         const uint16_t* Wt, int64_t ldw, int32_t N, const float* bias, int32_t act, const float* residual, int64_t ldr,
+                         void* out, int64_t ldc, int32_t out_fp32, void* stream);
+
+/* Host-only plan query for a convolution (touches neither device nor driver).  conv_info[SV_CONV_PLAN_INFO_LEN]: 0 A operand form
+ * (SV_GEMM_A_IM2COL: sv_op_conv_gemm_bf16 runs it; SV_GEMM_A_TILED: not eligible, the im2col buffer + 2-D tiled A map path), 1 Ho,
+ * 2 Wo, 3 M = B * Ho * Wo, 4 K = k * k * C.  gemm_info (may be NULL): sv_op_gemm_plan_info of that GEMM (K rounded up to a multiple
+ * of 8 on the tiled path).  Bad arguments -> SV_ERR_INVALID. */
+#define SV_GEMM_A_TILED 0
+#define SV_GEMM_A_IM2COL 1
+#define SV_CONV_PLAN_INFO_LEN 5
+int sv_op_conv_gemm_plan_info(int32_t B, int32_t H, int32_t W, int32_t C, int32_t k, int32_t stride, int32_t pad, int32_t N, int32_t out_fp32,
+                              int32_t has_residual, int32_t pair_request, int32_t num_sms, int32_t* conv_info, int32_t* gemm_info);
+
 /* LayerNorm over the last dim of fp32 [rows, C] -> optional fp32 and/or bf16 outputs (either may be NULL). */
 int sv_op_layernorm(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int32_t C,
                     float* out_f32, uint16_t* out_bf16, void* stream);
