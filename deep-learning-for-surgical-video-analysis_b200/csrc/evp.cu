@@ -17,6 +17,8 @@
 #include <memory>
 #include <utility>
 #include <string>
+#include <type_traits>
+#include <variant>
 #include <vector>
 
 #include "gemm.cuh"
@@ -57,33 +59,104 @@ struct CrossW {
   Norm norm;
 };
 
+// profile classes (sv_evp_get_profile, the `kind` column of sv_evp_dump_profile); the order is part of the ABI
 enum OpKind { OP_GEMM, OP_LN, OP_IM2COL, OP_DWCONV, OP_ATTN, OP_GAUSS, OP_BILINEAR, OP_MEAN, OP_STEM, OP_KINDS };
-enum Ext { EXT_NONE = 0, EXT_X, EXT_SEG, EXT_FLOW, EXT_OUT };
+
+// The pointers of one forward call for one micro-batch: a plan is built once and replayed on every call's inputs and outputs.
+struct CallIO {
+  const float *x, *seg, *flow; float* out;
+  float* const* maps;  // per encoder block, where this micro-batch's attention maps go (capture plans only)
+};
+// where im2col and the stem read their fp32 NCHW input: a workspace buffer, or the call's x or flow
+enum Ext { EXT_NONE, EXT_X, EXT_FLOW };
+const float* nchw_input(Ext ext, const float* ws, const CallIO& io) { return ext == EXT_X ? io.x : ext == EXT_FLOW ? io.flow : ws; }
+struct ProfCols { long long M; int i[5]; };  // columns M, i0..i4 of a non-GEMM row of sv_evp_dump_profile
+
+// One record per launch form: its launcher's arguments under the launcher's names and in its order, and its profile class.
+struct GemmOp {  // GEMM or implicit-GEMM conv
+  static constexpr OpKind kind = OP_GEMM;
+  GemmPlan plan;
+  int launch(const CallIO&, cudaStream_t st) const { return gemm_launch(plan, st); }
+};
+struct LayerNormOp {  // out_patch: optional second bf16 copy in the sr conv's patch order (pH x pW grid, psr x psr patches)
+  static constexpr OpKind kind = OP_LN;
+  const float *x, *gamma, *beta; float eps; int64_t rows; int C; float* out_f32; bf16 *out_bf16, *out_patch; int pH, pW, psr;
+  int launch(const CallIO&, cudaStream_t st) const { return launch_layernorm_patch(x, gamma, beta, eps, rows, C, out_f32, out_bf16, out_patch, pH, pW, psr, st); }
+  ProfCols cols() const { return {rows, {C, pH, pW, psr, 0}}; }
+};
+struct Im2colOp {
+  static constexpr OpKind kind = OP_IM2COL;
+  Ext ext; const float* src_nchw_f32; const bf16* src_nhwc_bf16; int B, Cin, H, W, k, stride, pad; bf16* out; int64_t ldo;
+  int launch(const CallIO& io, cudaStream_t st) const {
+    return launch_im2col(nchw_input(ext, src_nchw_f32, io), src_nhwc_bf16, B, Cin, H, W, k, stride, pad, out, ldo, st);
+  }
+  ProfCols cols() const { return {ldo, {B, Cin, H, W, k}}; }
+};
+struct DwconvTmaOp {
+  static constexpr OpKind kind = OP_DWCONV;
+  DwconvPlan plan;
+  int launch(const CallIO&, cudaStream_t st) const { return dwconv_tma_launch(plan, st); }
+  ProfCols cols() const { return {plan.ldo, {plan.B, plan.H, plan.W, plan.C, 0}}; }
+};
+struct DwconvOp {  // channel counts the TMA form does not take (dwconv_tma_supported)
+  static constexpr OpKind kind = OP_DWCONV;
+  const bf16* x; const float *w9c, *bias; int B, H, W, C; bf16* out; int64_t ldo;
+  int launch(const CallIO&, cudaStream_t st) const { return launch_dwconv3x3_gelu(x, w9c, bias, B, H, W, C, out, ldo, st); }
+  ProfCols cols() const { return {ldo, {B, H, W, C, 0}}; }
+};
+struct AttnTcOp {
+  static constexpr OpKind kind = OP_ATTN;
+  AttnTcPlan plan;
+  int64_t ldq; int hd;  // for the profile only: the plan keeps neither
+  int launch(const CallIO&, cudaStream_t st) const { return attention_tc_launch(plan, st); }
+  ProfCols cols() const { return {ldq, {plan.B, plan.heads, plan.Nq, plan.Nkv, hd}}; }
+};
+struct AttnOp {  // mma.sync kernels: head_dim 20/32/40, or SURGVID_ATTN_TC=0
+  static constexpr OpKind kind = OP_ATTN;
+  const bf16* q; int64_t ldq; const bf16* k; int64_t ldk; const bf16* v; int64_t ldv; bf16* o; int64_t ldo; int B, heads, Nq, Nkv, hd; float scale;
+  int launch(const CallIO&, cudaStream_t st) const { return launch_attention(q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, hd, scale, st); }
+  ProfCols cols() const { return {ldq, {B, heads, Nq, Nkv, hd}}; }
+};
+struct ProbsOp {  // softmax(Q K^T * scale) of encoder block `block` into the call's maps[block]
+  static constexpr OpKind kind = OP_ATTN;
+  const bf16* q; int64_t ldq; const bf16* k; int64_t ldk; int B, heads, Nq, Nkv, hd; float scale; int block;
+  int launch(const CallIO& io, cudaStream_t st) const { return launch_attention_probs(q, ldq, k, ldk, B, heads, Nq, Nkv, hd, scale, io.maps[block], st); }
+  ProfCols cols() const { return {ldq, {B, heads, Nq, Nkv, hd}}; }
+};
+struct GaussOp {  // of the call's seg
+  static constexpr OpKind kind = OP_GAUSS;
+  float* out; int planes, H, W;
+  int launch(const CallIO& io, cudaStream_t st) const { return launch_gauss5x5(io.seg, out, planes, H, W, st); }
+  ProfCols cols() const { return {0, {planes, H, W, 0, 0}}; }
+};
+struct BilinearOp {
+  static constexpr OpKind kind = OP_BILINEAR;
+  const bf16* x; int B, H, W, C, Ho, Wo; bf16* out; int64_t ldo;
+  int launch(const CallIO&, cudaStream_t st) const { return launch_bilinear_tokens(x, B, H, W, C, Ho, Wo, out, ldo, st); }
+  ProfCols cols() const { return {ldo, {B, H, W, C, Ho}}; }
+};
+struct MeanOp {  // into the call's out
+  static constexpr OpKind kind = OP_MEAN;
+  const float* x; int B, tokens, C;
+  int launch(const CallIO& io, cudaStream_t st) const { return launch_token_mean(x, B, tokens, C, io.out, st); }
+  ProfCols cols() const { return {0, {B, tokens, C, 0, 0}}; }
+};
+struct StemOp {  // mode 0: LayerNorm, 1: ReLU
+  static constexpr OpKind kind = OP_STEM;
+  Ext ext; const float* src; const bf16* w; int ldw; const float *bias, *gamma, *beta; float eps; int mode; int B, Cin, H, W, Cout;
+  float* out_f32; bf16* out_bf16;
+  int launch(const CallIO& io, cudaStream_t st) const {
+    return launch_stem_conv(nchw_input(ext, src, io), w, ldw, bias, gamma, beta, eps, mode, B, Cin, H, W, Cout, out_f32, out_bf16, st);
+  }
+  ProfCols cols() const { return {0, {B, Cin, H, W, Cout}}; }
+};
 
 struct Op {
-  OpKind kind;
-  GemmPlan gemm;
-  DwconvPlan dw;
-  bool dw_tma = false;
-  AttnTcPlan attn_tc;
-  bool attn_tc_on = false;
-  bool probs = false;  // OP_ATTN that writes the attention maps of encoder block i[5] (capture plans only)
-  // generic arguments (meaning depends on kind)
-  const void* src = nullptr;
-  const void* src2 = nullptr;
-  const void* src3 = nullptr;
-  void* dst = nullptr;
-  void* dst2 = nullptr;
-  void* dst3 = nullptr;
-  const float* p0 = nullptr;
-  const float* p1 = nullptr;
-  int64_t l0 = 0, l1 = 0, l2 = 0, l3 = 0;
-  int i[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  float f0 = 0.f;
-  int ext_src = EXT_NONE, ext_dst = EXT_NONE;
+  std::variant<GemmOp, LayerNormOp, Im2colOp, DwconvTmaOp, DwconvOp, AttnTcOp, AttnOp, ProbsOp, GaussOp, BilinearOp, MeanOp, StemOp> rec;
   double alg_bytes = 0.0;         // algorithmic HBM bytes of this launch (operands + results once)
   mutable double prof_ms = 0.0;   // filled only in profiling mode
   mutable long long prof_n = 0;
+  OpKind kind() const { return std::visit([](const auto& r) { return r.kind; }, rec); }
 };
 
 struct Tap {
@@ -464,129 +537,108 @@ struct Builder {
   Builder(sv_evp* hh, Plan* p, void* ws) : h(hh), plan(p), arena(ws) {}
   bool dry() const { return plan == nullptr; }
   const bf16* W(const Lin& l) const { return h->d_wb + l.w; }
-  const bf16* W_(const Lin& l) const { return h->d_wb + l.w; }
   const float* Bf(const Lin& l) const { return l.has_bias ? h->d_wf + l.b : nullptr; }
   const float* F(size_t off) const { return h->d_wf + off; }
 
-  void push(const Op& op) {
+  template <typename R>
+  void push(const R& rec, double alg_bytes) {
     if (dry() || status != SV_OK) return;
-    plan->ops.push_back(op);
-    plan->bytes_by_kind[op.kind] += op.alg_bytes;
+    plan->ops.push_back(Op{rec, alg_bytes});
+    plan->bytes_by_kind[R::kind] += alg_bytes;
+  }
+  // the step gemm() and conv() share: the result and the A operand (a_bytes from d.A) must lie inside one workspace buffer each
+  void push_gemm(const GemmDesc& d, size_t a_bytes, double alg_bytes, const char* bounds_error) {
+    if (dry() || status != SV_OK) return;
+    if (!arena.contains(d.out, (static_cast<size_t>(d.M - 1) * d.ldc + d.N) * (d.out_fp32 ? 4 : 2)) || !arena.contains(d.A, a_bytes)) {
+      status = fail(SV_ERR_STATE, bounds_error);
+      return;
+    }
+    GemmOp op;
+    status = gemm_plan(d, &op.plan);
+    plan->gemm_flops += op.plan.flops;
+    push(op, alg_bytes);
   }
 
   // A2/lda2/K2: optional second A segment for the last K2 columns of K (see GemmDesc)
   void gemm(const bf16* A, int64_t lda, const Lin& l, int M, int act, const float* resid, int64_t ldr, void* out, int64_t ldc, int out_fp32,
             const bf16* A2 = nullptr, int64_t lda2 = 0, int K2 = 0) {
-    if (dry() || status != SV_OK) return;
-    {  // every GEMM result (and its A operand) must lie inside one workspace buffer
-      const size_t out_bytes = (static_cast<size_t>(M - 1) * ldc + l.N) * (out_fp32 ? 4 : 2);
-      const size_t a_bytes = (static_cast<size_t>(M - 1) * lda + (l.ldw - K2)) * 2;
-      if (!arena.contains(out, out_bytes) || !arena.contains(A, a_bytes)) {
-        status = fail(SV_ERR_STATE, "evp: internal error: a GEMM of the plan addresses memory outside its workspace buffer");
-        return;
-      }
-    }
     GemmDesc d;
     d.A = A; d.lda = lda; d.W = W(l); d.ldw = l.ldw; d.M = M; d.N = l.N; d.bias = Bf(l); d.act = act;
     d.A2 = A2; d.lda2 = lda2; d.K2 = K2;
     d.K = l.ldw;  // K padded to a multiple of 8; pad columns are zero in both the packed weight and the im2col buffer
     d.residual = resid; d.ldr = ldr; d.out = out; d.ldc = ldc; d.out_fp32 = out_fp32;
-    Op op;
-    op.kind = OP_GEMM;
-    status = gemm_plan(d, &op.gemm);
-    plan->gemm_flops += op.gemm.flops;
-    op.alg_bytes = 2.0 * M * d.K + 2.0 * l.N * d.K + static_cast<double>(M) * l.N * (out_fp32 ? 4 : 2) + (resid ? 4.0 * M * l.N : 0.0);
-    push(op);
+    push_gemm(d, (static_cast<size_t>(M - 1) * lda + (l.ldw - K2)) * 2,
+              2.0 * M * d.K + 2.0 * l.N * d.K + static_cast<double>(M) * l.N * (out_fp32 ? 4 : 2) + (resid ? 4.0 * M * l.N : 0.0),
+              "evp: internal error: a GEMM of the plan addresses memory outside its workspace buffer");
   }
   // convolution of an NHWC bf16 input with (kh, kw, cin)-packed weights: an implicit GEMM whose A tiles the TMA gathers through an
   // im2col-mode map when the geometry allows (conv_gemm_im2col_ok), else an im2col gather into `col` and a GEMM over it
   void conv(const bf16* x, const ConvGeom& cg, const Lin& l, int act, void* out, int64_t ldc, int out_fp32, bf16* col) {
     const int M = cg.B * cg.Ho() * cg.Wo();
     if (!conv_gemm_im2col_ok(cg)) {
-      im2col(nullptr, x, cg.B, cg.C, cg.H, cg.W, cg.k, cg.stride, cg.pad, col, l.ldw);
+      im2col(EXT_NONE, nullptr, x, cg.B, cg.C, cg.H, cg.W, cg.k, cg.stride, cg.pad, col, l.ldw);
       gemm(col, l.ldw, l, M, act, nullptr, 0, out, ldc, out_fp32);
       return;
     }
-    if (dry() || status != SV_OK) return;
     const size_t x_bytes = static_cast<size_t>(cg.B) * cg.H * cg.W * cg.C * 2;
-    if (!arena.contains(out, (static_cast<size_t>(M - 1) * ldc + l.N) * (out_fp32 ? 4 : 2)) || !arena.contains(x, x_bytes)) {
-      status = fail(SV_ERR_STATE, "evp: internal error: a conv GEMM of the plan addresses memory outside its workspace buffer");
-      return;
-    }
     GemmDesc d;
     d.A = x; d.conv = cg; d.W = W(l); d.ldw = l.ldw; d.M = M; d.N = l.N; d.K = l.ldw; d.bias = Bf(l); d.act = act;
     d.out = out; d.ldc = ldc; d.out_fp32 = out_fp32;
-    Op op;
-    op.kind = OP_GEMM;
-    status = gemm_plan(d, &op.gemm);
-    plan->gemm_flops += op.gemm.flops;
-    op.alg_bytes = static_cast<double>(x_bytes) + 2.0 * l.N * d.K + static_cast<double>(M) * l.N * (out_fp32 ? 4 : 2);
-    push(op);
+    push_gemm(d, x_bytes, static_cast<double>(x_bytes) + 2.0 * l.N * d.K + static_cast<double>(M) * l.N * (out_fp32 ? 4 : 2),
+              "evp: internal error: a conv GEMM of the plan addresses memory outside its workspace buffer");
   }
   void ln(const float* x, const Norm& n, float eps, int64_t rows, float* of, bf16* ob, bf16* patch = nullptr, int pH = 0, int pW = 0, int psr = 0) {
-    Op op; op.kind = OP_LN; op.src = x; op.p0 = F(n.g); op.p1 = F(n.b); op.f0 = eps; op.l0 = rows; op.i[0] = n.C; op.dst = of; op.dst2 = ob;
-    op.dst3 = patch; op.i[1] = pH; op.i[2] = pW; op.i[3] = psr;
-    op.alg_bytes = static_cast<double>(rows) * n.C * (4 + (of ? 4 : 0) + (ob ? 2 : 0) + (patch ? 2 : 0));
-    push(op);
+    push(LayerNormOp{x, F(n.g), F(n.b), eps, rows, n.C, of, ob, patch, pH, pW, psr},
+         static_cast<double>(rows) * n.C * (4 + (of ? 4 : 0) + (ob ? 2 : 0) + (patch ? 2 : 0)));
   }
-  void im2col(const float* nchw, const bf16* nhwc, int B, int Cin, int H, int W, int k, int stride, int pad, bf16* out, int64_t ldo, int ext = EXT_NONE) {
-    Op op; op.kind = OP_IM2COL; op.src = nchw; op.src2 = nhwc; op.dst = out; op.l0 = ldo; op.ext_src = ext;
-    op.i[0] = B; op.i[1] = Cin; op.i[2] = H; op.i[3] = W; op.i[4] = k; op.i[5] = stride; op.i[6] = pad;
-    op.alg_bytes = static_cast<double>(B) * Cin * H * W * (nhwc ? 2 : 4) +
-                   2.0 * B * conv_out_dim(H, k, stride, pad) * conv_out_dim(W, k, stride, pad) * static_cast<double>(ldo);
-    push(op);
+  void im2col(Ext ext, const float* nchw, const bf16* nhwc, int B, int Cin, int H, int W, int k, int stride, int pad, bf16* out, int64_t ldo) {
+    push(Im2colOp{ext, nchw, nhwc, B, Cin, H, W, k, stride, pad, out, ldo},
+         static_cast<double>(B) * Cin * H * W * (nhwc ? 2 : 4) +
+             2.0 * B * conv_out_dim(H, k, stride, pad) * conv_out_dim(W, k, stride, pad) * static_cast<double>(ldo));
   }
   void dwconv(const bf16* x, size_t w, size_t b, int B, int H, int W, int C, bf16* out, int64_t ldo) {
-    Op op; op.kind = OP_DWCONV; op.src = x; op.p0 = F(w); op.p1 = F(b); op.dst = out; op.i[0] = B; op.i[1] = H; op.i[2] = W; op.i[3] = C;
-    op.l0 = ldo;
-    op.alg_bytes = 2.0 * 2.0 * B * H * W * static_cast<double>(C);
-    if (!dry() && status == SV_OK && dwconv_tma_supported(C)) {
-      op.dw_tma = true;
-      status = dwconv_tma_plan(x, F(w), F(b), B, H, W, C, out, ldo, &op.dw);
-    }
-    push(op);
+    if (dry() || status != SV_OK) return;
+    const double bytes = 2.0 * 2.0 * B * H * W * static_cast<double>(C);
+    if (!dwconv_tma_supported(C)) return push(DwconvOp{x, F(w), F(b), B, H, W, C, out, ldo}, bytes);
+    DwconvTmaOp op;
+    status = dwconv_tma_plan(x, F(w), F(b), B, H, W, C, out, ldo, &op.plan);
+    push(op, bytes);
   }
   void attn(const bf16* q, int64_t ldq, const bf16* k, int64_t ldk, const bf16* v, int64_t ldv, bf16* o, int64_t ldo, int B, int heads, int Nq, int Nkv, int hd) {
-    Op op; op.kind = OP_ATTN; op.src = q; op.src2 = k; op.src3 = v; op.dst = o; op.l0 = ldq; op.l1 = ldk; op.l2 = ldv; op.l3 = ldo;
-    op.i[0] = B; op.i[1] = heads; op.i[2] = Nq; op.i[3] = Nkv; op.i[4] = hd; op.f0 = 1.0f / sqrtf(static_cast<float>(hd));
-    op.alg_bytes = 2.0 * B * heads * hd * (2.0 * Nq + 2.0 * Nkv);
-    if (!dry() && status == SV_OK && attention_tc_enabled() && attention_tc_supported(hd, Nkv, ldq, ldk, ldv, ldo, q, k, v, o)) {
-      op.attn_tc_on = true;
-      status = attention_tc_plan(q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, op.f0, &op.attn_tc);
-    }
-    push(op);
+    if (dry() || status != SV_OK) return;
+    const float scale = 1.0f / sqrtf(static_cast<float>(hd));
+    const double bytes = 2.0 * B * heads * hd * (2.0 * Nq + 2.0 * Nkv);
+    if (!attention_tc_enabled() || !attention_tc_supported(hd, Nkv, ldq, ldk, ldv, ldo, q, k, v, o))
+      return push(AttnOp{q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, hd, scale}, bytes);
+    AttnTcOp op{{}, ldq, hd};
+    status = attention_tc_plan(q, ldq, k, ldk, v, ldv, o, ldo, B, heads, Nq, Nkv, scale, &op.plan);
+    push(op, bytes);
   }
   // P = softmax(Q K^T * scale) of encoder block `block` into the caller's maps buffer (resolved per call, see run_plan)
   void probs(const bf16* q, int64_t ldq, const bf16* k, int64_t ldk, int B, int heads, int Nq, int Nkv, int hd, int block) {
-    Op op; op.kind = OP_ATTN; op.probs = true; op.src = q; op.src2 = k; op.l0 = ldq; op.l1 = ldk;
-    op.i[0] = B; op.i[1] = heads; op.i[2] = Nq; op.i[3] = Nkv; op.i[4] = hd; op.i[5] = block; op.f0 = 1.0f / sqrtf(static_cast<float>(hd));
-    op.alg_bytes = 2.0 * B * heads * hd * (static_cast<double>(Nq) + Nkv) + 4.0 * B * heads * static_cast<double>(Nq) * Nkv;
-    push(op);
+    push(ProbsOp{q, ldq, k, ldk, B, heads, Nq, Nkv, hd, 1.0f / sqrtf(static_cast<float>(hd)), block},
+         2.0 * B * heads * hd * (static_cast<double>(Nq) + Nkv) + 4.0 * B * heads * static_cast<double>(Nq) * Nkv);
   }
-  void gauss(float* out, int planes, int H, int W) {
-    Op op; op.kind = OP_GAUSS; op.dst = out; op.i[0] = planes; op.i[1] = H; op.i[2] = W; op.ext_src = EXT_SEG;
-    op.alg_bytes = 8.0 * planes * H * W;
-    push(op);
-  }
-  void bilinear(const bf16* x, int B, int H, int W, int C, int Ho, int Wo, bf16* out, int64_t ldo) {
-    Op op; op.kind = OP_BILINEAR; op.src = x; op.dst = out; op.l0 = ldo; op.i[0] = B; op.i[1] = H; op.i[2] = W; op.i[3] = C; op.i[4] = Ho; op.i[5] = Wo;
-    push(op);
-  }
-  void mean(const float* x, int B, int tokens, int C) {
-    Op op; op.kind = OP_MEAN; op.src = x; op.i[0] = B; op.i[1] = tokens; op.i[2] = C; op.ext_dst = EXT_OUT;
-    push(op);
-  }
+  void gauss(float* out, int planes, int H, int W) { push(GaussOp{out, planes, H, W}, 8.0 * planes * H * W); }
+  void bilinear(const bf16* x, int B, int H, int W, int C, int Ho, int Wo, bf16* out, int64_t ldo) { push(BilinearOp{x, B, H, W, C, Ho, Wo, out, ldo}, 0.0); }
+  void mean(const float* x, int B, int tokens, int C) { push(MeanOp{x, B, tokens, C}, 0.0); }
   // fused k7s4p3 conv on an fp32 NCHW input + LayerNorm (norm != nullptr) or ReLU
-  void stem(const float* src, int ext, const Lin& l, const Norm* norm, int B, int Cin, int H, int W, float* of, bf16* ob) {
-    Op op; op.kind = OP_STEM; op.src = src; op.ext_src = ext; op.src2 = W_(l); op.p0 = Bf(l); op.dst = of; op.dst2 = ob;
-    op.p1 = norm ? F(norm->g) : nullptr; op.src3 = norm ? F(norm->b) : nullptr;
-    op.i[0] = B; op.i[1] = Cin; op.i[2] = H; op.i[3] = W; op.i[4] = l.N; op.i[5] = l.ldw; op.i[6] = norm ? 0 : 1; op.f0 = 1e-5f;
+  void stem(Ext ext, const float* src, const Lin& l, const Norm* norm, int B, int Cin, int H, int W, float* of, bf16* ob) {
     const double outpx = static_cast<double>(B) * conv_out_dim(H, 7, 4, 3) * conv_out_dim(W, 7, 4, 3);
-    op.alg_bytes = 4.0 * B * Cin * H * W + outpx * l.N * ((of ? 4 : 0) + (ob ? 2 : 0));
-    push(op);
+    push(StemOp{ext, src, this->W(l), l.ldw, Bf(l), norm ? F(norm->g) : nullptr, norm ? F(norm->b) : nullptr, 1e-5f, norm ? 0 : 1, B, Cin, H, W, l.N, of, ob},
+         4.0 * B * Cin * H * W + outpx * l.N * ((of ? 4 : 0) + (ob ? 2 : 0)));
   }
   void tap(const std::string& name, const bf16* p, int64_t elems) { if (!dry()) plan->taps[name] = Tap{p, elems}; }
 };
+
+// MotionGuidedCrossAttention is nn.MultiheadAttention(dim, 8 heads) (mix_transformer_evp.py:866-870): C/8 of stages 3 and 4 is its head_dim
+bool flow_supported(const sv_evp_cfg& c) {
+  for (int j = 2; j < 4; ++j) {
+    const int hd = c.embed_dims[j] / 8;
+    if (c.embed_dims[j] % 8 != 0 || (hd != 20 && hd != 32 && hd != 40 && hd != 64)) return false;
+  }
+  return true;
+}
 
 // Builds (or only sizes, when plan == nullptr) the launch schedule for n frames of HxW.
 int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, bool capture, size_t* bytes_out) {
@@ -598,13 +650,7 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
   for (int s = 0; s < 4; ++s) {
     if (g[s].H < 1 || g[s].W < 1 || g[s].Hk < 1 || g[s].Wk < 1) return fail(SV_ERR_INVALID, "evp: input too small for the 4-stage pyramid");
   }
-  if (with_flow) {  // MotionGuidedCrossAttention is nn.MultiheadAttention(dim, 8 heads) (mix_transformer_evp.py:866-870)
-    for (int j = 2; j < 4; ++j) {
-      const int hd = c.embed_dims[j] / 8;
-      if (c.embed_dims[j] % 8 != 0 || (hd != 20 && hd != 32 && hd != 40 && hd != 64))
-        return fail(SV_ERR_UNSUPPORTED, "evp: flow cross-attention head_dim (C/8) must be 20, 32, 40 or 64");
-    }
-  }
+  if (with_flow && !flow_supported(c)) return fail(SV_ERR_UNSUPPORTED, "evp: flow cross-attention head_dim (C/8) must be 20, 32, 40 or 64");
   const int E = c.embedding_dim;
   const int ks[4] = {7, 3, 3, 3}, strd[4] = {4, 2, 2, 2};
   const int fch[5] = {2, 64, 128, c.embed_dims[2], c.embed_dims[3]};
@@ -681,10 +727,10 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
       const StageW& S = h->st[s];
       const int M = n * g[s].N;
       if (s == 0 && stem_conv_supported(cinp, S.hc.N, S.hc.ldw)) {
-        b.stem(seg_g, EXT_NONE, S.hc, &S.hc_norm, n, cinp, hh, ww, hc_f32[s], hc_b16[s]);
+        b.stem(EXT_NONE, seg_g, S.hc, &S.hc_norm, n, cinp, hh, ww, hc_f32[s], hc_b16[s]);
       } else {
         if (s == 0) {
-          b.im2col(seg_g, nullptr, n, cinp, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.hc.ldw);
+          b.im2col(EXT_NONE, seg_g, nullptr, n, cinp, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.hc.ldw);
           b.gemm(col, S.hc.ldw, S.hc, M, ACT_NONE, nullptr, 0, conv_out, g[s].Cp, 1);
         } else {
           b.conv(hc_b16[s - 1], geom(n, hh, ww, cinp, ks[s], strd[s], ks[s] / 2), S.hc, ACT_NONE, conv_out, g[s].Cp, 1, col);
@@ -704,10 +750,10 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
       const int M = n * G.N, Mk = n * G.Nkv, C = G.C;
       const int cin = s == 0 ? 3 : c.embed_dims[s - 1];
       if (s == 0 && stem_conv_supported(cin, S.pe.N, S.pe.ldw)) {
-        b.stem(nullptr, EXT_X, S.pe, &S.pe_norm, n, cin, hh, ww, x, xn);
+        b.stem(EXT_X, nullptr, S.pe, &S.pe_norm, n, cin, hh, ww, x, xn);
       } else {
         if (s == 0) {
-          b.im2col(nullptr, nullptr, n, cin, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.pe.ldw, EXT_X);
+          b.im2col(EXT_X, nullptr, nullptr, n, cin, hh, ww, ks[s], strd[s], ks[s] / 2, col, S.pe.ldw);
           b.gemm(col, S.pe.ldw, S.pe, M, ACT_NONE, nullptr, 0, conv_out, C, 1);
         } else {
           b.conv(c_b16[s - 1], geom(n, hh, ww, cin, ks[s], strd[s], ks[s] / 2), S.pe, ACT_NONE, conv_out, C, 1, col);
@@ -772,10 +818,10 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
       const Lin& L = h->flow[i];
       const int M = n * g[i].N;
       if (i == 0 && stem_conv_supported(2, L.N, L.ldw)) {
-        b.stem(nullptr, EXT_FLOW, L, nullptr, n, 2, hh, ww, nullptr, fl[i]);
+        b.stem(EXT_FLOW, nullptr, L, nullptr, n, 2, hh, ww, nullptr, fl[i]);
       } else {
         if (i == 0) {
-          b.im2col(nullptr, nullptr, n, 2, hh, ww, 7, 4, 3, col, L.ldw, EXT_FLOW);
+          b.im2col(EXT_FLOW, nullptr, nullptr, n, 2, hh, ww, 7, 4, 3, col, L.ldw);
           b.gemm(col, L.ldw, L, M, ACT_RELU, nullptr, 0, fl[i], fch[i + 1], 0);
         } else {
           b.conv(fl[i - 1], geom(n, hh, ww, fch[i], 3, 2, 1), L, ACT_RELU, fl[i], fch[i + 1], 0, col);
@@ -834,8 +880,7 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
   return b.status;
 }
 
-// maps: per encoder block, where this micro-batch's attention maps go (capture plans only)
-int run_plan(sv_evp* h, const Plan& p, const float* x, const float* seg, const float* flow, float* out, float* const* maps, cudaStream_t st) {
+int run_plan(sv_evp* h, const Plan& p, const CallIO& io, cudaStream_t st) {
   const bool prof = h->profile;
   if (prof) {
     while (h->prof_events.size() < 2 * p.ops.size()) {
@@ -846,52 +891,8 @@ int run_plan(sv_evp* h, const Plan& p, const float* x, const float* seg, const f
   }
   size_t op_idx = 0;
   for (const Op& op : p.ops) {
-    int rc = SV_OK;
     if (prof) SV_CUDA_OK(cudaEventRecord(h->prof_events[2 * op_idx], st));
-    switch (op.kind) {
-      case OP_GEMM: rc = gemm_launch(op.gemm, st); break;
-      case OP_LN:
-        rc = launch_layernorm_patch(static_cast<const float*>(op.src), op.p0, op.p1, op.f0, op.l0, op.i[0], static_cast<float*>(op.dst),
-                                    static_cast<bf16*>(op.dst2), static_cast<bf16*>(op.dst3), op.i[1], op.i[2], op.i[3], st);
-        break;
-      case OP_IM2COL: {
-        const float* nchw = static_cast<const float*>(op.src);
-        if (op.ext_src == EXT_X) nchw = x;
-        if (op.ext_src == EXT_FLOW) nchw = flow;
-        rc = launch_im2col(nchw, static_cast<const bf16*>(op.src2), op.i[0], op.i[1], op.i[2], op.i[3], op.i[4], op.i[5], op.i[6],
-                           static_cast<bf16*>(op.dst), op.l0, st);
-        break;
-      }
-      case OP_DWCONV:
-        if (op.dw_tma) { rc = dwconv_tma_launch(op.dw, st); break; }
-        rc = launch_dwconv3x3_gelu(static_cast<const bf16*>(op.src), op.p0, op.p1, op.i[0], op.i[1], op.i[2], op.i[3], static_cast<bf16*>(op.dst), op.l0, st);
-        break;
-      case OP_ATTN:
-        if (op.probs) {
-          rc = launch_attention_probs(static_cast<const bf16*>(op.src), op.l0, static_cast<const bf16*>(op.src2), op.l1, op.i[0], op.i[1], op.i[2],
-                                      op.i[3], op.i[4], op.f0, maps[op.i[5]], st);
-          break;
-        }
-        if (op.attn_tc_on) { rc = attention_tc_launch(op.attn_tc, st); break; }
-        rc = launch_attention(static_cast<const bf16*>(op.src), op.l0, static_cast<const bf16*>(op.src2), op.l1, static_cast<const bf16*>(op.src3),
-                              op.l2, static_cast<bf16*>(op.dst), op.l3, op.i[0], op.i[1], op.i[2], op.i[3], op.i[4], op.f0, st);
-        break;
-      case OP_GAUSS: rc = launch_gauss5x5(seg, static_cast<float*>(op.dst), op.i[0], op.i[1], op.i[2], st); break;
-      case OP_BILINEAR:
-        rc = launch_bilinear_tokens(static_cast<const bf16*>(op.src), op.i[0], op.i[1], op.i[2], op.i[3], op.i[4], op.i[5],
-                                    static_cast<bf16*>(op.dst), op.l0, st);
-        break;
-      case OP_STEM: {
-        const float* src = static_cast<const float*>(op.src);
-        if (op.ext_src == EXT_X) src = x;
-        if (op.ext_src == EXT_FLOW) src = flow;
-        rc = launch_stem_conv(src, static_cast<const bf16*>(op.src2), op.i[5], op.p0, op.p1, static_cast<const float*>(op.src3), op.f0, op.i[6],
-                              op.i[0], op.i[1], op.i[2], op.i[3], op.i[4], static_cast<float*>(op.dst), static_cast<bf16*>(op.dst2), st);
-        break;
-      }
-      case OP_MEAN: rc = launch_token_mean(static_cast<const float*>(op.src), op.i[0], op.i[1], op.i[2], out, st); break;
-      default: break;
-    }
+    const int rc = std::visit([&](const auto& r) { return r.launch(io, st); }, op.rec);
     if (rc != SV_OK) return rc;
     if (prof) SV_CUDA_OK(cudaEventRecord(h->prof_events[2 * op_idx + 1], st));
     ++op_idx;
@@ -902,8 +903,8 @@ int run_plan(sv_evp* h, const Plan& p, const float* x, const float* seg, const f
     for (size_t i = 0; i < p.ops.size(); ++i) {
       float ms = 0.f;
       SV_CUDA_OK(cudaEventElapsedTime(&ms, h->prof_events[2 * i], h->prof_events[2 * i + 1]));
-      h->prof_ms[p.ops[i].kind] += ms;
-      h->prof_n[p.ops[i].kind] += 1;
+      h->prof_ms[p.ops[i].kind()] += ms;
+      h->prof_n[p.ops[i].kind()] += 1;
       p.ops[i].prof_ms += ms;
       p.ops[i].prof_n += 1;
     }
@@ -996,16 +997,9 @@ int sv_evp_pack_weights(sv_evp_handle* h) {
 size_t sv_evp_workspace_bytes(const sv_evp_handle* h, int32_t micro_batch, int32_t H, int32_t W) {
   if (!h || micro_batch <= 0 || H <= 0 || W <= 0) return 0;
   size_t bytes = 0;
-  // sized for the larger of the two schedules (with the flow branch); configurations whose flow branch is unsupported
-  // (cross-attention head_dim, see build()) can only ever run without it
-  const bool flow_ok = [&] {
-    for (int j = 2; j < 4; ++j) {
-      const int hd = h->cfg.embed_dims[j] / 8;
-      if (h->cfg.embed_dims[j] % 8 != 0 || (hd != 20 && hd != 32 && hd != 40 && hd != 64)) return false;
-    }
-    return true;
-  }();
-  if (sv::build(const_cast<sv_evp*>(h), nullptr, nullptr, micro_batch, H, W, flow_ok, false, &bytes) != SV_OK) return 0;
+  // sized for the larger of the two schedules (with the flow branch); configurations whose flow branch is unsupported can only
+  // ever run without it
+  if (sv::build(const_cast<sv_evp*>(h), nullptr, nullptr, micro_batch, H, W, sv::flow_supported(h->cfg), false, &bytes) != SV_OK) return 0;
   return bytes;
 }
 
@@ -1054,8 +1048,9 @@ int evp_forward(sv_evp_handle* h, const float* x, const float* seg, const float*
     const size_t in_off = static_cast<size_t>(b0) * 3 * H * W;
     for (size_t k = 0; k < block_maps.size(); ++k)
       block_maps[k] = maps + off[k] + static_cast<int64_t>(b0) * dims[3 * k] * dims[3 * k + 1] * dims[3 * k + 2];
-    SV_TRY(run_plan(h, plan, x + in_off, seg + in_off, with_flow ? flow + static_cast<size_t>(b0) * 2 * H * W : nullptr,
-                    out_features + static_cast<size_t>(b0) * E, block_maps.data(), st));
+    const CallIO io{x + in_off, seg + in_off, with_flow ? flow + static_cast<size_t>(b0) * 2 * H * W : nullptr, out_features + static_cast<size_t>(b0) * E,
+                    block_maps.data()};
+    SV_TRY(run_plan(h, plan, io, st));
     h->last_plan = it->second.get();
   }
   return SV_OK;
@@ -1152,13 +1147,17 @@ int sv_evp_dump_profile(const sv_evp_handle* h, const char* path) {
     for (size_t i = 0; i < p.ops.size(); ++i) {
       const Op& op = p.ops[i];
       if (op.prof_n == 0) continue;
-      const GemmParams& g = op.gemm.p;
-      if (op.kind == OP_GEMM)
-        fprintf(f, "%d,%zu,%s,%d,%d,%d,%d,%d,%d,%d,%d,%d,0,0,0,0,0,%lld,%.6f\n", p.n, i, kinds[op.kind], g.M, g.N, g.K, g.block_n, g.num_stages,
-                op.gemm.grid, g.act, g.out_fp32, g.residual != nullptr, op.prof_n, op.prof_ms);
-      else
-        fprintf(f, "%d,%zu,%s,%lld,0,0,0,0,0,0,0,0,%d,%d,%d,%d,%d,%lld,%.6f\n", p.n, i, kinds[op.kind], static_cast<long long>(op.l0), op.i[0], op.i[1],
-                op.i[2], op.i[3], op.i[4], op.prof_n, op.prof_ms);
+      std::visit([&](const auto& r) {
+        if constexpr (std::is_same_v<std::decay_t<decltype(r)>, GemmOp>) {
+          const GemmParams& g = r.plan.p;
+          fprintf(f, "%d,%zu,%s,%d,%d,%d,%d,%d,%d,%d,%d,%d,0,0,0,0,0,%lld,%.6f\n", p.n, i, kinds[r.kind], g.M, g.N, g.K, g.block_n, g.num_stages,
+                  r.plan.grid, g.act, g.out_fp32, g.residual != nullptr, op.prof_n, op.prof_ms);
+        } else {
+          const ProfCols c = r.cols();
+          fprintf(f, "%d,%zu,%s,%lld,0,0,0,0,0,0,0,0,%d,%d,%d,%d,%d,%lld,%.6f\n", p.n, i, kinds[r.kind], c.M, c.i[0], c.i[1], c.i[2], c.i[3], c.i[4],
+                  op.prof_n, op.prof_ms);
+        }
+      }, op.rec);
     }
   }
   fclose(f);

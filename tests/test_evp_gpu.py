@@ -150,6 +150,40 @@ def test_other_variants_match_oracle(variant, hw, with_flow):
     _check(out, ref, f"{variant} {hw[0]}x{hw[1]} flow={with_flow} vs oracle")
 
 
+def test_simt_dwconv_and_im2col_from_input_match_oracle(tmp_path):
+    """Two launch forms no mit_bX_evp reaches: stage 1's MixFFN width 96 x 2 = 192 is not a multiple of 128, so its DWConv runs the
+    SIMT kernel instead of the TMA one, and stage 1's patch embed (Cout 96) cannot use the fused stem, so im2col reads the call's x.
+    The plan's profile shows both: im2col with Cin 3 for the handcrafted prompt and the patch embed, DWConv with C 192."""
+    import csv
+    from collections import OrderedDict
+    from functools import partial
+
+    from surgvid_b200 import _native
+    from surgvid_b200.models.mix_transformer_evp import MixVisionTransformerEVP
+    cfg = dict(embed_dims=[96, 192, 320, 512], num_heads=[3, 3, 5, 8], depths=[2, 2, 2, 2], sr_ratios=[8, 4, 2, 1])
+    m = MixVisionTransformerEVP(patch_size=4, mlp_ratios=[2] * 4, qkv_bias=True, norm_layer=partial(torch.nn.LayerNorm, eps=1e-6),
+                                drop_rate=0.0, drop_path_rate=0.1, **cfg)
+    sd = S.synth_state_dict(OrderedDict((k, tuple(v.shape)) for k, v in m.state_dict().items()), seed=2, mode="stress")
+    m.load_state_dict(sd, strict=True)
+    m = m.to(DEV).eval()
+    x, seg, flow = S.synth_frames(3, seed=77)
+    ref = EO.evp_forward(sd, cfg, x, seg, flow)
+    with torch.no_grad():
+        out = m(x.to(DEV), seg.to(DEV), flow.to(DEV), return_features=True)
+    _check(out, ref, "embed_dims 96/192/320/512, mlp_ratio 2 vs oracle")
+    lib, h = _native.lib(), m._native[0]["handle"]
+    _native.check(lib.sv_evp_set_profile(h, 1), "sv_evp_set_profile")
+    with torch.no_grad():
+        m(x.to(DEV), seg.to(DEV), flow.to(DEV), return_features=True)
+    torch.cuda.synchronize()
+    path = tmp_path / "ops.csv"
+    _native.check(lib.sv_evp_dump_profile(h, str(path).encode()), "sv_evp_dump_profile")
+    _native.check(lib.sv_evp_set_profile(h, 0), "sv_evp_set_profile")
+    rows = list(csv.DictReader(open(path)))
+    assert sum(r["kind"] == "im2col" and r["i1"] == "3" for r in rows) == 2, rows
+    assert any(r["kind"] == "dwconv" and r["i3"] == "192" for r in rows), rows
+
+
 def test_full_size_video_properties():
     """BASELINE configs[1] at full size (one 2 300-frame video, the bench's micro-batch of 800) through size-independent properties:
     (1) frames are independent, so the features of the whole video are bit-identical to those of any sub-range processed on its own
