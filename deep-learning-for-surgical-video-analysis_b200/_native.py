@@ -212,3 +212,14 @@ def last_error() -> str:
 def check(status: int, what: str = "libsurgvid"):
     if status != SV_OK:
         raise RuntimeError(f"{what} failed (status {status}): {last_error()}")
+
+
+def set_tensors(set_tensor, handle, named_tensors, what: str):
+    """Hand (name, tensor) pairs, e.g. `module.state_dict().items()`, to a handle's `sv_*_set_tensor` as contiguous fp32 host copies."""
+    import numpy as np
+    import torch
+
+    for name, t in named_tensors:
+        a = np.ascontiguousarray(t.detach().to("cpu", torch.float32).numpy())
+        shape = (c_int64 * max(a.ndim, 1))(*a.shape)
+        check(set_tensor(handle, name.encode(), a.ctypes.data_as(c_void_p), shape, a.ndim), what)

@@ -20,9 +20,9 @@
 // normalises and stages one half of the output columns.
 #include <stdlib.h>
 
-#include <mutex>
 #include <string>
 
+#include "host.cuh"
 #include "kernels.cuh"
 #include "ptx.cuh"
 
@@ -664,34 +664,13 @@ attention_tc_single_kernel(const __grid_constant__ CUtensorMap tmap_q, const __g
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  });
-  return fn;
-}
-
 // [frames, N, ld] bf16 (token-major, row stride ld) seen as a 3-D tensor {cols, N, frames}; box = 64 columns x rows x 1 frame, 128B swizzle
 int encode_tokens_map(CUtensorMap* map, const bf16* base, int cols, int N, int B, int64_t ld, int box_rows) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) return fail(SV_ERR_CUDA, "cuTensorMapEncodeTiled driver entry point unavailable (no CUDA driver?)");
   cuuint64_t gdim[3] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(N), static_cast<cuuint64_t>(B)};
   cuuint64_t gstr[2] = {static_cast<cuuint64_t>(ld) * 2, static_cast<cuuint64_t>(N) * static_cast<cuuint64_t>(ld) * 2};
   cuuint32_t box[3] = {static_cast<cuuint32_t>(kHD), static_cast<cuuint32_t>(box_rows), 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<bf16*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(SV_ERR_CUDA, "cuTensorMapEncodeTiled(attention) failed, CUresult " + std::to_string(static_cast<int>(r)));
-  return SV_OK;
+  return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                      "attention");
 }
 
 }  // namespace

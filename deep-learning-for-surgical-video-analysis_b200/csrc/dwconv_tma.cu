@@ -9,9 +9,9 @@
 // Many tiles are in flight per SM regardless of register pressure, which the register-only version could not do.
 #include <stdlib.h>
 
-#include <mutex>
 #include <type_traits>
 
+#include "host.cuh"
 #include "kernels.cuh"
 #include "ptx.cuh"
 
@@ -218,22 +218,6 @@ dwconv3x3_gelu_tma_kernel(const __grid_constant__ CUtensorMap tmap_x, const DwPa
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  });
-  return fn;
-}
-
 }  // namespace
 
 static int dw_cpl() {
@@ -246,16 +230,12 @@ int dwconv_tma_plan(const bf16* x, const float* w9c, const float* bias, int B, i
   SV_CHECK(ldo >= C && ldo % 4 == 0, "dwconv output row stride");
   SV_CHECK(dwconv_tma_supported(C), "dwconv TMA path needs C % 128 == 0");
   SV_CHECK((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 7) == 0, "dwconv alignment");
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) return fail(SV_ERR_CUDA, "cuTensorMapEncodeTiled driver entry point unavailable");
   cuuint64_t gdim[4] = {static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H), static_cast<cuuint64_t>(B)};
   cuuint64_t gstr[3] = {static_cast<cuuint64_t>(C) * 2, static_cast<cuuint64_t>(W) * C * 2, static_cast<cuuint64_t>(H) * W * C * 2};
   const int tw = (W % 8 == 0) ? 8 : ((W % 7 == 0) ? 7 : 8);
   cuuint32_t box[4] = {static_cast<cuuint32_t>(32 * dw_cpl()), static_cast<cuuint32_t>(tw + 2), kBoxH, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = fn(&plan->tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<bf16*>(x), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(SV_ERR_CUDA, "cuTensorMapEncodeTiled(dwconv) failed, CUresult " + std::to_string(static_cast<int>(r)));
+  SV_TRY(encode_tiled(&plan->tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, x, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_NONE,
+                      CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "dwconv"));
   plan->w9c = w9c; plan->bias = bias; plan->out = out; plan->B = B; plan->H = H; plan->W = W; plan->C = C; plan->ldo = ldo; plan->tw = tw;
   plan->cpl = dw_cpl();
   return SV_OK;

@@ -22,15 +22,11 @@
 #include <vector>
 
 #include "gemm.cuh"
+#include "host.cuh"
 #include "kernels.cuh"
 
 namespace sv {
 namespace {
-
-struct HostTensor {
-  std::vector<float> data;
-  std::vector<int64_t> shape;
-};
 
 struct Lin {        // packed nn.Linear / patchified conv: bf16 W[N, ldw] + fp32 bias[N]
   size_t w = 0;     // element offset into the bf16 blob
@@ -211,8 +207,7 @@ struct StageGeom {
 struct sv_evp {
   sv_evp_cfg cfg;
   int device = 0;
-  std::map<std::string, sv::HostTensor> tensors;
-  bool packed = false;
+  sv::StateDict sd;
   sv::bf16* d_wb = nullptr;
   float* d_wf = nullptr;
   sv::StageW st[4];
@@ -255,11 +250,10 @@ struct Packer {
   size_t alloc_b(size_t n) { size_t o = wb.size(); wb.resize(o + ((n + 7) / 8) * 8, 0); return o; }
   size_t alloc_f(size_t n) { size_t o = wf.size(); wf.resize(o + ((n + 3) / 4) * 4, 0.f); return o; }
 
-  const HostTensor* get(const std::string& key, std::vector<int64_t> shape) {
-    auto it = h->tensors.find(key);
-    if (it == h->tensors.end()) { if (err.empty()) err = "missing state_dict key '" + key + "'"; return nullptr; }
-    if (it->second.shape != shape) { if (err.empty()) err = "wrong shape for state_dict key '" + key + "'"; return nullptr; }
-    return &it->second;
+  const HostTensor* get(const std::string& key, const std::vector<int64_t>& shape) {
+    const HostTensor* t;
+    if (h->sd.get(key, shape, "evp pack_weights", &t) != SV_OK && err.empty()) err = sv_last_error();
+    return t;
   }
   size_t vec(const std::string& key, int64_t n) {
     const HostTensor* t = get(key, {n});
@@ -475,18 +469,13 @@ int pack_all(sv_evp* h) {
     h->fc_b[a][0] = P.vec(std::string(fcn[a]) + ".0.bias", 512);
     h->fc_b[a][1] = P.vec(std::string(fcn[a]) + ".2.bias", 7);
   }
-  if (!P.err.empty()) return fail(SV_ERR_STATE, "evp pack_weights: " + P.err);
+  if (!P.err.empty()) return fail(SV_ERR_STATE, P.err);
 
-  SV_CUDA_OK(cudaSetDevice(h->device));
-  if (h->d_wb) { cudaFree(h->d_wb); h->d_wb = nullptr; }
-  if (h->d_wf) { cudaFree(h->d_wf); h->d_wf = nullptr; }
-  SV_CUDA_OK(cudaMalloc(&h->d_wb, P.wb.size() * sizeof(uint16_t)));
-  SV_CUDA_OK(cudaMalloc(&h->d_wf, P.wf.size() * sizeof(float)));
-  SV_CUDA_OK(cudaMemcpy(h->d_wb, P.wb.data(), P.wb.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
-  SV_CUDA_OK(cudaMemcpy(h->d_wf, P.wf.data(), P.wf.size() * sizeof(float), cudaMemcpyHostToDevice));
+  SV_TRY(upload(h->device, &h->d_wb, P.wb));
+  SV_TRY(upload(h->device, &h->d_wf, P.wf));
   h->plans.clear();
   h->last_plan = nullptr;
-  h->packed = true;
+  h->sd.packed = true;
   return SV_OK;
 }
 
@@ -978,14 +967,7 @@ int sv_evp_set_tensor(sv_evp_handle* h, const char* name, const float* host_data
   using namespace sv;
   SV_CHECK(h && name, "null argument");
   SV_CHECK(ndim >= 0 && ndim <= 4, "evp: tensor rank");
-  HostTensor t;
-  int64_t n = 1;
-  for (int i = 0; i < ndim; ++i) { t.shape.push_back(shape[i]); n *= shape[i]; }
-  if (host_data) t.data.assign(host_data, host_data + n);
-  else t.data.assign(static_cast<size_t>(n), 0.f);
-  h->tensors[name] = std::move(t);
-  h->packed = false;
-  return SV_OK;
+  return h->sd.set(name, host_data, shape, ndim);
 }
 
 int sv_evp_pack_weights(sv_evp_handle* h) {
@@ -1013,7 +995,7 @@ int evp_forward(sv_evp_handle* h, const float* x, const float* seg, const float*
                 const std::vector<int32_t>& dims, int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace, size_t workspace_bytes,
                 void* stream) {
   SV_CHECK(h && x && seg && out_features && workspace, "null argument");
-  if (!h->packed) return fail(SV_ERR_STATE, "evp: pack_weights() has not been called");
+  if (!h->sd.packed) return fail(SV_ERR_STATE, "evp: pack_weights() has not been called");
   SV_CHECK(B > 0 && micro_batch > 0, "evp: B and micro_batch must be positive");
   SV_CHECK((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "evp: workspace must be 256-byte aligned");
   SV_CHECK(static_cast<int64_t>(micro_batch) * H * W < (1LL << 28), "evp: micro_batch * H * W too large");
@@ -1100,7 +1082,7 @@ int sv_evp_forward_attention(sv_evp_handle* h, const float* x, const float* seg,
 int sv_evp_classify(sv_evp_handle* h, const float* feats, float* y, float* y_ant, int32_t B, void* stream) {
   using namespace sv;
   SV_CHECK(h && feats && y && y_ant && B > 0, "bad argument");
-  if (!h->packed) return fail(SV_ERR_STATE, "evp: pack_weights() has not been called");
+  if (!h->sd.packed) return fail(SV_ERR_STATE, "evp: pack_weights() has not been called");
   SV_CHECK(h->cfg.embedding_dim == 2048, "evp: classifier heads expect 2048-d features");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* outs[2] = {y, y_ant};

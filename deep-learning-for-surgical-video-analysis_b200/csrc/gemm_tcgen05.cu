@@ -18,12 +18,12 @@
 #include <stdlib.h>
 
 #include <algorithm>
-#include <mutex>
 #include <string>
 #include <vector>
 
 #include "gemm.cuh"
 #include "gemm_epi.cuh"
+#include "host.cuh"
 #include "ptx.cuh"
 
 namespace sv {
@@ -586,67 +586,21 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  });
-  return fn;
-}
-
 // 2-D bf16 row-major [rows, cols] tensor, row stride ld elements; box = [box_rows, 64 cols], 128B swizzle, zero OOB fill.
 int encode_operand_map(CUtensorMap* map, const bf16* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
-  EncodeTiledFn fn = get_encode_fn();
-  if (fn == nullptr) return fail(SV_ERR_CUDA, "cuTensorMapEncodeTiled driver entry point unavailable (no CUDA driver?)");
   if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return fail(SV_ERR_INVALID, "GEMM operand base must be 16-byte aligned");
   if ((ld * 2) % 16 != 0) return fail(SV_ERR_INVALID, "GEMM operand row stride must be a multiple of 8 elements");
   cuuint64_t gdim[2] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(rows)};
   cuuint64_t gstride[1] = {static_cast<cuuint64_t>(ld) * 2};
   cuuint32_t box[2] = {static_cast<cuuint32_t>(kBlockK), static_cast<cuuint32_t>(box_rows)};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<bf16*>(base), gdim, gstride, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    char buf[256];
-    snprintf(buf, sizeof(buf), "cuTensorMapEncodeTiled failed (CUresult %d) rows=%lld cols=%lld ld=%lld box_rows=%d", static_cast<int>(r),
-             static_cast<long long>(rows), static_cast<long long>(cols), static_cast<long long>(ld), box_rows);
-    return fail(SV_ERR_CUDA, buf);
-  }
-  return SV_OK;
-}
-
-typedef CUresult (*EncodeIm2colFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const int*,
-                                  const int*, cuuint32_t, cuuint32_t, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeIm2colFn get_encode_im2col_fn() {
-  static EncodeIm2colFn fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeIm2colFn>(p);
-  });
-  return fn;
+  return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, gdim, gstride, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                      CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "gemm operand");
 }
 
 // im2col-mode map of an NHWC bf16 conv input: each load is one 128-pixel column of one tap, 64 channels (128 B) per pixel, 128B swizzle —
 // the tile a 2-D map with box [128 rows, 64 cols] writes.  The bounding box [-pad, W - 1 + pad - (k - 1)] (and the same along H), walked
 // with the conv stride, holds exactly the Ho x Wo window origins; zero OOB fill is the conv's padding and the rows past M.
 int encode_im2col_map(CUtensorMap* map, const bf16* base, const ConvGeom& g) {
-  EncodeIm2colFn fn = get_encode_im2col_fn();
-  if (fn == nullptr) return fail(SV_ERR_CUDA, "cuTensorMapEncodeIm2col driver entry point unavailable (no CUDA driver?)");
   if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) return fail(SV_ERR_INVALID, "conv GEMM input must be 16-byte aligned");
   const cuuint64_t es = 2;
   cuuint64_t gdim[4] = {static_cast<cuuint64_t>(g.C), static_cast<cuuint64_t>(g.W), static_cast<cuuint64_t>(g.H), static_cast<cuuint64_t>(g.B)};
@@ -654,15 +608,8 @@ int encode_im2col_map(CUtensorMap* map, const bf16* base, const ConvGeom& g) {
   const int lower[2] = {-g.pad, -g.pad};
   const int upper[2] = {g.pad - (g.k - 1), g.pad - (g.k - 1)};
   cuuint32_t estr[4] = {1, static_cast<cuuint32_t>(g.stride), static_cast<cuuint32_t>(g.stride), 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<bf16*>(base), gdim, gstride, lower, upper, kBlockK, kBlockM, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    char buf[256];
-    snprintf(buf, sizeof(buf), "cuTensorMapEncodeIm2col failed (CUresult %d) B=%d H=%d W=%d C=%d k=%d stride=%d pad=%d", static_cast<int>(r), g.B, g.H,
-             g.W, g.C, g.k, g.stride, g.pad);
-    return fail(SV_ERR_CUDA, buf);
-  }
-  return SV_OK;
+  return encode_im2col(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, gdim, gstride, lower, upper, kBlockK, kBlockM, estr, CU_TENSOR_MAP_SWIZZLE_128B,
+                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "conv gemm input");
 }
 
 // Host-side checks of a convolution's geometry; no device access.
@@ -815,21 +762,16 @@ int gemm_plan(const GemmDesc& d, GemmPlan* plan) {
   plan->tmap_res = plan->tmap_a;
   if (p.tma_out) {
     // bf16: box = 32 columns x 32 rows; fp32: box = 16 columns x 32 rows; 64 bytes per box row, 64-byte swizzle
-    EncodeTiledFn fn = get_encode_fn();
-    if (fn == nullptr) return fail(SV_ERR_CUDA, "cuTensorMapEncodeTiled driver entry point unavailable (no CUDA driver?)");
-    auto enc = [&](CUtensorMap* m, const void* base, int64_t ld) -> int {
+    auto enc = [&](CUtensorMap* m, const void* base, int64_t ld, const char* what) -> int {
       const int es = d.out_fp32 ? 4 : 2;
       cuuint64_t gdim[2] = {static_cast<cuuint64_t>(d.N), static_cast<cuuint64_t>(d.M)};
       cuuint64_t gstride[1] = {static_cast<cuuint64_t>(ld) * es};
       cuuint32_t box[2] = {static_cast<cuuint32_t>(64 / es), 32};
-      cuuint32_t estr[2] = {1, 1};
-      CUresult r = fn(m, d.out_fp32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gdim, gstride, box, estr,
-                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return fail(SV_ERR_CUDA, "cuTensorMapEncodeTiled(gemm out) failed, CUresult " + std::to_string(static_cast<int>(r)));
-      return SV_OK;
+      return encode_tiled(m, d.out_fp32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, gdim, gstride, box,
+                          CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, what);
     };
-    SV_TRY(enc(&plan->tmap_out, d.out, d.ldc));
-    if (d.residual) SV_TRY(enc(&plan->tmap_res, d.residual, d.ldr));
+    SV_TRY(enc(&plan->tmap_out, d.out, d.ldc, "gemm out"));
+    if (d.residual) SV_TRY(enc(&plan->tmap_res, d.residual, d.ldr, "gemm residual"));
   }
   return SV_OK;
 }
@@ -889,6 +831,19 @@ int gemm_launch(const GemmPlan& plan, cudaStream_t stream) {
   return launch_status("gemm_bf16_tcgen05_kernel");
 }
 
+namespace {
+
+// The end of every sv_op_*gemm* entry point.  SURGVID_GEMM_PAIR, read on every call so that a test can change it between calls,
+// forces CTA-pair mode on (1) or off (0).
+int plan_and_launch(GemmDesc& d, void* stream) {
+  if (const char* e = getenv("SURGVID_GEMM_PAIR")) d.pair = atoi(e);
+  GemmPlan plan;
+  SV_TRY(gemm_plan(d, &plan));
+  return gemm_launch(plan, static_cast<cudaStream_t>(stream));
+}
+
+}  // namespace
+
 }  // namespace sv
 
 #ifdef SV_GEMM_TRACE
@@ -903,10 +858,7 @@ extern "C" int sv_op_gemm_bf16(const uint16_t* A, int64_t lda, const uint16_t* W
   d.W = reinterpret_cast<const sv::bf16*>(W); d.ldw = ldw;
   d.M = M; d.N = N; d.K = K; d.bias = bias; d.act = act; d.residual = residual; d.ldr = ldr;
   d.out = out; d.ldc = ldc; d.out_fp32 = out_fp32;
-  if (const char* e = getenv("SURGVID_GEMM_PAIR")) d.pair = atoi(e);  // test hook: force CTA-pair mode on (1) / off (0)
-  sv::GemmPlan plan;
-  SV_TRY(sv::gemm_plan(d, &plan));
-  return sv::gemm_launch(plan, static_cast<cudaStream_t>(stream));
+  return sv::plan_and_launch(d, stream);
 }
 
 extern "C" int sv_op_gemm_plan_info(int32_t M, int32_t N, int32_t K, int32_t K2, int32_t out_fp32, int32_t has_residual, int32_t pair_request,
@@ -939,10 +891,7 @@ extern "C" int sv_op_conv_gemm_bf16(const uint16_t* x, int32_t B, int32_t H, int
   d.W = reinterpret_cast<const sv::bf16*>(Wt); d.ldw = ldw;
   d.M = B * d.conv.Ho() * d.conv.Wo(); d.N = N; d.K = k * k * C; d.bias = bias; d.act = act; d.residual = residual; d.ldr = ldr;
   d.out = out; d.ldc = ldc; d.out_fp32 = out_fp32;
-  if (const char* e = getenv("SURGVID_GEMM_PAIR")) d.pair = atoi(e);  // test hook, as in sv_op_gemm_bf16
-  sv::GemmPlan plan;
-  SV_TRY(sv::gemm_plan(d, &plan));
-  return sv::gemm_launch(plan, static_cast<cudaStream_t>(stream));
+  return sv::plan_and_launch(d, stream);
 }
 
 extern "C" int sv_op_conv_gemm_plan_info(int32_t B, int32_t H, int32_t W, int32_t C, int32_t k, int32_t stride, int32_t pad, int32_t N, int32_t out_fp32,
@@ -967,8 +916,5 @@ extern "C" int sv_op_gemm_bf16_cat(const uint16_t* A, int64_t lda, const uint16_
   d.W = reinterpret_cast<const sv::bf16*>(W); d.ldw = ldw;
   d.M = M; d.N = N; d.K = K; d.bias = bias; d.act = act; d.residual = residual; d.ldr = ldr;
   d.out = out; d.ldc = ldc; d.out_fp32 = out_fp32;
-  if (const char* e = getenv("SURGVID_GEMM_PAIR")) d.pair = atoi(e);  // test hook, as in sv_op_gemm_bf16
-  sv::GemmPlan plan;
-  SV_TRY(sv::gemm_plan(d, &plan));
-  return sv::gemm_launch(plan, static_cast<cudaStream_t>(stream));
+  return sv::plan_and_launch(d, stream);
 }

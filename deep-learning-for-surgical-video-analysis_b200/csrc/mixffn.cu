@@ -21,9 +21,9 @@
 #include <stdlib.h>
 
 #include <algorithm>
-#include <mutex>
 
 #include "gemm_epi.cuh"
+#include "host.cuh"
 #include "kernels.cuh"
 #include "ptx.cuh"
 
@@ -357,33 +357,6 @@ mixffn_fc2_kernel(const __grid_constant__ CUtensorMap tmap_h1, const __grid_cons
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  });
-  return fn;
-}
-
-int encode(CUtensorMap* map, CUtensorMapDataType dt, int rank, const void* base, const cuuint64_t* gdim, const cuuint64_t* gstr,
-           const cuuint32_t* box, CUtensorMapSwizzle sw, const char* what) {
-  EncodeTiledFn fn = encode_fn();
-  if (fn == nullptr) return fail(SV_ERR_CUDA, "cuTensorMapEncodeTiled driver entry point unavailable (no CUDA driver?)");
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = fn(map, dt, static_cast<cuuint32_t>(rank), const_cast<void*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(SV_ERR_CUDA, std::string("cuTensorMapEncodeTiled(mixffn ") + what + ") failed, CUresult " + std::to_string(static_cast<int>(r)));
-  return SV_OK;
-}
-
 // rows of a tile: the largest R with R*W <= 128, then evened out over the frame height
 int pick_rows(int H, int W) {
   const int rmax = std::min(H, kBlockM / W);
@@ -454,26 +427,30 @@ int mixffn_fc2_plan(const bf16* h1, const float* w10c, const bf16* Wcat, int64_t
     cuuint64_t gdim[4] = {static_cast<cuuint64_t>(hidden), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H), static_cast<cuuint64_t>(frames)};
     cuuint64_t gstr[3] = {static_cast<cuuint64_t>(hidden) * 2, static_cast<cuuint64_t>(W) * hidden * 2, static_cast<cuuint64_t>(H) * W * hidden * 2};
     cuuint32_t box[4] = {kBlockK, static_cast<cuuint32_t>(W + 2), static_cast<cuuint32_t>(p.R + 2), 1};
-    SV_TRY(encode(&plan->tmap_h1, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, h1, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_NONE, "h1"));
+    SV_TRY(encode_tiled(&plan->tmap_h1, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, h1, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_NONE,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "mixffn h1"));
   }
   {  // depthwise taps + bias as fp32 [10, hidden]
     cuuint64_t gdim[2] = {static_cast<cuuint64_t>(hidden), 10};
     cuuint64_t gstr[1] = {static_cast<cuuint64_t>(hidden) * 4};
     cuuint32_t box[2] = {kBlockK, 10};
-    SV_TRY(encode(&plan->tmap_dw, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, w10c, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_NONE, "dw"));
+    SV_TRY(encode_tiled(&plan->tmap_dw, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, w10c, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_NONE,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "mixffn dw"));
   }
   {  // [N, hidden + tail] bf16 weight, K-major, 128B swizzle
     cuuint64_t gdim[2] = {static_cast<cuuint64_t>(hidden + tail_cols), static_cast<cuuint64_t>(N)};
     cuuint64_t gstr[1] = {static_cast<cuuint64_t>(ldw) * 2};
     cuuint32_t box[2] = {kBlockK, static_cast<cuuint32_t>(p.bn)};
-    SV_TRY(encode(&plan->tmap_w, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, Wcat, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B, "w"));
+    SV_TRY(encode_tiled(&plan->tmap_w, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, Wcat, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "mixffn w"));
   }
   if (tail_cols > 0) {
     SV_CHECK((reinterpret_cast<uintptr_t>(tail) & 15) == 0 && ldt % 8 == 0 && ldt >= tail_cols, "mixffn: tail operand alignment");
     cuuint64_t gdim[2] = {static_cast<cuuint64_t>(tail_cols), static_cast<cuuint64_t>(p.M)};
     cuuint64_t gstr[1] = {static_cast<cuuint64_t>(ldt) * 2};
     cuuint32_t box[2] = {kBlockK, kBlockM};
-    SV_TRY(encode(&plan->tmap_t, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, tail, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B, "tail"));
+    SV_TRY(encode_tiled(&plan->tmap_t, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, tail, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "mixffn tail"));
   } else {
     plan->tmap_t = plan->tmap_w;  // never dereferenced
   }

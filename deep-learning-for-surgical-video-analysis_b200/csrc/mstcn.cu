@@ -14,6 +14,7 @@
 #include <string>
 #include <vector>
 
+#include "host.cuh"
 #include "kernels.cuh"
 
 namespace sv {
@@ -523,42 +524,26 @@ __global__ void mstcn_stream_commit_kernel(const float* __restrict__ act, int64_
   }
 }
 
-struct HostTensor {
-  std::vector<float> data;
-  std::vector<int64_t> shape;
-};
-
 }  // namespace
 }  // namespace sv
 
 struct sv_mstcn {
   sv_mstcn_cfg cfg;
   int device = 0;
-  std::map<std::string, sv::HostTensor> tensors;
-  bool packed = false;
+  sv::StateDict sd;
   float* d_weights = nullptr;  // single device blob
   // offsets (in floats) into the blob
   struct Stage { size_t w_in, b_in, w_out, b_out, w_next, b_next, w_in_hi = 0, w_in_lo = 0; std::vector<size_t> layer, layer_tc; };
   std::vector<Stage> stages;
   int q_out = 0;  // rows of the optional query head `fc.weight` packed next to the stage-1 projection (0 = absent)
   int64_t launches = 0;
-  // host copy of the frame counters of every stream state reset through this handle, keyed by the state's address: the handle is the
-  // only writer of those counters, and the copy lets a step be refused before launch (unknown state, position past 2^31)
-  std::map<const void*, std::vector<int64_t>> stream_seen;
+  sv::StreamRegistry streams{"mstcn stream"};
 };
 
 namespace sv {
 namespace {
 
 std::string stage_prefix(int s) { return s == 0 ? std::string("stage1_phase") : "stages." + std::to_string(s - 1); }
-
-int expect(const sv_mstcn* h, const std::string& key, std::initializer_list<int64_t> shape, const HostTensor** out) {
-  auto it = h->tensors.find(key);
-  if (it == h->tensors.end()) return fail(SV_ERR_STATE, "mstcn: missing state_dict key '" + key + "'");
-  if (it->second.shape != std::vector<int64_t>(shape)) return fail(SV_ERR_INVALID, "mstcn: wrong shape for '" + key + "'");
-  *out = &it->second;
-  return SV_OK;
-}
 
 constexpr int kQCols = 16;  // query-head columns appended to the stage-1 projection (out_features <= 16)
 
@@ -582,9 +567,8 @@ struct StreamStep {
   int64_t stream_stride;
 };
 
-// Stream-state layout (documented in surgvid.h): int64 seen[n_streams], padded to 256 B, then per stream, per stage, per layer l a ring
-// of 2 * 2^l rows x f_maps floats (ring of layer l starts 2 * (2^l - 1) rows into the stage's 2 * (2^layers - 1) rows).
-size_t stream_seen_bytes(int32_t n_streams) { return (static_cast<size_t>(n_streams) * sizeof(int64_t) + 255) & ~static_cast<size_t>(255); }
+// Stream-state layout (documented in surgvid.h): the counters of StreamRegistry, then per stream, per stage, per layer l a ring of
+// 2 * 2^l rows x f_maps floats (ring of layer l starts 2 * (2^l - 1) rows into the stage's 2 * (2^layers - 1) rows).
 int64_t stream_ring_rows(const sv_mstcn_cfg& c) { return 2 * ((int64_t{1} << c.layers) - 1); }   // per stage
 int64_t stream_stride_floats(const sv_mstcn_cfg& c) { return c.stages * stream_ring_rows(c) * c.f_maps; }
 
@@ -704,14 +688,8 @@ int sv_mstcn_destroy(sv_mstcn_handle* h) {
 
 int sv_mstcn_set_tensor(sv_mstcn_handle* h, const char* name, const float* host_data, const int64_t* shape, int32_t ndim) {
   using namespace sv;
-  SV_CHECK(h && name && host_data && (shape || ndim == 0), "null argument");
-  HostTensor t;
-  int64_t n = 1;
-  for (int i = 0; i < ndim; ++i) { t.shape.push_back(shape[i]); n *= shape[i]; }
-  t.data.assign(host_data, host_data + n);
-  h->tensors[name] = std::move(t);
-  h->packed = false;
-  return SV_OK;
+  SV_CHECK(h && name && host_data, "null argument");
+  return h->sd.set(name, host_data, shape, ndim);
 }
 
 int sv_mstcn_pack_weights(sv_mstcn_handle* h) {
@@ -727,8 +705,8 @@ int sv_mstcn_pack_weights(sv_mstcn_handle* h) {
     const int64_t dim = s == 0 ? c.f_dim : C;
     sv_mstcn::Stage& S = h->stages[s];
     const HostTensor *w, *b;
-    SV_TRY(expect(h, p + ".conv_1x1.weight", {F, dim, 1}, &w));
-    SV_TRY(expect(h, p + ".conv_1x1.bias", {F}, &b));
+    SV_TRY(h->sd.get(p + ".conv_1x1.weight", {F, dim, 1}, "mstcn", &w));
+    SV_TRY(h->sd.get(p + ".conv_1x1.bias", {F}, "mstcn", &b));
     // k-major [dim][F] so that a K-chunk of W is contiguous over f
     S.w_in = reserve(dim * F);
     for (int64_t f = 0; f < F; ++f)
@@ -747,8 +725,8 @@ int sv_mstcn_pack_weights(sv_mstcn_handle* h) {
       // optional query head of the Trans-SVNet wrapper: `fc.weight` [out_q, f_dim], no bias (adapter_transformer.py:325)
       h->q_out = 0;
       const HostTensor* fc = nullptr;
-      auto fit = h->tensors.find("fc.weight");
-      if (fit != h->tensors.end()) {
+      auto fit = h->sd.tensors.find("fc.weight");
+      if (fit != h->sd.tensors.end()) {
         fc = &fit->second;
         if (fc->shape.size() != 2 || fc->shape[1] != dim || fc->shape[0] < 1 || fc->shape[0] > kQCols)
           return fail(SV_ERR_INVALID, "mstcn: 'fc.weight' must be [out_features <= 16, f_dim]");
@@ -771,10 +749,10 @@ int sv_mstcn_pack_weights(sv_mstcn_handle* h) {
     for (int l = 0; l < c.layers; ++l) {
       const std::string lp = p + ".layers." + std::to_string(l);
       const HostTensor *wd, *bd, *w1, *b1;
-      SV_TRY(expect(h, lp + ".conv_dilated.weight", {F, F, 3}, &wd));
-      SV_TRY(expect(h, lp + ".conv_dilated.bias", {F}, &bd));
-      SV_TRY(expect(h, lp + ".conv_1x1.weight", {F, F, 1}, &w1));
-      SV_TRY(expect(h, lp + ".conv_1x1.bias", {F}, &b1));
+      SV_TRY(h->sd.get(lp + ".conv_dilated.weight", {F, F, 3}, "mstcn", &wd));
+      SV_TRY(h->sd.get(lp + ".conv_dilated.bias", {F}, "mstcn", &bd));
+      SV_TRY(h->sd.get(lp + ".conv_1x1.weight", {F, F, 1}, "mstcn", &w1));
+      SV_TRY(h->sd.get(lp + ".conv_1x1.bias", {F}, "mstcn", &b1));
       const size_t off = reserve(3 * F * F + F * F + 2 * F);
       S.layer.push_back(off);
       // Wd[tap][cin][cout] ; conv1d weight is [cout][cin][tap], tap k multiplies x[t-(2-k)d]
@@ -815,8 +793,8 @@ int sv_mstcn_pack_weights(sv_mstcn_handle* h) {
         std::copy(b1->data.begin(), b1->data.end(), blob.begin() + ob1);
       }
     }
-    SV_TRY(expect(h, p + ".conv_out_classes.weight", {C, F, 1}, &w));
-    SV_TRY(expect(h, p + ".conv_out_classes.bias", {C}, &b));
+    SV_TRY(h->sd.get(p + ".conv_out_classes.weight", {C, F, 1}, "mstcn", &w));
+    SV_TRY(h->sd.get(p + ".conv_out_classes.bias", {C}, "mstcn", &b));
     S.w_out = reserve(C * F);
     std::copy(w->data.begin(), w->data.end(), blob.begin() + S.w_out);  // [C][F]
     S.b_out = reserve(C);
@@ -827,11 +805,8 @@ int sv_mstcn_pack_weights(sv_mstcn_handle* h) {
     h->stages[s].w_next = h->stages[s + 1].w_in;
     h->stages[s].b_next = h->stages[s + 1].b_in;
   }
-  if (h->d_weights) { cudaFree(h->d_weights); h->d_weights = nullptr; }
-  SV_CUDA_OK(cudaSetDevice(h->device));
-  SV_CUDA_OK(cudaMalloc(&h->d_weights, blob.size() * sizeof(float)));
-  SV_CUDA_OK(cudaMemcpy(h->d_weights, blob.data(), blob.size() * sizeof(float), cudaMemcpyHostToDevice));
-  h->packed = true;
+  SV_TRY(upload(h->device, &h->d_weights, blob));
+  h->sd.packed = true;
   return SV_OK;
 }
 
@@ -850,7 +825,7 @@ int sv_mstcn_forward_query(sv_mstcn_handle* h, const float* feats, const int64_t
                            void* workspace, size_t workspace_bytes, void* stream) {
   using namespace sv;
   SV_CHECK(h && feats && video_offsets && logits && workspace, "null argument");
-  if (!h->packed) return fail(SV_ERR_STATE, "mstcn: pack_weights() has not been called");
+  if (!h->sd.packed) return fail(SV_ERR_STATE, "mstcn: pack_weights() has not been called");
   if (query != nullptr && h->q_out == 0) return fail(SV_ERR_STATE, "mstcn: a query output was requested but no 'fc.weight' tensor was set");
   SV_CHECK(n_videos >= 1 && n_videos < 4096, "mstcn: 1 <= n_videos < 4096");
   SV_CHECK(video_offsets[0] == 0, "mstcn: video_offsets[0] must be 0");
@@ -871,7 +846,7 @@ int sv_mstcn_forward_query(sv_mstcn_handle* h, const float* feats, const int64_t
 
 size_t sv_mstcn_stream_state_bytes(const sv_mstcn_handle* h, int32_t n_streams) {
   if (!h || n_streams < 1) return 0;
-  return sv::stream_seen_bytes(n_streams) + static_cast<size_t>(n_streams) * sv::stream_stride_floats(h->cfg) * sizeof(float);
+  return sv::StreamRegistry::counter_bytes(n_streams) + static_cast<size_t>(n_streams) * sv::stream_stride_floats(h->cfg) * sizeof(float);
 }
 
 size_t sv_mstcn_stream_workspace_bytes(const sv_mstcn_handle* h, int64_t rows) {
@@ -885,59 +860,18 @@ int sv_mstcn_stream_reset(sv_mstcn_handle* h, void* state, size_t state_bytes, i
                           void* stream) {
   using namespace sv;
   SV_CHECK(h && state, "null argument");
-  SV_CHECK(n_streams >= 1, "mstcn stream: n_streams >= 1");
-  SV_CHECK(state_bytes >= sv_mstcn_stream_state_bytes(h, n_streams), "mstcn stream: state too small");
-  SV_CHECK((reinterpret_cast<uintptr_t>(state) & 255) == 0, "mstcn stream: state must be 256-byte aligned");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int64_t* seen = static_cast<int64_t*>(state);
-  if (stream_ids == nullptr) {   // every stream: the whole state, so that no stale ring row is left behind
-    SV_CUDA_OK(cudaMemsetAsync(state, 0, sv_mstcn_stream_state_bytes(h, n_streams), st));
-    h->stream_seen[state].assign(n_streams, 0);
-    return SV_OK;
-  }
-  auto it = h->stream_seen.find(state);
-  if (it == h->stream_seen.end()) return fail(SV_ERR_STATE, "mstcn stream: reset every stream of a new state (stream_ids = NULL) first");
-  SV_CHECK(static_cast<int32_t>(it->second.size()) == n_streams, "mstcn stream: n_streams differs from the state's last full reset");
-  SV_CHECK(n_ids >= 1, "mstcn stream: n_ids >= 1");
-  std::vector<char> hit(n_streams, 0);
-  for (int i = 0; i < n_ids; ++i) {
-    SV_CHECK(stream_ids[i] >= 0 && stream_ids[i] < n_streams, "mstcn stream: stream id out of range");
-    SV_CHECK(!hit[stream_ids[i]], "mstcn stream: duplicate stream id");
-    hit[stream_ids[i]] = 1;
-  }
-  // only the counter: ring rows are read at positions [0, seen) alone, and those are rewritten before they are read again
-  for (int i = 0; i < n_ids; ++i) {
-    SV_CUDA_OK(cudaMemsetAsync(seen + stream_ids[i], 0, sizeof(int64_t), st));
-    it->second[stream_ids[i]] = 0;
-  }
-  return SV_OK;
+  return h->streams.reset(state, state_bytes, sv_mstcn_stream_state_bytes(h, n_streams), n_streams, stream_ids, n_ids,
+                          static_cast<cudaStream_t>(stream));
 }
 
 int sv_mstcn_stream_step(sv_mstcn_handle* h, void* state, size_t state_bytes, int32_t n_streams, const float* feats, const int32_t* stream_ids,
                          const int64_t* counts, int32_t n_ids, float* logits, float* query, void* workspace, size_t workspace_bytes, void* stream) {
   using namespace sv;
   SV_CHECK(h && state && feats && stream_ids && counts && logits && workspace, "null argument");
-  if (!h->packed) return fail(SV_ERR_STATE, "mstcn: pack_weights() has not been called");
+  if (!h->sd.packed) return fail(SV_ERR_STATE, "mstcn: pack_weights() has not been called");
   if (query != nullptr && h->q_out == 0) return fail(SV_ERR_STATE, "mstcn: a query output was requested but no 'fc.weight' tensor was set");
-  SV_CHECK(n_streams >= 1, "mstcn stream: n_streams >= 1");
-  SV_CHECK(state_bytes >= sv_mstcn_stream_state_bytes(h, n_streams), "mstcn stream: state too small");
-  auto it = h->stream_seen.find(state);
-  if (it == h->stream_seen.end()) return fail(SV_ERR_STATE, "mstcn stream: the state was not reset through this handle (reset every stream first)");
-  SV_CHECK(static_cast<int32_t>(it->second.size()) == n_streams, "mstcn stream: n_streams differs from the state's last full reset");
-  SV_CHECK(n_ids >= 1 && n_ids <= n_streams, "mstcn stream: 1 <= n_ids <= n_streams");
-  std::vector<int64_t> tab(2 * static_cast<size_t>(n_ids) + 1);   // chunk row offsets [n_ids + 1], then stream ids [n_ids]
-  std::vector<char> hit(n_streams, 0);
-  for (int i = 0; i < n_ids; ++i) {
-    const int32_t s = stream_ids[i];
-    SV_CHECK(s >= 0 && s < n_streams, "mstcn stream: stream id out of range");
-    SV_CHECK(!hit[s], "mstcn stream: duplicate stream id");
-    hit[s] = 1;
-    SV_CHECK(counts[i] >= 1, "mstcn stream: counts must be >= 1");
-    SV_CHECK(counts[i] < (1LL << 31) - it->second[s], "mstcn stream: a stream position would pass 2^31");
-    tab[i + 1] = tab[i] + counts[i];
-    SV_CHECK(tab[i + 1] < (1LL << 31), "mstcn stream: too many rows in one step");
-    tab[n_ids + 1 + i] = s;
-  }
+  std::vector<int64_t> tab;
+  SV_TRY(h->streams.check_step(state, state_bytes, sv_mstcn_stream_state_bytes(h, n_streams), n_streams, stream_ids, counts, n_ids, &tab));
   const int64_t T = tab[n_ids];
   SV_CHECK(workspace_bytes >= sv_mstcn_stream_workspace_bytes(h, T), "mstcn stream: workspace too small");
   SV_CHECK((reinterpret_cast<uintptr_t>(feats) & 15) == 0 && (reinterpret_cast<uintptr_t>(workspace) & 255) == 0 &&
@@ -952,12 +886,12 @@ int sv_mstcn_stream_step(sv_mstcn_handle* h, void* state, size_t state_bytes, in
   ss.tab = d_tab;
   ss.n_ids = n_ids;
   ss.seen = static_cast<int64_t*>(state);
-  ss.rings = reinterpret_cast<float*>(static_cast<char*>(state) + stream_seen_bytes(n_streams));
+  ss.rings = reinterpret_cast<float*>(static_cast<char*>(state) + StreamRegistry::counter_bytes(n_streams));
   ss.stream_stride = stream_stride_floats(h->cfg);
   const int rc = h->cfg.f_maps == 32 ? run_forward<32>(h, feats, nullptr, 0, T, logits, query, workspace, st, &ss)
                                      : run_forward<64>(h, feats, nullptr, 0, T, logits, query, workspace, st, &ss);
   if (rc != SV_OK) return rc;
-  for (int i = 0; i < n_ids; ++i) it->second[stream_ids[i]] += counts[i];
+  h->streams.advance(state, stream_ids, counts, n_ids);
   return SV_OK;
 }
 

@@ -20,6 +20,7 @@
 #include <string>
 #include <vector>
 
+#include "host.cuh"
 #include "kernels.cuh"
 
 namespace sv {
@@ -395,24 +396,17 @@ __global__ void trans_stream_commit_kernel(const float* __restrict__ logits, int
   if (threadIdx.x == 0) seen[s] = seen0 + cnt;
 }
 
-struct HostTensor {
-  std::vector<float> data;
-  std::vector<int64_t> shape;
-};
-
 }  // namespace
 }  // namespace sv
 
 struct sv_trans {
   sv_trans_cfg cfg;
   int device = 0;
-  std::map<std::string, sv::HostTensor> tensors;
-  bool packed = false;
+  sv::StateDict sd;
   float* d_blob = nullptr;
   int64_t* d_offsets = nullptr;
   int offsets_cap = 0;
-  // host copy of the frame counters of every stream state reset through this handle (see sv_mstcn)
-  std::map<const void*, std::vector<int64_t>> stream_seen;
+  sv::StreamRegistry streams{"trans stream"};
 };
 
 namespace sv {
@@ -420,23 +414,22 @@ namespace {
 
 // nn.Linear weight [rows, cols] (+ optional bias [rows]) -> blob[w_off + r * ld + c], blob[b_off + r]
 int put_linear(const sv_trans* h, const std::string& p, int rows, int cols, int ld, std::vector<float>* blob, int w_off, int b_off) {
-  auto it = h->tensors.find(p + ".weight");
-  if (it == h->tensors.end()) return fail(SV_ERR_STATE, "trans: missing state_dict key '" + p + ".weight'");
-  if (it->second.shape != std::vector<int64_t>{rows, cols}) return fail(SV_ERR_INVALID, "trans: wrong shape for '" + p + ".weight'");
+  const HostTensor* w;
+  SV_TRY(h->sd.get(p + ".weight", {rows, cols}, "trans", &w));
   for (int r = 0; r < rows; ++r)
-    for (int c = 0; c < cols; ++c) (*blob)[w_off + r * ld + c] = it->second.data[static_cast<size_t>(r) * cols + c];
-  auto ib = h->tensors.find(p + ".bias");
-  if (ib != h->tensors.end()) {   // bias-free variants of the upstream code: treated as zero
-    if (ib->second.shape != std::vector<int64_t>{rows}) return fail(SV_ERR_INVALID, "trans: wrong shape for '" + p + ".bias'");
-    for (int r = 0; r < rows; ++r) (*blob)[b_off + r] = ib->second.data[r];
+    for (int c = 0; c < cols; ++c) (*blob)[w_off + r * ld + c] = w->data[static_cast<size_t>(r) * cols + c];
+  if (h->sd.tensors.count(p + ".bias")) {   // bias-free variants of the upstream code: treated as zero
+    const HostTensor* b;
+    SV_TRY(h->sd.get(p + ".bias", {rows}, "trans", &b));
+    for (int r = 0; r < rows; ++r) (*blob)[b_off + r] = b->data[r];
   }
   return SV_OK;
 }
 int put_norm(const sv_trans* h, const std::string& p, int D, std::vector<float>* blob, int g_off, int b_off) {
-  auto ig = h->tensors.find(p + ".weight"), ib = h->tensors.find(p + ".bias");
-  if (ig == h->tensors.end() || ib == h->tensors.end()) return fail(SV_ERR_STATE, "trans: missing LayerNorm '" + p + "'");
-  if (ig->second.shape != std::vector<int64_t>{D} || ib->second.shape != std::vector<int64_t>{D}) return fail(SV_ERR_INVALID, "trans: wrong shape for '" + p + "'");
-  for (int c = 0; c < D; ++c) { (*blob)[g_off + c] = ig->second.data[c]; (*blob)[b_off + c] = ib->second.data[c]; }
+  const HostTensor *g, *b;
+  SV_TRY(h->sd.get(p + ".weight", {D}, "trans", &g));
+  SV_TRY(h->sd.get(p + ".bias", {D}, "trans", &b));
+  for (int c = 0; c < D; ++c) { (*blob)[g_off + c] = g->data[c]; (*blob)[b_off + c] = b->data[c]; }
   return SV_OK;
 }
 
@@ -513,14 +506,8 @@ int sv_trans_destroy(sv_trans_handle* h) {
 
 int sv_trans_set_tensor(sv_trans_handle* h, const char* name, const float* host_data, const int64_t* shape, int32_t ndim) {
   using namespace sv;
-  SV_CHECK(h && name && host_data && (shape || ndim == 0), "null argument");
-  HostTensor t;
-  int64_t n = 1;
-  for (int i = 0; i < ndim; ++i) { t.shape.push_back(shape[i]); n *= shape[i]; }
-  t.data.assign(host_data, host_data + n);
-  h->tensors[name] = std::move(t);
-  h->packed = false;
-  return SV_OK;
+  SV_CHECK(h && name && host_data, "null argument");
+  return h->sd.set(name, host_data, shape, ndim);
 }
 
 int sv_trans_pack_weights(sv_trans_handle* h) {
@@ -528,10 +515,8 @@ int sv_trans_pack_weights(sv_trans_handle* h) {
   SV_CHECK(h, "null handle");
   std::vector<float> blob;
   SV_TRY(h->cfg.d_k == 64 ? pack_blob<64>(h, &blob) : pack_blob<32>(h, &blob));
-  SV_CUDA_OK(cudaSetDevice(h->device));
-  if (!h->d_blob) SV_CUDA_OK(cudaMalloc(&h->d_blob, blob.size() * sizeof(float)));
-  SV_CUDA_OK(cudaMemcpy(h->d_blob, blob.data(), blob.size() * sizeof(float), cudaMemcpyHostToDevice));
-  h->packed = true;
+  SV_TRY(upload(h->device, &h->d_blob, blob));
+  h->sd.packed = true;
   return SV_OK;
 }
 
@@ -539,7 +524,7 @@ int sv_trans_forward(sv_trans_handle* h, const float* logits, int64_t ldx, const
                      float* out, void* stream) {
   using namespace sv;
   SV_CHECK(h && logits && query && video_offsets && out, "null argument");
-  if (!h->packed) return fail(SV_ERR_STATE, "trans: pack_weights() has not been called");
+  if (!h->sd.packed) return fail(SV_ERR_STATE, "trans: pack_weights() has not been called");
   SV_CHECK(n_videos >= 1 && video_offsets[0] == 0, "trans: offsets");
   for (int i = 0; i < n_videos; ++i) SV_CHECK(video_offsets[i + 1] > video_offsets[i], "trans: empty video / non-increasing offsets");
   const int64_t T = video_offsets[n_videos];
@@ -559,65 +544,26 @@ int sv_trans_forward(sv_trans_handle* h, const float* logits, int64_t ldx, const
 
 size_t sv_trans_stream_state_bytes(const sv_trans_handle* h, int32_t n_streams) {
   if (!h || n_streams < 1) return 0;
-  const size_t seen = (static_cast<size_t>(n_streams) * sizeof(int64_t) + 255) & ~static_cast<size_t>(255);
-  return seen + static_cast<size_t>(n_streams) * (h->cfg.len_q - 1) * h->cfg.d_model * sizeof(float);
+  return sv::StreamRegistry::counter_bytes(n_streams) + static_cast<size_t>(n_streams) * (h->cfg.len_q - 1) * h->cfg.d_model * sizeof(float);
 }
 
 int sv_trans_stream_reset(sv_trans_handle* h, void* state, size_t state_bytes, int32_t n_streams, const int32_t* stream_ids, int32_t n_ids,
                           void* stream) {
   using namespace sv;
   SV_CHECK(h && state, "null argument");
-  SV_CHECK(n_streams >= 1, "trans stream: n_streams >= 1");
-  SV_CHECK(state_bytes >= sv_trans_stream_state_bytes(h, n_streams), "trans stream: state too small");
-  SV_CHECK((reinterpret_cast<uintptr_t>(state) & 255) == 0, "trans stream: state must be 256-byte aligned");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (stream_ids == nullptr) {
-    SV_CUDA_OK(cudaMemsetAsync(state, 0, sv_trans_stream_state_bytes(h, n_streams), st));
-    h->stream_seen[state].assign(n_streams, 0);
-    return SV_OK;
-  }
-  auto it = h->stream_seen.find(state);
-  if (it == h->stream_seen.end()) return fail(SV_ERR_STATE, "trans stream: reset every stream of a new state (stream_ids = NULL) first");
-  SV_CHECK(static_cast<int32_t>(it->second.size()) == n_streams, "trans stream: n_streams differs from the state's last full reset");
-  SV_CHECK(n_ids >= 1, "trans stream: n_ids >= 1");
-  std::vector<char> hit(n_streams, 0);
-  for (int i = 0; i < n_ids; ++i) {
-    SV_CHECK(stream_ids[i] >= 0 && stream_ids[i] < n_streams, "trans stream: stream id out of range");
-    SV_CHECK(!hit[stream_ids[i]], "trans stream: duplicate stream id");
-    hit[stream_ids[i]] = 1;
-  }
-  for (int i = 0; i < n_ids; ++i) {   // ring rows are read at positions [0, seen) alone
-    SV_CUDA_OK(cudaMemsetAsync(static_cast<int64_t*>(state) + stream_ids[i], 0, sizeof(int64_t), st));
-    it->second[stream_ids[i]] = 0;
-  }
-  return SV_OK;
+  return h->streams.reset(state, state_bytes, sv_trans_stream_state_bytes(h, n_streams), n_streams, stream_ids, n_ids,
+                          static_cast<cudaStream_t>(stream));
 }
 
 int sv_trans_stream_forward(sv_trans_handle* h, void* state, size_t state_bytes, int32_t n_streams, const float* logits, int64_t ldx,
                             const float* query, const int32_t* stream_ids, const int64_t* counts, int32_t n_ids, float* out, void* stream) {
   using namespace sv;
   SV_CHECK(h && state && logits && query && stream_ids && counts && out, "null argument");
-  if (!h->packed) return fail(SV_ERR_STATE, "trans: pack_weights() has not been called");
-  SV_CHECK(n_streams >= 1, "trans stream: n_streams >= 1");
-  SV_CHECK(state_bytes >= sv_trans_stream_state_bytes(h, n_streams), "trans stream: state too small");
+  if (!h->sd.packed) return fail(SV_ERR_STATE, "trans: pack_weights() has not been called");
+  // a misaligned state cannot have been reset: say what is wrong with it before looking it up
   SV_CHECK((reinterpret_cast<uintptr_t>(state) & 255) == 0, "trans stream: state must be 256-byte aligned");
-  auto it = h->stream_seen.find(state);
-  if (it == h->stream_seen.end()) return fail(SV_ERR_STATE, "trans stream: the state was not reset through this handle (reset every stream first)");
-  SV_CHECK(static_cast<int32_t>(it->second.size()) == n_streams, "trans stream: n_streams differs from the state's last full reset");
-  SV_CHECK(n_ids >= 1 && n_ids <= n_streams, "trans stream: 1 <= n_ids <= n_streams");
-  std::vector<int64_t> tab(2 * static_cast<size_t>(n_ids) + 1);   // chunk row offsets [n_ids + 1], then stream ids [n_ids]
-  std::vector<char> hit(n_streams, 0);
-  for (int i = 0; i < n_ids; ++i) {
-    const int32_t s = stream_ids[i];
-    SV_CHECK(s >= 0 && s < n_streams, "trans stream: stream id out of range");
-    SV_CHECK(!hit[s], "trans stream: duplicate stream id");
-    hit[s] = 1;
-    SV_CHECK(counts[i] >= 1, "trans stream: counts must be >= 1");
-    SV_CHECK(counts[i] < (1LL << 31) - it->second[s], "trans stream: a stream position would pass 2^31");
-    tab[i + 1] = tab[i] + counts[i];
-    SV_CHECK(tab[i + 1] < (1LL << 31), "trans stream: too many rows in one step");
-    tab[n_ids + 1 + i] = s;
-  }
+  std::vector<int64_t> tab;
+  SV_TRY(h->streams.check_step(state, state_bytes, sv_trans_stream_state_bytes(h, n_streams), n_streams, stream_ids, counts, n_ids, &tab));
   const int64_t T = tab[n_ids];
   SV_CHECK(ldx >= T, "trans: logits row stride");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -631,12 +577,12 @@ int sv_trans_stream_forward(sv_trans_handle* h, void* state, size_t state_bytes,
   p.D = h->cfg.d_model; p.L = h->cfg.len_q; p.FF = h->cfg.d_ff; p.n_videos = n_ids;
   p.scale = 1.0f / sqrtf(static_cast<float>(h->cfg.d_k));
   int64_t* seen = static_cast<int64_t*>(state);
-  float* ring = reinterpret_cast<float*>(static_cast<char*>(state) + ((static_cast<size_t>(n_streams) * sizeof(int64_t) + 255) & ~static_cast<size_t>(255)));
+  float* ring = reinterpret_cast<float*>(static_cast<char*>(state) + StreamRegistry::counter_bytes(n_streams));
   const StreamWindow win{h->d_offsets + n_ids + 1, seen, ring};
   SV_TRY(launch_head(h->cfg.d_k, logits, ldx, query, h->d_offsets, T, h->d_blob, out, p, win, st));
   trans_stream_commit_kernel<<<n_ids, 128, 0, st>>>(logits, ldx, h->d_offsets, n_ids, p.D, p.L, ring, seen);
   SV_TRY(launch_status("trans_stream_commit_kernel"));
-  for (int i = 0; i < n_ids; ++i) it->second[stream_ids[i]] += counts[i];
+  h->streams.advance(state, stream_ids, counts, n_ids);
   return SV_OK;
 }
 

@@ -21,7 +21,6 @@ import os
 from functools import partial
 from typing import Optional
 
-import numpy as np
 import torch
 import torch.nn as nn
 
@@ -273,10 +272,7 @@ class MixVisionTransformerEVP(nn.Module):
                 self._native[idx] = st
             elif st["fold_head"] != self.fold_head:
                 raise RuntimeError("fold_head cannot change after the first forward on a device")
-            for name, t in self.state_dict().items():
-                a = np.ascontiguousarray(t.detach().to("cpu", torch.float32).numpy())
-                shape = (ctypes.c_int64 * max(a.ndim, 1))(*a.shape)
-                _native.check(lib.sv_evp_set_tensor(st["handle"], name.encode(), a.ctypes.data_as(ctypes.c_void_p), shape, a.ndim), "sv_evp_set_tensor")
+            _native.set_tensors(lib.sv_evp_set_tensor, st["handle"], self.state_dict().items(), "sv_evp_set_tensor")
             _native.check(lib.sv_evp_pack_weights(st["handle"]), "sv_evp_pack_weights")
         st["stamp"] = stamp
         if st["id"] is None:

@@ -99,14 +99,8 @@ class MultiStageModel_S(nn.Module):
                 _native.check(lib.sv_mstcn_create(ctypes.byref(cfg), ctypes.byref(h)), "sv_mstcn_create")
                 st = {"handle": h, "workspace": None, "id": None}
                 self._native[idx] = st
-            for name, t in self.state_dict().items():
-                a = np.ascontiguousarray(t.detach().to("cpu", torch.float32).numpy())
-                shape = (ctypes.c_int64 * max(a.ndim, 1))(*a.shape)
-                _native.check(lib.sv_mstcn_set_tensor(st["handle"], name.encode(), a.ctypes.data_as(ctypes.c_void_p), shape, a.ndim), "sv_mstcn_set_tensor")
-            if self._fc_weight is not None:
-                a = self._fc_weight.numpy()
-                shape = (ctypes.c_int64 * 2)(*a.shape)
-                _native.check(lib.sv_mstcn_set_tensor(st["handle"], b"fc.weight", a.ctypes.data_as(ctypes.c_void_p), shape, 2), "sv_mstcn_set_tensor")
+            fc = [] if self._fc_weight is None else [("fc.weight", self._fc_weight)]
+            _native.set_tensors(lib.sv_mstcn_set_tensor, st["handle"], list(self.state_dict().items()) + fc, "sv_mstcn_set_tensor")
             _native.check(lib.sv_mstcn_pack_weights(st["handle"]), "sv_mstcn_pack_weights")
         st["stamp"] = self._weights_epoch
         if st["id"] is None:

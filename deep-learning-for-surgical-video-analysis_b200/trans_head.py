@@ -146,10 +146,7 @@ class Transformer2_3_1(nn.Module):
                 _native.check(lib.sv_trans_create(ctypes.byref(cfg), ctypes.byref(h)), "sv_trans_create")
                 st = {"handle": h}
                 self._native[idx] = st
-            for name, t in self.state_dict().items():
-                a = np.ascontiguousarray(t.detach().to("cpu", torch.float32).numpy())
-                shape = (ctypes.c_int64 * max(a.ndim, 1))(*a.shape)
-                _native.check(lib.sv_trans_set_tensor(st["handle"], name.encode(), a.ctypes.data_as(ctypes.c_void_p), shape, a.ndim), "sv_trans_set_tensor")
+            _native.set_tensors(lib.sv_trans_set_tensor, st["handle"], self.state_dict().items(), "sv_trans_set_tensor")
             _native.check(lib.sv_trans_pack_weights(st["handle"]), "sv_trans_pack_weights")
         st["stamp"] = self._weights_epoch
         return st

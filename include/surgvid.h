@@ -67,11 +67,12 @@ int sv_evp_destroy(sv_evp_handle* h);
 
 /* Hand one state_dict entry (fp32, HOST memory, contiguous) to the handle.  `name` is the reference's
  * state_dict key (SURVEY.md §8b), e.g. "block3.7.attn.kv.weight".  replaces: load_state_dict
- * (generate_evp_LFB.py:414).  Unknown names -> SV_ERR_INVALID; wrong shape -> SV_ERR_INVALID. */
+ * (generate_evp_LFB.py:414).  host_data == NULL stores zeros; ndim <= 4.  Tensors are stored by name and checked at
+ * sv_evp_pack_weights; shape == NULL with ndim > 0, or a negative dimension -> SV_ERR_INVALID. */
 int sv_evp_set_tensor(sv_evp_handle* h, const char* name, const float* host_data, const int64_t* shape, int32_t ndim);
 
 /* Fold BatchNorm (eval) into the preceding conv, reorder conv weights to (kh,kw,cin)-major implicit-GEMM
- * form, convert to bf16 and upload.  Fails with SV_ERR_STATE listing the first missing key. */
+ * form, convert to bf16 and upload.  Fails with SV_ERR_STATE naming the first missing or wrongly shaped key. */
 int sv_evp_pack_weights(sv_evp_handle* h);
 
 /* Bytes of scratch the forward needs for `micro_batch` frames of HxW (frames are processed in
@@ -143,6 +144,8 @@ typedef struct sv_mstcn sv_mstcn_handle;
 
 int sv_mstcn_create(const sv_mstcn_cfg* cfg, sv_mstcn_handle** out);
 int sv_mstcn_destroy(sv_mstcn_handle* h);
+/* Tensors are stored by name and checked at sv_mstcn_pack_weights (missing key -> SV_ERR_STATE, wrong shape -> SV_ERR_INVALID);
+ * shape == NULL with ndim > 0, or a negative dimension -> SV_ERR_INVALID. */
 int sv_mstcn_set_tensor(sv_mstcn_handle* h, const char* name, const float* host_data, const int64_t* shape, int32_t ndim);
 int sv_mstcn_pack_weights(sv_mstcn_handle* h);
 size_t sv_mstcn_workspace_bytes(const sv_mstcn_handle* h, int64_t total_frames);
@@ -332,6 +335,8 @@ typedef struct sv_trans_cfg {
 typedef struct sv_trans sv_trans_handle;
 int sv_trans_create(const sv_trans_cfg* cfg, sv_trans_handle** out);
 int sv_trans_destroy(sv_trans_handle* h);
+/* Tensors are stored by name and checked at sv_trans_pack_weights (missing key -> SV_ERR_STATE, wrong shape -> SV_ERR_INVALID);
+ * shape == NULL with ndim > 0, or a negative dimension -> SV_ERR_INVALID. */
 int sv_trans_set_tensor(sv_trans_handle* h, const char* name, const float* host_data, const int64_t* shape, int32_t ndim);
 int sv_trans_pack_weights(sv_trans_handle* h);
 /* logits: fp32 channel-major [d_model][ldx] = the LAST stage of sv_mstcn_forward's output for the concatenated videos
