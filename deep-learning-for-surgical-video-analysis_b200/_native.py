@@ -34,11 +34,13 @@ EXPORTED_SYMBOLS = [
     "sv_trans_stream_state_bytes", "sv_trans_stream_reset", "sv_trans_stream_forward",
     "sv_evp_attention_maps_layout", "sv_evp_forward_attention", "sv_op_attention_probs", "sv_op_gemm_plan_info",
     "sv_op_conv_gemm_bf16", "sv_op_conv_gemm_plan_info",
+    "sv_evp_stage_shapes", "sv_evp_forward_features", "sv_op_layernorm_nchw",
 ]
 
 # entry points an earlier build of the library, loaded through SURGVID_LIB for a same-box A/B run, may not have (build() still requires
 # every EXPORTED_SYMBOLS entry of the library it builds)
-_ABSENT_IN_EARLIER_BUILDS = ("sv_op_conv_gemm_bf16", "sv_op_conv_gemm_plan_info")
+_ABSENT_IN_EARLIER_BUILDS = ("sv_op_conv_gemm_bf16", "sv_op_conv_gemm_plan_info", "sv_evp_stage_shapes", "sv_evp_forward_features",
+                             "sv_op_layernorm_nchw")
 
 
 class EvpCfg(Structure):
@@ -137,6 +139,11 @@ def _declare(lib):
                                              c_void_p, c_int32, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_void_p]
         lib.sv_op_conv_gemm_plan_info.argtypes = [c_int32] * 12 + [POINTER(c_int32), POINTER(c_int32)]
     lib.sv_op_layernorm.argtypes = [c_void_p, c_void_p, c_void_p, c_float, c_int64, c_int32, c_void_p, c_void_p, c_void_p]
+    if hasattr(lib, "sv_evp_forward_features"):   # see _ABSENT_IN_EARLIER_BUILDS
+        lib.sv_op_layernorm_nchw.argtypes = [c_void_p, c_void_p, c_void_p, c_float, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p]
+        lib.sv_evp_stage_shapes.argtypes = [POINTER(EvpCfg), c_int32, c_int32, POINTER(c_int32)]
+        lib.sv_evp_forward_features.argtypes = [c_void_p, c_void_p, c_void_p, POINTER(c_void_p), i64p, c_void_p, c_int64, c_int32, c_int32,
+                                                c_int32, c_int32, c_void_p, c_size_t, c_void_p]
     lib.sv_op_im2col.argtypes = [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int64, c_void_p]
     lib.sv_op_dwconv3x3_gelu.argtypes = [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]
     lib.sv_op_attention.argtypes = [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_int32, c_int32,

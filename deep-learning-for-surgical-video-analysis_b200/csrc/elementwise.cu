@@ -14,8 +14,13 @@ namespace {
 // The kernel is instruction-issue-bound before it is memory-bound, so the arithmetic is kept lean: 1/C is passed in, rstd is one
 // MUFU.RSQ (2 ulp, far below the bf16 rounding of the outputs), normalisation is one FFMA per element with per-channel a = rstd*gamma,
 // b = beta - mean*a.
-template <int LPR, int NV, bool EXACT>
-__global__ void __launch_bounds__(256, 5) layernorm_kernel(const float* __restrict__ x, const float* __restrict__ gamma,
+// NCHW: the fp32 result goes channel-major instead, out_f32[frame][c][token] with pH tokens per frame (the MiT stage maps that
+// forward_features returns); out_patch must be NULL.  The CTA's 8 * RPW rows are staged in shared memory, then every thread stores one
+// token position for C * RPW / 32 channels, so each channel's run of consecutive tokens goes out as one contiguous store of
+// 32 * RPW bytes (split where the run crosses a frame).  Arithmetic and lane mapping are those of the token-major form, so the fp32
+// written is the value out_bf16 rounds.  Four CTAs per SM instead of five: at five, the staging address math spills for C = 40, 80, 512.
+template <int LPR, int NV, bool EXACT, bool NCHW = false>
+__global__ void __launch_bounds__(256, NCHW ? 4 : 5) layernorm_kernel(const float* __restrict__ x, const float* __restrict__ gamma,
                                                          const float* __restrict__ beta, float eps, float inv_c, int64_t rows, int C,
                                                          float* __restrict__ out_f32, bf16* __restrict__ out_bf16,
                                                          bf16* __restrict__ out_patch, int pH, int pW, int psr) {
@@ -52,7 +57,9 @@ __global__ void __launch_bounds__(256, 5) layernorm_kernel(const float* __restri
 #pragma unroll
   for (int o = LPR / 2; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
   const float rstd = rsqrtf(q * inv_c + eps);
-  if (!row_ok) return;
+  if constexpr (!NCHW) {
+    if (!row_ok) return;
+  }
   // optional second bf16 copy in "sr-patch" order: token (b,h,w) -> row (b, h/sr, w/sr), column ((h%sr)*sr + w%sr)*C + c,
   // i.e. the A operand of the spatial-reduction conv (k = stride = sr, no padding) as a plain GEMM.
   int64_t patch_off = -1;
@@ -71,8 +78,12 @@ __global__ void __launch_bounds__(256, 5) layernorm_kernel(const float* __restri
   }
   const float4* g4 = reinterpret_cast<const float4*>(gamma) + sub;
   const float4* b4 = reinterpret_cast<const float4*>(beta) + sub;
-  float* of = out_f32 ? out_f32 + row * C + sub * 4 : nullptr;
-  bf16* ob = out_bf16 ? out_bf16 + row * C + sub * 4 : nullptr;
+  float* of = !NCHW && out_f32 ? out_f32 + row * C + sub * 4 : nullptr;
+  bf16* ob = out_bf16 && (!NCHW || row_ok) ? out_bf16 + row * C + sub * 4 : nullptr;
+  // NCHW staging tile [c][row of the CTA], row stride R + P: P makes the 4 scalar stores of a warp hit distinct banks where RPW >= 4
+  constexpr int R = 8 * RPW, P = RPW >= 4 ? RPW / 4 : 1;
+  __shared__ float tile[NCHW ? 4 * LPR * NV * (R + P) : 1];
+  const int lr = (threadIdx.x >> 5) * RPW + lane / LPR;
   bf16* op = patch_off >= 0 ? out_patch + patch_off + sub * 4 : nullptr;
   const float nm = -mean * rstd;
 #pragma unroll
@@ -86,6 +97,15 @@ __global__ void __launch_bounds__(256, 5) layernorm_kernel(const float* __restri
       y.z = fmaf(v[i].z, rstd * g.z, fmaf(nm, g.z, b.z));
       y.w = fmaf(v[i].w, rstd * g.w, fmaf(nm, g.w, b.w));
       if (of) *reinterpret_cast<float4*>(of + i * LPR * 4) = y;
+      if constexpr (NCHW) {
+        if (row_ok) {
+          float* t = tile + (sub + i * LPR) * 4 * (R + P) + lr;
+          t[0] = y.x;
+          t[R + P] = y.y;
+          t[2 * (R + P)] = y.z;
+          t[3 * (R + P)] = y.w;
+        }
+      }
       if (ob || op) {
         uint2 o;
         o.x = pack_bf16x2(y.x, y.y);
@@ -95,9 +115,22 @@ __global__ void __launch_bounds__(256, 5) layernorm_kernel(const float* __restri
       }
     }
   }
+  if constexpr (NCHW) {
+    __syncthreads();
+    // thread -> (row R-periodic, channel every 256 / R): the row, and with it the frame and token, is fixed per thread (32-bit math:
+    // rows * C < 2^31 is checked by the launcher)
+    const uint32_t t = threadIdx.x;
+    const uint32_t r32 = blockIdx.x * static_cast<uint32_t>(R) + (t & (R - 1));
+    if (r32 < static_cast<uint32_t>(rows)) {
+      const uint32_t hw = static_cast<uint32_t>(pH);
+      const uint32_t f = r32 / hw;
+      float* dst = out_f32 + f * static_cast<uint32_t>(C) * hw + (r32 - f * hw);
+      for (uint32_t c = t / R; c < static_cast<uint32_t>(C); c += 256 / R) __stcs(dst + c * hw, tile[c * (R + P) + (t & (R - 1))]);
+    }
+  }
 }
 
-template <int LPR, int NV>
+template <int LPR, int NV, bool NCHW>
 int ln_launch(const float* x, const float* g, const float* b, float eps, int64_t rows, int C, float* of, bf16* ob, bf16* op, int pH, int pW,
               int psr, cudaStream_t st) {
   constexpr int RPW = 32 / LPR;
@@ -105,10 +138,40 @@ int ln_launch(const float* x, const float* g, const float* b, float eps, int64_t
   const int64_t blocks = ceil_div64(warps, 8);
   const float inv_c = 1.0f / static_cast<float>(C);
   if (C == 4 * LPR * NV)
-    layernorm_kernel<LPR, NV, true><<<static_cast<unsigned>(blocks), 256, 0, st>>>(x, g, b, eps, inv_c, rows, C, of, ob, op, pH, pW, psr);
+    layernorm_kernel<LPR, NV, true, NCHW><<<static_cast<unsigned>(blocks), 256, 0, st>>>(x, g, b, eps, inv_c, rows, C, of, ob, op, pH, pW, psr);
   else
-    layernorm_kernel<LPR, NV, false><<<static_cast<unsigned>(blocks), 256, 0, st>>>(x, g, b, eps, inv_c, rows, C, of, ob, op, pH, pW, psr);
+    layernorm_kernel<LPR, NV, false, NCHW><<<static_cast<unsigned>(blocks), 256, 0, st>>>(x, g, b, eps, inv_c, rows, C, of, ob, op, pH, pW, psr);
   return launch_status("layernorm_kernel");
+}
+
+// lane mapping per width: one table for both output forms, so a channel-major result is bit-identical to the token-major one
+template <bool NCHW>
+int ln_dispatch(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int C, float* out_f32, bf16* out_bf16,
+                bf16* out_patch, int pH, int pW, int psr, cudaStream_t st) {
+  const int nvec = C / 4;
+#define SV_LN(L, N) return ln_launch<L, N, NCHW>(x, gamma, beta, eps, rows, C, out_f32, out_bf16, out_patch, pH, pW, psr, st)
+  // exact lane mappings first (every slot a real element): the model's widths 16/32/64/128/256/512 and 40/80/160/320
+  // (narrow rows: fewer lanes per row and two float4 per lane — the fixed per-thread work, shuffles and patch index math are
+  //  amortised over more bytes: 64 -> 49 us for 627200 x 64, 28 -> 26 us for 156800 x 128; ten float4 per lane for C = 320 spills)
+  if (nvec == 4) SV_LN(2, 2);
+  if (nvec == 8) SV_LN(4, 2);
+  if (nvec == 16) SV_LN(8, 2);
+  if (nvec == 32) SV_LN(8, 4);
+  if (nvec == 64) SV_LN(16, 4);
+  if (nvec == 128) SV_LN(32, 4);
+  if (nvec == 10) SV_LN(2, 5);
+  if (nvec == 20) SV_LN(4, 5);
+  if (nvec == 40) SV_LN(8, 5);
+  if (nvec == 80) SV_LN(16, 5);
+  // anything else: predicated slots
+  if (nvec <= 4) SV_LN(4, 1);
+  if (nvec <= 8) SV_LN(8, 1);
+  if (nvec <= 16) SV_LN(16, 1);
+  if (nvec <= 32) SV_LN(32, 1);
+  if (nvec <= 64) SV_LN(32, 2);
+  if (nvec <= 96) SV_LN(32, 3);
+  SV_LN(32, 4);
+#undef SV_LN
 }
 
 // ------------------------------------------------------------------------------------------ im2col
@@ -385,30 +448,20 @@ int launch_layernorm_patch(const float* x, const float* gamma, const float* beta
   if (out_patch)
     SV_CHECK(pH > 0 && pW > 0 && psr > 0 && (psr & (psr - 1)) == 0 && rows % (static_cast<int64_t>(pH) * pW) == 0 && rows < (1LL << 31),
              "layernorm patch geometry (sr must be a power of two)");
-  const int nvec = C / 4;
-#define SV_LN(L, N) return ln_launch<L, N>(x, gamma, beta, eps, rows, C, out_f32, out_bf16, out_patch, pH, pW, psr, st)
-  // exact lane mappings first (every slot a real element): the model's widths 16/32/64/128/256/512 and 40/80/160/320
-  // (narrow rows: fewer lanes per row and two float4 per lane — the fixed per-thread work, shuffles and patch index math are
-  //  amortised over more bytes: 64 -> 49 us for 627200 x 64, 28 -> 26 us for 156800 x 128; ten float4 per lane for C = 320 spills)
-  if (nvec == 4) SV_LN(2, 2);
-  if (nvec == 8) SV_LN(4, 2);
-  if (nvec == 16) SV_LN(8, 2);
-  if (nvec == 32) SV_LN(8, 4);
-  if (nvec == 64) SV_LN(16, 4);
-  if (nvec == 128) SV_LN(32, 4);
-  if (nvec == 10) SV_LN(2, 5);
-  if (nvec == 20) SV_LN(4, 5);
-  if (nvec == 40) SV_LN(8, 5);
-  if (nvec == 80) SV_LN(16, 5);
-  // anything else: predicated slots
-  if (nvec <= 4) SV_LN(4, 1);
-  if (nvec <= 8) SV_LN(8, 1);
-  if (nvec <= 16) SV_LN(16, 1);
-  if (nvec <= 32) SV_LN(32, 1);
-  if (nvec <= 64) SV_LN(32, 2);
-  if (nvec <= 96) SV_LN(32, 3);
-  SV_LN(32, 4);
-#undef SV_LN
+  return ln_dispatch<false>(x, gamma, beta, eps, rows, C, out_f32, out_bf16, out_patch, pH, pW, psr, st);
+}
+
+int launch_layernorm_nchw(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int C, int tokens, float* out_nchw,
+                          bf16* out_bf16, cudaStream_t st) {
+  SV_CHECK(x && gamma && beta && out_nchw, "layernorm_nchw: null argument");
+  SV_CHECK(C % 4 == 0 && C >= 4 && C <= 512, "layernorm supports C%4==0, C<=512");
+  SV_CHECK(tokens > 0 && rows > 0 && rows % tokens == 0, "layernorm_nchw: rows must be a positive multiple of the tokens per frame");
+  SV_CHECK(rows * C < (1LL << 31), "layernorm_nchw: rows * C must be below 2^31");
+  SV_CHECK((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(gamma) & 15) == 0 &&
+               (reinterpret_cast<uintptr_t>(beta) & 15) == 0 && (reinterpret_cast<uintptr_t>(out_nchw) & 3) == 0 &&
+               (reinterpret_cast<uintptr_t>(out_bf16) & 7) == 0,
+           "layernorm_nchw: alignment (x, gamma, beta 16 bytes, out_bf16 8, out_nchw 4)");
+  return ln_dispatch<true>(x, gamma, beta, eps, rows, C, out_nchw, out_bf16, nullptr, tokens, 0, 0, st);
 }
 
 int launch_layernorm(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int C, float* out_f32,
@@ -485,6 +538,11 @@ extern "C" {
 int sv_op_layernorm(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int32_t C, float* out_f32,
                     uint16_t* out_bf16, void* stream) {
   return sv::launch_layernorm(x, gamma, beta, eps, rows, C, out_f32, reinterpret_cast<sv::bf16*>(out_bf16), static_cast<cudaStream_t>(stream));
+}
+int sv_op_layernorm_nchw(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int32_t C, int32_t tokens_per_frame,
+                         float* out_nchw, uint16_t* out_bf16, void* stream) {
+  return sv::launch_layernorm_nchw(x, gamma, beta, eps, rows, C, tokens_per_frame, out_nchw, reinterpret_cast<sv::bf16*>(out_bf16),
+                                   static_cast<cudaStream_t>(stream));
 }
 int sv_op_im2col(const float* src_nchw_f32, const uint16_t* src_nhwc_bf16, int32_t B, int32_t Cin, int32_t H, int32_t W, int32_t k,
                  int32_t stride, int32_t pad, uint16_t* out, int64_t ldo, void* stream) {

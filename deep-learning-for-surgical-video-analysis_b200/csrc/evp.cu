@@ -62,6 +62,7 @@ enum OpKind { OP_GEMM, OP_LN, OP_IM2COL, OP_DWCONV, OP_ATTN, OP_GAUSS, OP_BILINE
 struct CallIO {
   const float *x, *seg, *flow; float* out;
   float* const* maps;  // per encoder block, where this micro-batch's attention maps go (capture plans only)
+  float* const* stage_out;  // per stage, where this micro-batch's fp32 NCHW stage map goes (encoder-only plans only)
 };
 // where im2col and the stem read their fp32 NCHW input: a workspace buffer, or the call's x or flow
 enum Ext { EXT_NONE, EXT_X, EXT_FLOW };
@@ -119,6 +120,14 @@ struct ProbsOp {  // softmax(Q K^T * scale) of encoder block `block` into the ca
   int launch(const CallIO& io, cudaStream_t st) const { return launch_attention_probs(q, ldq, k, ldk, B, heads, Nq, Nkv, hd, scale, io.maps[block], st); }
   ProfCols cols() const { return {ldq, {B, heads, Nq, Nkv, hd}}; }
 };
+struct StageNormOp {  // stage norm of the encoder-only plans: fp32 result channel-major into the call's stage_out[stage]
+  static constexpr OpKind kind = OP_LN;
+  const float *x, *gamma, *beta; float eps; int64_t rows; int C, tokens; bf16* out_bf16; int stage;
+  int launch(const CallIO& io, cudaStream_t st) const {
+    return launch_layernorm_nchw(x, gamma, beta, eps, rows, C, tokens, io.stage_out[stage], out_bf16, st);
+  }
+  ProfCols cols() const { return {rows, {C, tokens, 0, 0, stage}}; }
+};
 struct GaussOp {  // of the call's seg
   static constexpr OpKind kind = OP_GAUSS;
   float* out; int planes, H, W;
@@ -148,7 +157,8 @@ struct StemOp {  // mode 0: LayerNorm, 1: ReLU
 };
 
 struct Op {
-  std::variant<GemmOp, LayerNormOp, Im2colOp, DwconvTmaOp, DwconvOp, AttnTcOp, AttnOp, ProbsOp, GaussOp, BilinearOp, MeanOp, StemOp> rec;
+  std::variant<GemmOp, LayerNormOp, Im2colOp, DwconvTmaOp, DwconvOp, AttnTcOp, AttnOp, ProbsOp, StageNormOp, GaussOp, BilinearOp, MeanOp, StemOp>
+      rec;
   double alg_bytes = 0.0;         // algorithmic HBM bytes of this launch (operands + results once)
   mutable double prof_ms = 0.0;   // filled only in profiling mode
   mutable long long prof_n = 0;
@@ -496,17 +506,35 @@ void stage_geometry(const sv_evp_cfg& c, int H, int W, StageGeom (&g)[4]) {
   }
 }
 
+// stage_geometry of a checked config and input size (the host-only queries take the config from the caller)
+int pyramid(const sv_evp_cfg& c, int H, int W, StageGeom (&g)[4]) {
+  if (H <= 0 || W <= 0) return fail(SV_ERR_INVALID, "evp: H and W must be positive");
+  for (int s = 0; s < 4; ++s)
+    if (c.embed_dims[s] <= 0 || c.num_heads[s] <= 0 || c.depths[s] <= 0 || c.sr_ratios[s] <= 0 || c.embed_dims[s] % c.num_heads[s] != 0)
+      return fail(SV_ERR_INVALID, "evp: bad config (non-positive entry or dim not divisible by heads)");
+  stage_geometry(c, H, W, g);
+  for (int s = 0; s < 4; ++s)
+    if (g[s].H < 1 || g[s].W < 1 || g[s].Hk < 1 || g[s].Wk < 1) return fail(SV_ERR_INVALID, "evp: input too small for the 4-stage pyramid");
+  return SV_OK;
+}
+
+// pyramid() for forward_features, which also rejects what the reference's forward_features cannot run: a stage map smaller than
+// its spatial-reduction window (Conv2d(kernel = stride = sr) raises there; at 224 / 4 / 8 / ... the smallest input is 29 x 29)
+int features_pyramid(const sv_evp_cfg& c, int H, int W, StageGeom (&g)[4]) {
+  SV_TRY(pyramid(c, H, W, g));
+  for (int s = 0; s < 4; ++s)
+    if (g[s].sr > 1 && (g[s].H < g[s].sr || g[s].W < g[s].sr))
+      return fail(SV_ERR_INVALID, "evp: input too small for the 4-stage pyramid: stage " + std::to_string(s + 1) + " is " + std::to_string(g[s].H) +
+                                      "x" + std::to_string(g[s].W) + ", smaller than its spatial-reduction window " + std::to_string(g[s].sr));
+  return SV_OK;
+}
+
 // Where each encoder block's attention maps [B, heads, N, N_kv] (fp32) go in one buffer, in call order (stage 1 blocks first).
 // off has n_blocks + 1 entries (element offsets; the last is the total), dims 3 per block.
 int maps_layout(const sv_evp_cfg& c, int B, int H, int W, std::vector<int64_t>* off, std::vector<int32_t>* dims) {
   if (B <= 0 || H <= 0 || W <= 0) return fail(SV_ERR_INVALID, "evp: B, H and W must be positive");
-  for (int s = 0; s < 4; ++s)
-    if (c.embed_dims[s] <= 0 || c.num_heads[s] <= 0 || c.depths[s] <= 0 || c.sr_ratios[s] <= 0 || c.embed_dims[s] % c.num_heads[s] != 0)
-      return fail(SV_ERR_INVALID, "evp: bad config (non-positive entry or dim not divisible by heads)");
   StageGeom g[4];
-  stage_geometry(c, H, W, g);
-  for (int s = 0; s < 4; ++s)
-    if (g[s].H < 1 || g[s].W < 1 || g[s].Hk < 1 || g[s].Wk < 1) return fail(SV_ERR_INVALID, "evp: input too small for the 4-stage pyramid");
+  SV_TRY(pyramid(c, H, W, g));
   off->assign(1, 0);
   dims->clear();
   for (int s = 0; s < 4; ++s)
@@ -608,6 +636,10 @@ struct Builder {
     push(ProbsOp{q, ldq, k, ldk, B, heads, Nq, Nkv, hd, 1.0f / sqrtf(static_cast<float>(hd)), block},
          2.0 * B * heads * hd * (static_cast<double>(Nq) + Nkv) + 4.0 * B * heads * static_cast<double>(Nq) * Nkv);
   }
+  // stage norm of the encoder-only plans: channel-major fp32 into the caller's stage_out[stage] (resolved per call, see run_plan)
+  void stage_norm(const float* x, const Norm& n, float eps, int64_t rows, int tokens, bf16* ob, int stage) {
+    push(StageNormOp{x, F(n.g), F(n.b), eps, rows, n.C, tokens, ob, stage}, static_cast<double>(rows) * n.C * (4 + 4 + 2));
+  }
   void gauss(float* out, int planes, int H, int W) { push(GaussOp{out, planes, H, W}, 8.0 * planes * H * W); }
   void bilinear(const bf16* x, int B, int H, int W, int C, int Ho, int Wo, bf16* out, int64_t ldo) { push(BilinearOp{x, B, H, W, C, Ho, Wo, out, ldo}, 0.0); }
   void mean(const float* x, int B, int tokens, int C) { push(MeanOp{x, B, tokens, C}, 0.0); }
@@ -629,8 +661,10 @@ bool flow_supported(const sv_evp_cfg& c) {
   return true;
 }
 
-// Builds (or only sizes, when plan == nullptr) the launch schedule for n frames of HxW.
-int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, bool capture, size_t* bytes_out) {
+// Builds (or only sizes, when plan == nullptr) the launch schedule for n frames of HxW.  features_only: the encoder-only plan of
+// forward_features, which ends with the stage norms writing the call's fp32 NCHW stage maps (no flow branch, no head); it addresses a
+// prefix of the workspace of the full plan without flow.
+int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, bool capture, bool features_only, size_t* bytes_out) {
   const sv_evp_cfg& c = h->cfg;
   Builder b(h, plan, ws);
   Arena& A = b.arena;
@@ -792,10 +826,15 @@ int build(sv_evp* h, Plan* plan, void* ws, int n, int H, int W, bool with_flow, 
           b.gemm(h2, ldh, Bk.fc2, M, ACT_NONE, x, C, x, C, 1);
         }
       }
-      b.ln(x, S.norm, 1e-6f, M, c_f32[s], c_b16[s]);
+      if (features_only) b.stage_norm(x, S.norm, 1e-6f, M, G.N, c_b16[s], s);
+      else b.ln(x, S.norm, 1e-6f, M, c_f32[s], c_b16[s]);
       b.tap("stage" + std::to_string(s + 1) + "_tokens", c_b16[s], static_cast<int64_t>(M) * C);
       hh = G.H; ww = G.W;
     }
+  }
+  if (features_only) {
+    if (bytes_out) *bytes_out = ((A.off + 255) & ~static_cast<size_t>(255)) + 256;
+    return b.status;
   }
   // ---- 2. optical-flow branch (:423-444)
   const bf16* head_in[4] = {c_b16[0], c_b16[1], c_b16[2], c_b16[3]};
@@ -981,7 +1020,7 @@ size_t sv_evp_workspace_bytes(const sv_evp_handle* h, int32_t micro_batch, int32
   size_t bytes = 0;
   // sized for the larger of the two schedules (with the flow branch); configurations whose flow branch is unsupported can only
   // ever run without it
-  if (sv::build(const_cast<sv_evp*>(h), nullptr, nullptr, micro_batch, H, W, sv::flow_supported(h->cfg), false, &bytes) != SV_OK) return 0;
+  if (sv::build(const_cast<sv_evp*>(h), nullptr, nullptr, micro_batch, H, W, sv::flow_supported(h->cfg), false, false, &bytes) != SV_OK) return 0;
   return bytes;
 }
 
@@ -991,10 +1030,12 @@ namespace sv {
 namespace {
 // maps == nullptr: the plain forward.  Otherwise the capture plans run, and block k's maps of frames [b0, b0 + n) go to
 // maps + off[k] + b0 * heads_k * N_k * Nkv_k.
+// stage_out != nullptr: the encoder-only plans run (no flow, no features), and stage s of frames [b0, b0 + n) goes to
+// stage_out[s] + b0 * C_s * H_s * W_s.
 int evp_forward(sv_evp_handle* h, const float* x, const float* seg, const float* flow, float* out_features, float* maps, const std::vector<int64_t>& off,
-                const std::vector<int32_t>& dims, int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace, size_t workspace_bytes,
-                void* stream) {
-  SV_CHECK(h && x && seg && out_features && workspace, "null argument");
+                const std::vector<int32_t>& dims, float* const* stage_out, int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace,
+                size_t workspace_bytes, void* stream) {
+  SV_CHECK(h && x && seg && (out_features || stage_out) && workspace, "null argument");
   if (!h->sd.packed) return fail(SV_ERR_STATE, "evp: pack_weights() has not been called");
   SV_CHECK(B > 0 && micro_batch > 0, "evp: B and micro_batch must be positive");
   SV_CHECK((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "evp: workspace must be 256-byte aligned");
@@ -1004,15 +1045,20 @@ int evp_forward(sv_evp_handle* h, const float* x, const float* seg, const float*
   h->launches = 0;
   const int E = h->cfg.embedding_dim;
   const bool capture = maps != nullptr;
+  const bool features_only = stage_out != nullptr;
   std::vector<float*> block_maps(capture ? off.size() - 1 : 0);
+  StageGeom g[4];
+  if (features_only) stage_geometry(h->cfg, H, W, g);
+  float* stage_ptr[4] = {nullptr, nullptr, nullptr, nullptr};
   for (int b0 = 0; b0 < B; b0 += micro_batch) {
     const int n = std::min<int>(micro_batch, B - b0);
-    const long long key = (static_cast<long long>(n) << 40) ^ (static_cast<long long>(H) << 24) ^ (static_cast<long long>(W) << 8) ^ (with_flow ? 1 : 0) ^ (capture ? 2 : 0);
+    const long long key = (static_cast<long long>(n) << 40) ^ (static_cast<long long>(H) << 24) ^ (static_cast<long long>(W) << 8) ^ (with_flow ? 1 : 0) ^ (capture ? 2 : 0) ^
+                         (features_only ? 4 : 0);
     auto it = h->plans.find(key);
     if (it == h->plans.end() || it->second->ws != workspace) {
       std::unique_ptr<Plan> p(new Plan());
       p->n = n; p->H = H; p->W = W; p->with_flow = with_flow; p->ws = workspace;
-      SV_TRY(build(h, p.get(), workspace, n, H, W, with_flow, capture, &p->need));
+      SV_TRY(build(h, p.get(), workspace, n, H, W, with_flow, capture, features_only, &p->need));
       if (it == h->plans.end() && h->plans.size() >= kMaxPlans) {  // evict the least recently used plan (never the one just run)
         auto victim = h->plans.end();
         for (auto jt = h->plans.begin(); jt != h->plans.end(); ++jt)
@@ -1030,8 +1076,10 @@ int evp_forward(sv_evp_handle* h, const float* x, const float* seg, const float*
     const size_t in_off = static_cast<size_t>(b0) * 3 * H * W;
     for (size_t k = 0; k < block_maps.size(); ++k)
       block_maps[k] = maps + off[k] + static_cast<int64_t>(b0) * dims[3 * k] * dims[3 * k + 1] * dims[3 * k + 2];
-    const CallIO io{x + in_off, seg + in_off, with_flow ? flow + static_cast<size_t>(b0) * 2 * H * W : nullptr, out_features + static_cast<size_t>(b0) * E,
-                    block_maps.data()};
+    if (features_only)
+      for (int s = 0; s < 4; ++s) stage_ptr[s] = stage_out[s] + static_cast<int64_t>(b0) * g[s].C * g[s].N;
+    const CallIO io{x + in_off, seg + in_off, with_flow ? flow + static_cast<size_t>(b0) * 2 * H * W : nullptr,
+                    out_features ? out_features + static_cast<size_t>(b0) * E : nullptr, block_maps.data(), stage_ptr};
     SV_TRY(run_plan(h, plan, io, st));
     h->last_plan = it->second.get();
   }
@@ -1044,7 +1092,7 @@ extern "C" {
 
 int sv_evp_forward(sv_evp_handle* h, const float* x, const float* seg, const float* flow, float* out_features, int32_t B, int32_t H,
                    int32_t W, int32_t micro_batch, void* workspace, size_t workspace_bytes, void* stream) {
-  return sv::evp_forward(h, x, seg, flow, out_features, nullptr, {}, {}, B, H, W, micro_batch, workspace, workspace_bytes, stream);
+  return sv::evp_forward(h, x, seg, flow, out_features, nullptr, {}, {}, nullptr, B, H, W, micro_batch, workspace, workspace_bytes, stream);
 }
 
 int sv_evp_attention_maps_layout(const sv_evp_cfg* cfg, int32_t B, int32_t H, int32_t W, int64_t* block_offsets, int32_t* block_dims,
@@ -1076,7 +1124,49 @@ int sv_evp_forward_attention(sv_evp_handle* h, const float* x, const float* seg,
   if (maps_elems < off.back())
     return fail(SV_ERR_INVALID, "evp: maps buffer too small: " + std::to_string(maps_elems) + " elements given, " + std::to_string(off.back()) +
                                     " needed (sv_evp_attention_maps_layout)");
-  return evp_forward(h, x, seg, flow, out_features, maps, off, dims, B, H, W, micro_batch, workspace, workspace_bytes, stream);
+  return evp_forward(h, x, seg, flow, out_features, maps, off, dims, nullptr, B, H, W, micro_batch, workspace, workspace_bytes, stream);
+}
+
+int sv_evp_stage_shapes(const sv_evp_cfg* cfg, int32_t H, int32_t W, int32_t dims[12]) {
+  using namespace sv;
+  SV_CHECK(cfg && dims, "null argument");
+  StageGeom g[4];
+  SV_TRY(features_pyramid(*cfg, H, W, g));
+  for (int s = 0; s < 4; ++s) {
+    dims[3 * s] = g[s].C;
+    dims[3 * s + 1] = g[s].H;
+    dims[3 * s + 2] = g[s].W;
+  }
+  return SV_OK;
+}
+
+int sv_evp_forward_features(sv_evp_handle* h, const float* x, const float* seg, float* const stage_out[4], const int64_t stage_elems[4],
+                            float* maps, int64_t maps_elems, int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace,
+                            size_t workspace_bytes, void* stream) {
+  using namespace sv;
+  SV_CHECK(h && x && seg && stage_out && stage_elems && workspace, "null argument");
+  SV_CHECK(B > 0 && micro_batch > 0, "evp: B and micro_batch must be positive");
+  StageGeom g[4];
+  SV_TRY(features_pyramid(h->cfg, H, W, g));
+  for (int s = 0; s < 4; ++s) {
+    const std::string what = "evp: stage_out[" + std::to_string(s) + "]";
+    if (!stage_out[s]) return fail(SV_ERR_INVALID, what + " is NULL");
+    if ((reinterpret_cast<uintptr_t>(stage_out[s]) & 3) != 0) return fail(SV_ERR_INVALID, what + " must be 4-byte aligned");
+    const int64_t need = static_cast<int64_t>(B) * g[s].C * g[s].N;
+    if (stage_elems[s] < need)
+      return fail(SV_ERR_INVALID, what + " too small: " + std::to_string(stage_elems[s]) + " elements given, " + std::to_string(need) +
+                                      " needed (B * C * H * W of sv_evp_stage_shapes)");
+  }
+  std::vector<int64_t> off;
+  std::vector<int32_t> dims;
+  if (maps) {
+    SV_TRY(maps_layout(h->cfg, B, H, W, &off, &dims));
+    SV_CHECK((reinterpret_cast<uintptr_t>(maps) & 15) == 0, "evp: maps must be 16-byte aligned");
+    if (maps_elems < off.back())
+      return fail(SV_ERR_INVALID, "evp: maps buffer too small: " + std::to_string(maps_elems) + " elements given, " + std::to_string(off.back()) +
+                                      " needed (sv_evp_attention_maps_layout)");
+  }
+  return evp_forward(h, x, seg, nullptr, nullptr, maps, off, dims, stage_out, B, H, W, micro_batch, workspace, workspace_bytes, stream);
 }
 
 int sv_evp_classify(sv_evp_handle* h, const float* feats, float* y, float* y_ant, int32_t B, void* stream) {

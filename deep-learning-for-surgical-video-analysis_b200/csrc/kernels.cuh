@@ -8,6 +8,9 @@ int launch_layernorm(const float* x, const float* gamma, const float* beta, floa
                      bf16* out_bf16, cudaStream_t st);
 int launch_layernorm_patch(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int C, float* out_f32,
                            bf16* out_bf16, bf16* out_patch, int pH, int pW, int psr, cudaStream_t st);
+// the same LayerNorm with its fp32 result channel-major, out_nchw[frame][c][token] (tokens per frame; rows * C < 2^31)
+int launch_layernorm_nchw(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int C, int tokens, float* out_nchw,
+                          bf16* out_bf16, cudaStream_t st);
 int launch_im2col(const float* src_nchw_f32, const bf16* src_nhwc_bf16, int B, int Cin, int H, int W, int k, int stride, int pad,
                   bf16* out, int64_t ldo, cudaStream_t st);
 int launch_dwconv3x3_gelu(const bf16* x, const float* w9c, const float* bias, int B, int H, int W, int C, bf16* out, int64_t ldo,

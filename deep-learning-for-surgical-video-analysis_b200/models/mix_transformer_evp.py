@@ -4,7 +4,8 @@ Same constructors (`mit_b0_evp()` ... `mit_b5_evp()`, `MixVisionTransformerEVP(.
 `state_dict()` keys and shapes (722 keys for b3; SURVEY.md §8b), same call
 `model.forward(x, y, flow=None, return_features=False)` (mix_transformer_evp.py:418-449) — but the modules below are
 *parameter holders only*: the arithmetic runs in libsurgvid.so (hand-written sm_100a kernels) behind the custom op
-`torch.ops.surgvid.evp_lfb_forward`.  There is no PyTorch / CPU fallback: calling a holder directly, or calling the
+`torch.ops.surgvid.evp_lfb_forward` (and `torch.ops.surgvid.evp_forward_features` for the feature pyramid of
+`model.forward_features(x, y)`).  There is no PyTorch / CPU fallback: calling a holder directly, or calling the
 model on a non-CUDA tensor, raises.
 
 Differences from the reference, all deliberate:
@@ -255,6 +256,13 @@ class MixVisionTransformerEVP(nn.Module):
                       "sv_evp_attention_maps_layout")
         return list(off), [tuple(dims[3 * i:3 * i + 3]) for i in range(nb.value)]
 
+    def stage_shapes(self, H: int, W: int):
+        """Host only: [(C_s, H_s, W_s)] of the four stage maps `forward_features` returns for an HxW input (sv_evp_stage_shapes)."""
+        dims = (ctypes.c_int32 * 12)()
+        cfg = self._cfg()
+        _native.check(_native.lib().sv_evp_stage_shapes(ctypes.byref(cfg), H, W, dims), "sv_evp_stage_shapes")
+        return [tuple(dims[3 * s:3 * s + 3]) for s in range(4)]
+
     def _state(self, device: torch.device):
         """Per-device native handle with packed weights; re-packed after load_state_dict / .to() / refresh_weights()."""
         idx = device.index if device.index is not None else torch.cuda.current_device()
@@ -279,24 +287,29 @@ class MixVisionTransformerEVP(nn.Module):
             st["id"] = ops.register_handle(_EvpOpOwner(self, idx))
         return st
 
-    def _native_forward(self, idx: int, x, seg, flow, micro_batch, maps=None):
-        """maps: None, or an fp32 buffer of the layout's total element count (then the capture forward also fills it)."""
-        st = self._native[idx]
-        lib = _native.lib()
-        B, _, H, W = x.shape
-        mb = max(1, min(int(micro_batch), B))
+    @staticmethod
+    def _workspace(st, device, mb: int, H: int, W: int) -> torch.Tensor:
         # one grow-only workspace per device and resolution: smaller batches reuse it, so the cached launch plans (keyed by
         # frame count and workspace address inside the handle) stay valid across calls with different B
         key = (H, W)
-        nbytes = lib.sv_evp_workspace_bytes(st["handle"], mb, H, W)
+        nbytes = _native.lib().sv_evp_workspace_bytes(st["handle"], mb, H, W)
         if nbytes == 0:
             raise RuntimeError("sv_evp_workspace_bytes failed: " + _native.last_error())
         ws = st["workspace"].get(key)
         if ws is None or ws.numel() < nbytes:
             ws = None
             st["workspace"].pop(key, None)
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
             st["workspace"][key] = ws
+        return ws
+
+    def _native_forward(self, idx: int, x, seg, flow, micro_batch, maps=None):
+        """maps: None, or an fp32 buffer of the layout's total element count (then the capture forward also fills it)."""
+        st = self._native[idx]
+        lib = _native.lib()
+        B, _, H, W = x.shape
+        mb = max(1, min(int(micro_batch), B))
+        ws = self._workspace(st, x.device, mb, H, W)
         out = torch.empty((B, self.embedding_dim), dtype=torch.float32, device=x.device)
         args = (ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(seg.data_ptr()), ctypes.c_void_p(0 if flow is None else flow.data_ptr()),
                 ctypes.c_void_p(out.data_ptr()))
@@ -307,6 +320,22 @@ class MixVisionTransformerEVP(nn.Module):
             _native.check(lib.sv_evp_forward_attention(st["handle"], *args, ctypes.c_void_p(maps.data_ptr()), maps.numel(), *tail),
                           "sv_evp_forward_attention")
         return out
+
+    def _native_forward_features(self, idx: int, x, seg, micro_batch, maps=None):
+        """-> four fp32 [B, C_s, H_s, W_s] tensors from the encoder-only plans; maps as in `_native_forward`."""
+        st = self._native[idx]
+        B, _, H, W = x.shape
+        mb = max(1, min(int(micro_batch), B))
+        ws = self._workspace(st, x.device, mb, H, W)
+        outs = [torch.empty((B, c, h, w), dtype=torch.float32, device=x.device) for c, h, w in self.stage_shapes(H, W)]
+        ptrs = (ctypes.c_void_p * 4)(*[o.data_ptr() for o in outs])
+        elems = (ctypes.c_int64 * 4)(*[o.numel() for o in outs])
+        _native.check(_native.lib().sv_evp_forward_features(
+            st["handle"], ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(seg.data_ptr()), ptrs, elems,
+            ctypes.c_void_p(0 if maps is None else maps.data_ptr()), 0 if maps is None else maps.numel(), B, H, W, mb,
+            ctypes.c_void_p(ws.data_ptr()), ws.numel(), ctypes.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)),
+            "sv_evp_forward_features")
+        return outs
 
     def last_launch_count(self, device=None) -> int:
         idx = torch.cuda.current_device() if device is None else torch.device(device).index
@@ -331,8 +360,26 @@ class MixVisionTransformerEVP(nn.Module):
 
     # ------------------------------------------------------------------ forward
     def forward_features(self, x, y):
-        raise RuntimeError("forward_features is fused into torch.ops.surgvid.evp_lfb_forward; per-stage tensors are available "
-                           "through model.read_tap('stage{1..4}_tokens') after a forward")
+        """The encoder's feature pyramid (mix_transformer_evp.py:352-416): [norm_s(x_s) for s in 1..4] as four contiguous fp32 CUDA
+        tensors [B, C_s, H_s, W_s] (NCHW; `stage_shapes(H, W)`), from x, y of [B, 3, H, W] or [B, 1, 3, H, W] at any HxW `forward`
+        accepts.  Runs the encoder only: no flow branch, no SegFormer head.  Same rules as `forward` (inference only, CUDA only).
+        While `visualizer.get_local` is active it also appends the per-block attention maps to the cache, as `forward` does."""
+        x, y, _ = self._inputs(x, y, None)
+        if y.shape[0] != x.shape[0]:
+            raise ValueError(f"forward_features: x has {x.shape[0]} frames, y has {y.shape[0]}")
+        st = self._state(x.device)
+        caches = visualizer.active_caches()
+        if not caches:
+            return torch.ops.surgvid.evp_forward_features(x, y, st["id"], self.micro_batch)
+        B, _, H, W = x.shape
+        off, dims = self.attention_maps_layout(B, H, W)
+        buf = torch.empty(off[-1], dtype=torch.float32, device=x.device)
+        idx = x.device.index if x.device.index is not None else torch.cuda.current_device()
+        outs = self._native_forward_features(idx, x, y, self.micro_batch, maps=buf)
+        arrays = [buf[off[i]:off[i + 1]].view(B, *dims[i]).cpu().numpy() for i in range(len(dims))]
+        for cache in caches:
+            cache.setdefault(visualizer.QUALNAME, []).extend(arrays)
+        return outs
 
     def _inputs(self, x, y, flow):
         if self.training:
@@ -400,6 +447,12 @@ class _EvpOpOwner:
 
     def _native_forward(self, x, seg, flow, micro_batch):
         return self._model()._native_forward(self._idx, x, seg, flow, micro_batch)
+
+    def _native_forward_features(self, x, seg, micro_batch):
+        return self._model()._native_forward_features(self._idx, x, seg, micro_batch)
+
+    def stage_shapes(self, H, W):
+        return self._model().stage_shapes(H, W)
 
 
 # (embed_dims, depths) of the six published variants (mix_transformer_evp.py:894-943); everything else is shared:

@@ -7,7 +7,7 @@ from __future__ import annotations
 
 import ctypes
 import itertools
-from typing import Dict, Optional
+from typing import Dict, List, Optional
 
 import torch
 
@@ -42,6 +42,19 @@ def evp_lfb_forward(x: torch.Tensor, seg: torch.Tensor, flow: Optional[torch.Ten
 @evp_lfb_forward.register_fake
 def _(x, seg, flow, handle, micro_batch):
     return x.new_empty((x.shape[0], _HANDLES[handle].embedding_dim), dtype=torch.float32)
+
+
+@torch.library.custom_op("surgvid::evp_forward_features", mutates_args=())
+def evp_forward_features(x: torch.Tensor, seg: torch.Tensor, handle: int, micro_batch: int) -> List[torch.Tensor]:
+    """[B,3,H,W] frames + segmaps -> the encoder's four stage maps, fp32 NCHW [B, C_s, H_s, W_s] (encoder only: no flow, no head).
+    Replaces MixVisionTransformerEVP.forward_features(x, y) (mix_transformer_evp.py:352-416)."""
+    return _HANDLES[handle]._native_forward_features(x, seg, micro_batch)
+
+
+@evp_forward_features.register_fake
+def _(x, seg, handle, micro_batch):
+    B, _, H, W = x.shape
+    return [x.new_empty((B, c, h, w), dtype=torch.float32) for c, h, w in _HANDLES[handle].stage_shapes(H, W)]
 
 
 @torch.library.custom_op("surgvid::mstcn_forward", mutates_args=())
@@ -207,6 +220,19 @@ def layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: flo
     rc = _native.lib().sv_op_layernorm(_ptr(x), _ptr(gamma), _ptr(beta), eps, rows, C, _ptr(of), _ptr(ob), _stream_ptr(x.device))
     _native.check(rc, "sv_op_layernorm")
     return of, ob
+
+
+def layernorm_nchw(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, tokens_per_frame: int, want_bf16=False):
+    """LayerNorm of token-major fp32 x [frames * tokens_per_frame, C] -> (fp32 [frames, C, tokens_per_frame] channel-major, the
+    token-major bf16 [rows, C] or None); bit-identical to `layernorm(..., want_f32=True)[0]` permuted (sv_op_layernorm_nchw)."""
+    _require_cuda(x, gamma, beta)
+    rows, C = x.shape
+    out = torch.empty((rows // tokens_per_frame, C, tokens_per_frame), dtype=torch.float32, device=x.device)
+    ob = torch.empty((rows, C), dtype=torch.bfloat16, device=x.device) if want_bf16 else None
+    rc = _native.lib().sv_op_layernorm_nchw(_ptr(x), _ptr(gamma), _ptr(beta), eps, rows, C, tokens_per_frame, _ptr(out), _ptr(ob),
+                                            _stream_ptr(x.device))
+    _native.check(rc, "sv_op_layernorm_nchw")
+    return out, ob
 
 
 def im2col(src: torch.Tensor, k: int, stride: int, pad: int, ldo: Optional[int] = None) -> torch.Tensor:

@@ -9,8 +9,9 @@ this repository, so these semantics are not pinned against that file.
 Here the encoder runs in native kernels and no Python `Attention.forward` exists to decorate, so:
   * the decorator returns the function unchanged (no bytecode rewriting; the `bytecode` package is not needed);
   * while `get_local.is_activate` is true, `MixVisionTransformerEVP.forward` (and so `lfb.LFBExtractor`) runs the capture forward
-    (`sv_evp_forward_attention`) and appends one float32 array [B, heads, N, N_kv] per encoder block per call to
-    `get_local.cache['Attention.forward']`, in block order — what the reference's decorated `Attention.forward` records;
+    (`sv_evp_forward_attention`) and `forward_features` passes a maps buffer to `sv_evp_forward_features`; each appends one float32
+    array [B, heads, N, N_kv] per encoder block per call to `get_local.cache['Attention.forward']`, in block order — what the
+    reference's decorated `Attention.forward` records;
   * the switch is read at call time, so `activate()` also works after the model module has been imported (in the reference it must
     come before the import, because the decorator is applied then);
   * the flow cross-attention (`nn.MultiheadAttention`) is not decorated in the reference and is not captured here.

@@ -102,6 +102,25 @@ int sv_evp_forward_attention(sv_evp_handle* h, const float* x, const float* seg,
                              int64_t maps_elems, int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace,
                              size_t workspace_bytes, void* stream);
 
+/* Encoder feature pyramid: MixVisionTransformerEVP.forward_features(x, y) (mix_transformer_evp.py:352-416), the four stage outputs
+ * norm_s(x) as fp32 NCHW maps [B, C_s, H_s, W_s] (mit_b3_evp at 224x224: [B,64,56,56] [B,128,28,28] [B,320,14,14] [B,512,7,7]).
+ *   sv_evp_stage_shapes: host only (needs no device and no handle, only the config).  dims[3 * s .. 3 * s + 2] = (C_s, H_s, W_s) of
+ *     stage s for an HxW input: H_1 = (H + 2*3 - 7) / 4 + 1, then H_{s+1} = (H_s + 2 - 3) / 2 + 1 (W likewise).  Bad config, H or W,
+ *     or an input too small for the pyramid (a stage map smaller than its sr x sr spatial-reduction window, which the reference's
+ *     Conv2d rejects; 29 x 29 is the smallest input at sr 8 / 4 / 2 / 1) -> SV_ERR_INVALID; sv_evp_forward_features applies the same
+ *     checks.
+ *   sv_evp_forward_features: x, seg as sv_evp_forward; stage_out[s]: device, 4-byte aligned, >= B * C_s * H_s * W_s fp32 elements
+ *     (stage_elems[s] gives the size).  maps: NULL, or the attention maps of every encoder block in the layout of
+ *     sv_evp_attention_maps_layout (as sv_evp_forward_attention).  It runs encoder-only launch plans of its own: the encoder of
+ *     sv_evp_forward without the flow branch and the SegFormer head, whose stage norms write the NCHW maps; the plans of sv_evp_forward
+ *     and sv_evp_forward_attention are unchanged.  Workspace: sv_evp_workspace_bytes.  Every argument is checked before the device is
+ *     touched (SV_ERR_INVALID with the message in sv_last_error()).  Afterwards the "stage{1..4}_tokens" taps hold the last
+ *     micro-batch's stage outputs, as after sv_evp_forward. */
+int sv_evp_stage_shapes(const sv_evp_cfg* cfg, int32_t H, int32_t W, int32_t dims[12]);
+int sv_evp_forward_features(sv_evp_handle* h, const float* x, const float* seg, float* const stage_out[4], const int64_t stage_elems[4],
+                            float* maps, int64_t maps_elems, int32_t B, int32_t H, int32_t W, int32_t micro_batch, void* workspace,
+                            size_t workspace_bytes, void* stream);
+
 /* head.fc / head.fc_ant on extracted features (segformer_head.py:101-106,176-179):
  * feats [B,2048] fp32 device -> y [B,7], y_ant [B,7] fp32 device. */
 int sv_evp_classify(sv_evp_handle* h, const float* feats, float* y, float* y_ant, int32_t B, void* stream);
@@ -246,6 +265,13 @@ int sv_op_conv_gemm_plan_info(int32_t B, int32_t H, int32_t W, int32_t C, int32_
 /* LayerNorm over the last dim of fp32 [rows, C] -> optional fp32 and/or bf16 outputs (either may be NULL). */
 int sv_op_layernorm(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int32_t C,
                     float* out_f32, uint16_t* out_bf16, void* stream);
+
+/* The same LayerNorm with its fp32 result channel-major: rows = frames * tokens_per_frame token-major rows in, out_nchw[frame][c][token]
+ * out (the NCHW map of each frame), bit-identical to sv_op_layernorm's out_f32 permuted; out_bf16 (may be NULL) is token-major as in
+ * sv_op_layernorm.  rows must be a multiple of tokens_per_frame and rows * C < 2^31; x, gamma, beta 16-byte aligned, out_bf16 8-byte,
+ * out_nchw 4-byte.  Argument errors -> SV_ERR_INVALID before anything is launched. */
+int sv_op_layernorm_nchw(const float* x, const float* gamma, const float* beta, float eps, int64_t rows, int32_t C, int32_t tokens_per_frame,
+                         float* out_nchw, uint16_t* out_bf16, void* stream);
 
 /* Patch gather (im2col) with k index ordered (kh, kw, cin), row stride ldo (zero padded to ldo).
  * src_nchw_f32 != NULL: source is [B,Cin,H,W] fp32; else src_nhwc_bf16 is [B,H,W,Cin] bf16 (Cin%8==0). */

@@ -3,9 +3,10 @@
     python scripts/sass_offline_diff.py <earlier libsurgvid.so, e.g. from scripts/build_prev_lib.sh> <mstcn.o | libsurgvid.so> [...]
     python scripts/sass_offline_diff.py --all <earlier libsurgvid.so> <libsurgvid.so> [...]
 
-Default: the offline MS-TCN layer and Trans-SVNet head kernels.  The stream path gave these kernels a template parameter
-(`OfflineTaps` / `StreamTaps`, `OfflineWindow` / `StreamWindow`), and d_k = 64 gave the head kernel another
-(`trans_head_kernel<DK, Window>`); the offline instantiations and both d_k = 32 head instantiations must not change.
+Default: the offline MS-TCN layer and Trans-SVNet head kernels, and the LayerNorm kernel.  The stream path gave these kernels a
+template parameter (`OfflineTaps` / `StreamTaps`, `OfflineWindow` / `StreamWindow`), and d_k = 64 gave the head kernel another
+(`trans_head_kernel<DK, Window>`); the offline instantiations and both d_k = 32 head instantiations must not change.  The channel-major
+output form gave `layernorm_kernel<LPR, NV, EXACT, NCHW>` its last parameter; the 32 token-major instantiations must not change.
 
 --all: every kernel of the two builds, matched by name, for changes that must not touch device code (host-only refactors).  Both builds
 must have the same set of kernels.  Names in an anonymous namespace carry per-file hashes (`_GLOBAL__N__<8 hex>`, `_cu_<8 hex>`) that
@@ -42,6 +43,10 @@ PAIRS = [("mstcn_layer_tc_kernel(EPKf|INS0_11OfflineTaps)", "mstcn_layer_tc_kern
          ("mstcn_layer_kernelILi32ELi1E(EE|NS0_11OfflineTaps)", "mstcn_layer_kernelILi32ELi1ENS0_11OfflineTaps"),
          ("trans_head_kernel(EPKf|INS0_13OfflineWindow|ILi32ENS0_13OfflineWindow)", "trans_head_kernelILi32ENS0_13OfflineWindow"),
          ("trans_head_kernel(INS0_12StreamWindow|ILi32ENS0_12StreamWindow)", "trans_head_kernelILi32ENS0_12StreamWindow")]
+# the lane mappings of the LayerNorm dispatch table (elementwise.cu), exact and predicated; the earlier name has no NCHW parameter
+PAIRS += [(f"layernorm_kernelILi{l}ELi{n}ELb{e}EEEv", f"layernorm_kernelILi{l}ELi{n}ELb{e}ELb0EEEv")
+          for l, n in ((2, 2), (4, 2), (8, 2), (8, 4), (16, 4), (32, 4), (2, 5), (4, 5), (8, 5), (16, 5), (4, 1), (8, 1), (16, 1), (32, 1),
+                       (32, 2), (32, 3)) for e in (0, 1)]
 
 
 def by_stable_name(res):
