@@ -34,13 +34,13 @@ EXPORTED_SYMBOLS = [
     "sv_trans_stream_state_bytes", "sv_trans_stream_reset", "sv_trans_stream_forward",
     "sv_evp_attention_maps_layout", "sv_evp_forward_attention", "sv_op_attention_probs", "sv_op_gemm_plan_info",
     "sv_op_conv_gemm_bf16", "sv_op_conv_gemm_plan_info",
-    "sv_evp_stage_shapes", "sv_evp_forward_features", "sv_op_layernorm_nchw",
+    "sv_evp_stage_shapes", "sv_evp_forward_features", "sv_op_layernorm_nchw", "sv_op_dwconv_plan_info",
 ]
 
 # entry points an earlier build of the library, loaded through SURGVID_LIB for a same-box A/B run, may not have (build() still requires
 # every EXPORTED_SYMBOLS entry of the library it builds)
 _ABSENT_IN_EARLIER_BUILDS = ("sv_op_conv_gemm_bf16", "sv_op_conv_gemm_plan_info", "sv_evp_stage_shapes", "sv_evp_forward_features",
-                             "sv_op_layernorm_nchw")
+                             "sv_op_layernorm_nchw", "sv_op_dwconv_plan_info")
 
 
 class EvpCfg(Structure):
@@ -146,6 +146,8 @@ def _declare(lib):
                                                 c_int32, c_int32, c_void_p, c_size_t, c_void_p]
     lib.sv_op_im2col.argtypes = [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int64, c_void_p]
     lib.sv_op_dwconv3x3_gelu.argtypes = [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]
+    if hasattr(lib, "sv_op_dwconv_plan_info"):   # see _ABSENT_IN_EARLIER_BUILDS
+        lib.sv_op_dwconv_plan_info.argtypes = [c_int32, c_int32, c_int32, c_int32, c_int32, POINTER(c_int32)]
     lib.sv_op_attention.argtypes = [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_int32, c_int32,
                                     c_int32, c_int32, c_float, c_void_p]
     lib.sv_op_attention_kernel.argtypes = [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_int32]

@@ -83,15 +83,19 @@ __device__ __forceinline__ f32x2 f2_from_bf16x2(uint32_t v) {
   return r;
 }
 
-// GELU(erf) for two lanes without MUFU.  erf is odd, so with xc = clamp(x, -3*sqrt2, 3*sqrt2) and w = xc^2:
-//   erf(x/sqrt2) ~= (xc/sqrt2) * P(w/2),   P = degree-8 near-minimax fit of erf(z)/z on z in [0,3] (|erf err| <= 1.7e-5,
-//   erf(3) = 0.99998, clamped beyond), and   y = 0.5*x*(1 + erf(x/sqrt2)) = 0.5*x + (x*xc) * Q(w),
+// GELU(erf) for two lanes without MUFU.  erf is odd, so with xc = clamp(x, -lim, lim) and w = xc^2:
+//   erf(x/sqrt2) ~= (xc/sqrt2) * P(w/2),   P = degree-8 near-minimax fit of erf(z)/z on z in [0,3] (|erf err| <= 1.7e-5),
+//   and   y = 0.5*x*(1 + erf(x/sqrt2)) = 0.5*x + x * (xc * Q(w)),
 // Q(w) = 0.5/sqrt2 * P(w/2) with the constant factors folded into the coefficients.  |GELU error| <= 6.1e-5 absolute —
 // below the bf16 rounding of the stored result for |y| > 0.03 and negligible below that (end-to-end parity unchanged).
+// lim = 4.244771 (z = 3.0015, just past the fit's end, where P crosses 1) is an fp32 value at which the fp32 evaluation of
+// xc * Q(w) is exactly 0.5: beyond the clamp y is exactly x or 0, so the error does not grow with |x| (at 3*sqrt2 it was
+// 0.5 - 2.4e-6, an error of 2.4e-6 |x|).  |xc * Q| <= 0.5, so x * (xc * Q) cannot overflow for any finite x
+// ((x * xc) * Q did for |x| >= 8.0e37).
 __device__ __forceinline__ f32x2 f2_gelu_erf_poly(f32x2 x) {
   float x0, x1;
   f2_unpack(x, x0, x1);
-  const float lim = 4.2426406871192851f;  // 3*sqrt(2)
+  const float lim = 4.244771f;  // see above: fp32 xc * Q(w) == 0.5 exactly
   const f32x2 xc = f2_pack(fminf(fmaxf(x0, -lim), lim), fminf(fmaxf(x1, -lim), lim));
   const f32x2 w = f2_mul(xc, xc);
 #define SV_C2(v) f2_pack(v, v)
@@ -104,7 +108,7 @@ __device__ __forceinline__ f32x2 f2_gelu_erf_poly(f32x2 x) {
   q = f2_fma(q, w, SV_C2(9.818119241e-03f));
   q = f2_fma(q, w, SV_C2(-6.634692395e-02f));
   q = f2_fma(q, w, SV_C2(3.989031282e-01f));
-  return f2_fma(f2_mul(x, xc), q, f2_mul(x, SV_C2(0.5f)));
+  return f2_fma(x, f2_mul(xc, q), f2_mul(x, SV_C2(0.5f)));
 #undef SV_C2
 }
 
@@ -114,7 +118,7 @@ __device__ __forceinline__ void f2_gelu_erf_poly_x2(f32x2& xa, f32x2& xb) {
   float a0, a1, b0, b1;
   f2_unpack(xa, a0, a1);
   f2_unpack(xb, b0, b1);
-  const float lim = 4.2426406871192851f;
+  const float lim = 4.244771f;
   const f32x2 ca = f2_pack(fminf(fmaxf(a0, -lim), lim), fminf(fmaxf(a1, -lim), lim));
   const f32x2 cb = f2_pack(fminf(fmaxf(b0, -lim), lim), fminf(fmaxf(b1, -lim), lim));
   const f32x2 wa = f2_mul(ca, ca), wb = f2_mul(cb, cb);
@@ -130,14 +134,14 @@ __device__ __forceinline__ void f2_gelu_erf_poly_x2(f32x2& xa, f32x2& xb) {
   SV_STEP(-6.634692395e-02f)
   SV_STEP(3.989031282e-01f)
 #undef SV_STEP
-  xa = f2_fma(f2_mul(xa, ca), qa, f2_mul(xa, SV_C2(0.5f)));
-  xb = f2_fma(f2_mul(xb, cb), qb, f2_mul(xb, SV_C2(0.5f)));
+  xa = f2_fma(xa, f2_mul(ca, qa), f2_mul(xa, SV_C2(0.5f)));
+  xb = f2_fma(xb, f2_mul(cb, qb), f2_mul(xb, SV_C2(0.5f)));
 #undef SV_C2
 }
 
 // four independent evaluations, Horner steps in lockstep (used where only two warps share a scheduler)
 __device__ __forceinline__ void f2_gelu_erf_poly_x4(f32x2& xa, f32x2& xb, f32x2& xc, f32x2& xd) {
-  const float lim = 4.2426406871192851f;
+  const float lim = 4.244771f;
   auto clamp2 = [&](f32x2 v) {
     float v0, v1;
     f2_unpack(v, v0, v1);
@@ -159,10 +163,10 @@ __device__ __forceinline__ void f2_gelu_erf_poly_x4(f32x2& xa, f32x2& xb, f32x2&
   SV_STEP(-6.634692395e-02f)
   SV_STEP(3.989031282e-01f)
 #undef SV_STEP
-  xa = f2_fma(f2_mul(xa, ca), qa, f2_mul(xa, SV_C2(0.5f)));
-  xb = f2_fma(f2_mul(xb, cb), qb, f2_mul(xb, SV_C2(0.5f)));
-  xc = f2_fma(f2_mul(xc, cc), qc, f2_mul(xc, SV_C2(0.5f)));
-  xd = f2_fma(f2_mul(xd, cd), qd, f2_mul(xd, SV_C2(0.5f)));
+  xa = f2_fma(xa, f2_mul(ca, qa), f2_mul(xa, SV_C2(0.5f)));
+  xb = f2_fma(xb, f2_mul(cb, qb), f2_mul(xb, SV_C2(0.5f)));
+  xc = f2_fma(xc, f2_mul(cc, qc), f2_mul(xc, SV_C2(0.5f)));
+  xd = f2_fma(xd, f2_mul(cd, qd), f2_mul(xd, SV_C2(0.5f)));
 #undef SV_C2
 }
 

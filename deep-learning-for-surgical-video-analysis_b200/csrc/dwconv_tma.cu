@@ -226,47 +226,60 @@ static int dw_cpl() {
 }
 bool dwconv_tma_supported(int C) { return C % kCB == 0; }
 
+int dwconv_tma_shape(int B, int H, int W, int C, int sms, DwconvShape* s) {
+  SV_CHECK(B > 0 && H > 0 && W > 0 && sms > 0 && dwconv_tma_supported(C), "dwconv TMA shape");
+  static const int env_stages = [] { const char* e = getenv("SURGVID_DW_STAGES"); return e ? atoi(e) : 0; }();
+  static const int env_prefetch = [] { const char* e = getenv("SURGVID_DW_PREFETCH"); return e ? atoi(e) : 0; }();
+  static const int gelu_mode = [] { const char* e = getenv("SURGVID_DW_GELU"); const int v = e ? atoi(e) : 2; return v == 0 || v == 1 ? v : 2; }();
+  s->cpl = dw_cpl();
+  s->gelu = gelu_mode;
+  s->stages = std::min(kMaxStages, std::max(2, env_stages > 0 ? env_stages : kStages));
+  s->prefetch = std::min(s->stages - 1, std::max(1, env_prefetch > 0 ? env_prefetch : kPrefetch));
+  s->tw = (W % 8 == 0) ? 8 : ((W % 7 == 0) ? 7 : 8);
+  s->tiles_x = ceil_div(W, s->tw);
+  s->tiles_y = ceil_div(H, kTH);
+  s->cblks = C / (32 * s->cpl);
+  const long long nt = static_cast<long long>(s->cblks) * B * s->tiles_y * s->tiles_x;
+  if (nt >= (1LL << 31)) return fail(SV_ERR_INVALID, "dwconv: more than 2^31 tiles");
+  s->num_tiles = static_cast<int>(nt);
+  s->grid = static_cast<int>(std::min<long long>(s->num_tiles, (s->cpl == 4 ? 2LL : 4LL) * sms));
+  s->smem_bytes = s->stages * (kBoxH * kBoxW * 32 * s->cpl * 2) + 128;
+  return SV_OK;
+}
+
 int dwconv_tma_plan(const bf16* x, const float* w9c, const float* bias, int B, int H, int W, int C, bf16* out, int64_t ldo, DwconvPlan* plan) {
   SV_CHECK(ldo >= C && ldo % 4 == 0, "dwconv output row stride");
   SV_CHECK(dwconv_tma_supported(C), "dwconv TMA path needs C % 128 == 0");
   SV_CHECK((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 7) == 0, "dwconv alignment");
+  DwconvShape s;
+  SV_TRY(dwconv_tma_shape(B, H, W, C, 1, &s));   // tw and cpl do not depend on the SM count
   cuuint64_t gdim[4] = {static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H), static_cast<cuuint64_t>(B)};
   cuuint64_t gstr[3] = {static_cast<cuuint64_t>(C) * 2, static_cast<cuuint64_t>(W) * C * 2, static_cast<cuuint64_t>(H) * W * C * 2};
-  const int tw = (W % 8 == 0) ? 8 : ((W % 7 == 0) ? 7 : 8);
-  cuuint32_t box[4] = {static_cast<cuuint32_t>(32 * dw_cpl()), static_cast<cuuint32_t>(tw + 2), kBoxH, 1};
+  cuuint32_t box[4] = {static_cast<cuuint32_t>(32 * s.cpl), static_cast<cuuint32_t>(s.tw + 2), kBoxH, 1};
   SV_TRY(encode_tiled(&plan->tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, x, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_NONE,
                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "dwconv"));
-  plan->w9c = w9c; plan->bias = bias; plan->out = out; plan->B = B; plan->H = H; plan->W = W; plan->C = C; plan->ldo = ldo; plan->tw = tw;
-  plan->cpl = dw_cpl();
+  plan->w9c = w9c; plan->bias = bias; plan->out = out; plan->B = B; plan->H = H; plan->W = W; plan->C = C; plan->ldo = ldo; plan->tw = s.tw;
+  plan->cpl = s.cpl;
   return SV_OK;
 }
 
 int dwconv_tma_launch(const DwconvPlan& plan, cudaStream_t st) {
-  const int cb = 32 * plan.cpl;
-  static const int env_stages = [] { const char* e = getenv("SURGVID_DW_STAGES"); return e ? atoi(e) : 0; }();
-  static const int env_prefetch = [] { const char* e = getenv("SURGVID_DW_PREFETCH"); return e ? atoi(e) : 0; }();
-  const int stages = std::min(kMaxStages, std::max(2, env_stages > 0 ? env_stages : kStages));
-  const int prefetch = std::min(stages - 1, std::max(1, env_prefetch > 0 ? env_prefetch : kPrefetch));
-  const int smem_bytes = stages * (kBoxH * kBoxW * cb * 2) + 128;
-  static const int gelu_mode = [] { const char* e = getenv("SURGVID_DW_GELU"); return e ? atoi(e) : 2; }();
+  DwconvShape s;
+  SV_TRY(dwconv_tma_shape(plan.B, plan.H, plan.W, plan.C, device_sm_count(), &s));
   typedef void (*KernFn)(const CUtensorMap, const DwParams);
   KernFn kern;
-  if (plan.cpl == 4) kern = gelu_mode == 0 ? dwconv3x3_gelu_tma_kernel<0, 4> : (gelu_mode == 1 ? dwconv3x3_gelu_tma_kernel<1, 4> : dwconv3x3_gelu_tma_kernel<2, 4>);
-  else kern = gelu_mode == 0 ? dwconv3x3_gelu_tma_kernel<0, 2> : (gelu_mode == 1 ? dwconv3x3_gelu_tma_kernel<1, 2> : dwconv3x3_gelu_tma_kernel<2, 2>);
-  SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(kern), smem_bytes));
+  if (plan.cpl == 4) kern = s.gelu == 0 ? dwconv3x3_gelu_tma_kernel<0, 4> : (s.gelu == 1 ? dwconv3x3_gelu_tma_kernel<1, 4> : dwconv3x3_gelu_tma_kernel<2, 4>);
+  else kern = s.gelu == 0 ? dwconv3x3_gelu_tma_kernel<0, 2> : (s.gelu == 1 ? dwconv3x3_gelu_tma_kernel<1, 2> : dwconv3x3_gelu_tma_kernel<2, 2>);
+  SV_TRY(ensure_dynamic_smem(reinterpret_cast<const void*>(kern), s.smem_bytes));
   DwParams p;
   p.w9c = plan.w9c; p.bias = plan.bias; p.out = plan.out; p.B = plan.B; p.H = plan.H; p.W = plan.W; p.C = plan.C; p.ldo = plan.ldo;
   p.tw = plan.tw;
-  p.stages = stages; p.prefetch = prefetch;
-  p.tiles_x = ceil_div(plan.W, plan.tw); p.tiles_y = ceil_div(plan.H, kTH); p.cblks = plan.C / cb;
-  const long long nt = static_cast<long long>(p.cblks) * plan.B * p.tiles_y * p.tiles_x;
-  if (nt >= (1LL << 31)) return fail(SV_ERR_INVALID, "dwconv: more than 2^31 tiles");
-  p.num_tiles = static_cast<int>(nt);
+  p.stages = s.stages; p.prefetch = s.prefetch;
+  p.tiles_x = s.tiles_x; p.tiles_y = s.tiles_y; p.cblks = s.cblks;
+  p.num_tiles = s.num_tiles;
   p.tiles_per_cblk = plan.B * p.tiles_y * p.tiles_x;
   p.row_stride = static_cast<long long>(plan.W) * plan.ldo;
-  const int sms = device_sm_count();
-  const int grid = static_cast<int>(std::min<long long>(p.num_tiles, (plan.cpl == 4 ? 2LL : 4LL) * sms));
-  kern<<<grid, kThreads, smem_bytes, st>>>(plan.tmap, p);
+  kern<<<s.grid, kThreads, s.smem_bytes, st>>>(plan.tmap, p);
   return launch_status("dwconv3x3_gelu_tma_kernel");
 }
 

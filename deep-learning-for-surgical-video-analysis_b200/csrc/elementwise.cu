@@ -1,6 +1,8 @@
 // HBM-bound kernels of the LFB path: LayerNorm, patch gather (im2col), depthwise 3x3 + GELU, Gaussian 5x5,
 // bilinear token resize, token mean.  All 128-bit vectorised on channels-last (token-major == NHWC) tensors;
 // the reference's NCHW<->NLC transposes (mix_transformer_evp.py:26-28, 115-116, 212, 376) never happen.
+#include <algorithm>
+
 #include "kernels.cuh"
 
 namespace sv {
@@ -492,6 +494,7 @@ int launch_im2col(const float* src_nchw_f32, const bf16* src_nhwc_bf16, int B, i
 
 int launch_dwconv3x3_gelu(const bf16* x, const float* w9c, const float* bias, int B, int H, int W, int C, bf16* out, int64_t ldo,
                           cudaStream_t st) {
+  SV_CHECK(B > 0 && H > 0 && W > 0 && C > 0, "dwconv dims must be positive");
   SV_CHECK(ldo >= C && ldo % 4 == 0, "dwconv output row stride");
   if (dwconv_tma_supported(C)) {  // main path: TMA halo staging (dwconv_tma.cu); the register-window kernel below covers C % 128 != 0
     DwconvPlan plan;
@@ -505,6 +508,37 @@ int launch_dwconv3x3_gelu(const bf16* x, const float* w9c, const float* bias, in
   dim3 block(32, kDwCols);
   dwconv3x3_gelu_kernel<<<grid, block, 0, st>>>(x, w9c, bias, B, H, W, C, out, ldo);
   return launch_status("dwconv3x3_gelu_kernel");
+}
+
+int dwconv_plan_info(int B, int H, int W, int C, int sms, int32_t* info) {
+  SV_CHECK(info != nullptr, "dwconv plan info: null output");
+  SV_CHECK(B > 0 && H > 0 && W > 0 && C > 0 && sms > 0, "dwconv dims and SM count must be positive");
+  SV_CHECK(C % 4 == 0, "dwconv needs C%4==0");
+  if (dwconv_tma_supported(C)) {
+    DwconvShape s;
+    SV_TRY(dwconv_tma_shape(B, H, W, C, sms, &s));
+    // the tile ranges of dwconv3x3_gelu_tma_kernel: CTA i walks [i * per + min(i, extra), ... + per + (i < extra))
+    const int per = s.num_tiles / s.grid, extra = s.num_tiles % s.grid;
+    const int per_frame = s.tiles_y * s.tiles_x, per_cblk = B * per_frame;
+    int cross_frame = 0, cross_cblk = 0;
+    for (int i = 0; i < s.grid; ++i) {
+      const int tb = i * per + std::min(i, extra), te = tb + per + (i < extra ? 1 : 0);
+      if ((tb / per_frame + 1) * static_cast<int64_t>(per_frame) < te) cross_frame = 1;
+      if ((tb / per_cblk + 1) * static_cast<int64_t>(per_cblk) < te) cross_cblk = 1;
+    }
+    const int32_t t[SV_DWCONV_PLAN_INFO_LEN] = {SV_DWCONV_TMA, s.cpl, s.gelu, s.stages, s.prefetch, s.tw, s.tiles_x, s.tiles_y, s.cblks,
+                                               s.num_tiles, s.grid, per + (extra ? 1 : 0), cross_frame, cross_cblk};
+    std::copy(t, t + SV_DWCONV_PLAN_INFO_LEN, info);
+  } else {
+    const int hsegs = ceil_div(H, kDwRun);
+    SV_CHECK(static_cast<int64_t>(B) * hsegs <= 65535 && ceil_div(C, 128) <= 65535, "dwconv grid limits");
+    const int64_t blocks = static_cast<int64_t>(ceil_div(W, kDwCols)) * B * hsegs * ceil_div(C, 128);
+    SV_CHECK(blocks < (1LL << 31), "dwconv grid limits");
+    const int32_t t[SV_DWCONV_PLAN_INFO_LEN] = {SV_DWCONV_SIMT, 4, 0, 0, 0, kDwCols, ceil_div(W, kDwCols), hsegs, ceil_div(C, 128),
+                                               static_cast<int32_t>(blocks), static_cast<int32_t>(blocks), 1, 0, 0};
+    std::copy(t, t + SV_DWCONV_PLAN_INFO_LEN, info);
+  }
+  return SV_OK;
 }
 
 int launch_gauss5x5(const float* x, float* out, int planes, int H, int W, cudaStream_t st) {
@@ -553,6 +587,9 @@ int sv_op_dwconv3x3_gelu(const uint16_t* x, const float* w, const float* bias, i
                          void* stream) {
   return sv::launch_dwconv3x3_gelu(reinterpret_cast<const sv::bf16*>(x), w, bias, B, H, W, C, reinterpret_cast<sv::bf16*>(out), C,
                                    static_cast<cudaStream_t>(stream));
+}
+int sv_op_dwconv_plan_info(int32_t B, int32_t H, int32_t W, int32_t C, int32_t num_sms, int32_t* info) {
+  return sv::dwconv_plan_info(B, H, W, C, num_sms, info);
 }
 int sv_op_gauss5x5(const float* x, float* out, int32_t planes, int32_t H, int32_t W, void* stream) {
   return sv::launch_gauss5x5(x, out, planes, H, W, static_cast<cudaStream_t>(stream));

@@ -50,6 +50,12 @@ struct DwconvPlan {
   int cpl = 4;      // channels per lane: 4 (128-channel tiles) or 2 (64-channel tiles)
 };
 bool dwconv_tma_supported(int C);
+// launch geometry of the TMA form on a device with `sms` SMs (host only): dwconv_tma_launch and sv_op_dwconv_plan_info both take it from here
+struct DwconvShape {
+  int cpl, gelu, stages, prefetch, tw;
+  int tiles_x, tiles_y, cblks, num_tiles, grid, smem_bytes;
+};
+int dwconv_tma_shape(int B, int H, int W, int C, int sms, DwconvShape* s);
 int dwconv_tma_plan(const bf16* x, const float* w9c, const float* bias, int B, int H, int W, int C, bf16* out, int64_t ldo, DwconvPlan* plan);
 int dwconv_tma_launch(const DwconvPlan& plan, cudaStream_t st);
 

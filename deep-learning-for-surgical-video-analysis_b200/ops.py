@@ -262,6 +262,23 @@ def dwconv3x3_gelu(x: torch.Tensor, w9c: torch.Tensor, bias: torch.Tensor) -> to
     return out
 
 
+DWCONV_PLAN_FIELDS = ("kernel", "cpl", "gelu", "stages", "prefetch", "tw", "tiles_x", "tiles_y", "cblks", "num_tiles", "grid",
+                      "max_tiles_per_cta", "crosses_frame", "crosses_cblk")
+DWCONV_KERNELS = ("simt", "tma")   # SV_DWCONV_* in include/surgvid.h
+
+
+def dwconv_plan_info(B: int, H: int, W: int, C: int, num_sms: Optional[int] = None) -> dict:
+    """How dwconv3x3_gelu runs this problem (sv_op_dwconv_plan_info; host only).  `num_sms` defaults to the current device's SM count;
+    `kernel` is named by DWCONV_KERNELS."""
+    if num_sms is None:
+        num_sms = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+    info = (ctypes.c_int32 * len(DWCONV_PLAN_FIELDS))()
+    _native.check(_native.lib().sv_op_dwconv_plan_info(B, H, W, C, num_sms, info), "sv_op_dwconv_plan_info")
+    d = dict(zip(DWCONV_PLAN_FIELDS, info))
+    d["kernel"] = DWCONV_KERNELS[d["kernel"]]
+    return d
+
+
 def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, B: int, heads: int, hd: int, scale: float,
               out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """q [B*Nq, >=heads*hd] bf16, k/v [B*Nkv, ...] bf16 (row-strided views allowed) -> o [B*Nq, heads*hd] bf16, written into `out`

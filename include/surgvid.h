@@ -283,6 +283,20 @@ int sv_op_im2col(const float* src_nchw_f32, const uint16_t* src_nhwc_bf16, int32
 int sv_op_dwconv3x3_gelu(const uint16_t* x, const float* w, const float* bias, int32_t B, int32_t H, int32_t W,
                          int32_t C, uint16_t* out, void* stream);
 
+/* How sv_op_dwconv3x3_gelu runs a problem on a device with num_sms SMs.  Host only: touches neither device nor driver; the launch
+ * takes its geometry from the same function.  It depends on B, H, W, C and the switches SURGVID_DW_CPL / _GELU / _STAGES /
+ * _PREFETCH, read once per process.  info[SV_DWCONV_PLAN_INFO_LEN]:
+ *   0 kernel (SV_DWCONV_*), 1 channels per lane (cpl), 2 GELU form (0 erf polynomial, 1 sigmoid on ex2/rcp, 2 tanh.approx),
+ *   3 shared-memory ring stages, 4 prefetch distance (both 0 for the SIMT kernel), 5 output columns per tile (tw), 6 tiles_x,
+ *   7 tiles_y (7-row tiles), 8 channel blocks (32 * cpl channels), 9 num_tiles, 10 grid (CTAs), 11 most tiles one CTA walks,
+ *   12 some CTA's tile range crosses a frame boundary, 13 some CTA's range crosses a channel-block boundary.
+ * The TMA kernel takes C % 128 == 0; the SIMT kernel (one 7 x 8 x 128 tile per CTA, polynomial GELU) every other C % 4 == 0 and
+ * B * ceil(H / 7) <= 65535.  Shape errors (as sv_op_dwconv3x3_gelu reports them) -> SV_ERR_INVALID. */
+#define SV_DWCONV_SIMT 0
+#define SV_DWCONV_TMA 1
+#define SV_DWCONV_PLAN_INFO_LEN 14
+int sv_op_dwconv_plan_info(int32_t B, int32_t H, int32_t W, int32_t C, int32_t num_sms, int32_t* info);
+
 /* softmax(Q K^T * scale) V per (frame, head). Q rows = B*Nq, K/V rows = B*Nkv; head h occupies columns
  * [h*hd, (h+1)*hd) of each; hd in {20, 32, 40, 64} (mix_transformer_evp.py:123-127, 868-883).  ldq, ldk, ldv % 8 == 0 and
  * q, k, v 16-byte aligned; ldo even and o 4-byte aligned; only the [B*Nq, heads*hd] block of o is written. */

@@ -40,6 +40,7 @@ BIAS_GATE = 0.08                                      # mean signed bf16 roundin
 BIAS_MIN_ELEMS = 2000                                 # fewer eligible elements: the bias check is skipped
 BIAS_ELIGIBLE = 0.02                                  # eligible: accumulation bound <= 2 % of the element's bf16 ulp
 
+GELU_HUGE = (8.1e37, -8.1e37, 1e38, -1e38, 3e38, -3e38)   # pre-activations past 8.04e37 (gelu_sweep)
 STRESS = ("randn", "bigres", "colbias", "gelu_sweep", "cancel", "rowid")
 
 
@@ -140,7 +141,8 @@ def make_inputs(kind: str, M: int, N: int, K: int, K2: int = 0, seed: int = 0, d
       randn       A ~ N(0, 1), bias ~ 0.5 N(0, 1), residual ~ N(0, 1).
       bigres      |residual| ~ 1e3: a residual that passes through bf16 loses ~2 in the sum.
       colbias     bias is a per-column ramp (-4 ... 4): a bias slice shifted by a tile or a 16 / 32-column chunk is off by >= 16 steps.
-      gelu_sweep  small A W^T and a bias ramp over [-10, 10]: pre-activations cross the erf polynomial's clamp at +-3 sqrt2 and the tails.
+      gelu_sweep  small A W^T and a bias ramp over [-10, 10]: pre-activations cross the erf polynomial's clamp and the tails; the first
+                  columns' biases are GELU_HUGE, where x * xc * Q overflowed when it was evaluated as (x * xc) * Q.
       cancel      rows of A share a large mean (~32) and the rows of W sum to ~0: |ref| << |A| |W|^T.
       rowid       residual[r, c] = r % 1024 + c / 1024: any mix-up of rows, lane quarters or M tiles moves the result by >= 1 (values on
                   a grid: the gate's rounding-bias check does not apply)."""
@@ -161,6 +163,7 @@ def make_inputs(kind: str, M: int, N: int, K: int, K2: int = 0, seed: int = 0, d
     elif kind == "gelu_sweep":
         W = W * 0.3
         b = torch.linspace(-10.0, 10.0, N, device=device)[torch.randperm(N, generator=g, device=device)]
+        b[:len(GELU_HUGE)] = torch.tensor(GELU_HUGE, device=device)
     elif kind == "cancel":
         A = 32.0 + A
         W = W - W.mean(1, keepdim=True)
@@ -175,16 +178,24 @@ def make_inputs(kind: str, M: int, N: int, K: int, K2: int = 0, seed: int = 0, d
 
 
 # --------------------------------------------------------------------------------------------------------------- emulator
+GELU_POLY_LIM = 4.244771   # the polynomial's clamp: fp32 xc * Q(xc^2) is exactly 0.5 there (common.cuh)
+GELU_POLY_COEF = (5.626770213e-11, -5.371870724e-09, 2.268296714e-07, -5.646215765e-06, 9.359063167e-05, -1.109400333e-03, 9.818119241e-03,
+                  -6.634692395e-02, 3.989031282e-01)
+
+
 def gelu_poly_f32(x: torch.Tensor) -> torch.Tensor:
-    """f2_gelu_erf_poly (common.cuh) in fp32: 0.5 x + x clamp(x) Q(clamp(x)^2), the GELU of bf16 outputs."""
-    lim = 4.2426406871192851
-    xc = x.clamp(-lim, lim)
+    """f2_gelu_erf_poly (common.cuh) in fp32, FMA by FMA: 0.5 x + x (xc Q(xc^2)) with xc = clamp(x), the GELU of bf16 outputs."""
+    def fma(a, b, c):   # the product of two fp32 values is exact in float64
+        return (a.double() * b.double() + c.double()).float()
+
+    x = x.float()
+    lim = torch.tensor(GELU_POLY_LIM, dtype=torch.float32)
+    xc = torch.minimum(torch.maximum(x, -lim), lim)
     w = xc * xc
-    q = torch.full_like(x, 5.626770213e-11)
-    for c in (-5.371870724e-09, 2.268296714e-07, -5.646215765e-06, 9.359063167e-05, -1.109400333e-03, 9.818119241e-03,
-              -6.634692395e-02, 3.989031282e-01):
-        q = q * w + c
-    return (x * xc) * q + x * 0.5
+    q = fma(torch.tensor(GELU_POLY_COEF[0]), w, torch.tensor(GELU_POLY_COEF[1]))
+    for c in GELU_POLY_COEF[2:]:
+        q = fma(q, w, torch.tensor(c))
+    return fma(x, xc * q, x * 0.5)
 
 
 def gelu_erf_f32(x: torch.Tensor) -> torch.Tensor:
